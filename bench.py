@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
                     [--workload c2|c2rot|c2dense|c2gauss|c2w21|c2ref|c1|c3|c4|all] [--tune field=value,...]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the whole hot path over one batch of frame pairs taken from a synthetic
 sequence that is resident in HBM (device arm) / in pinned host memory (e2e).  Prints ONE JSON line.
@@ -10,6 +11,8 @@ Metric: BASELINE.json -> 1080p frame-pairs/sec (flow+FoE+mask), plus % of HBM ro
 Farneback iteration kernel.  `--impl reference` times the reference's own CPU path (cv2's Farneback +
 the NumPy restatement of the reference's FoE/phi/mask code in oracle/) on the host cores.
 `--workload all` measures C2 (the headline) and adds one line per other configuration under `extra`.
+`--dump-outputs DIR` writes what the headline workload's last timed step returned to its caller as DIR/<name>.npy
+(see dump_outputs); the inputs depend only on the arguments, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -53,6 +56,8 @@ WORKLOADS = {
 }
 EXTRA_ORDER = ['c2rot', 'c2dense', 'c2ref', 'c1', 'c3', 'c4']
 N_BATCHES = 4          # distinct resident batches cycled through (working set per step >> L2 anyway)
+DUMP_MASK_SAMPLES = 1 << 21   # fixed-mask pixels kept by --dump-outputs (C2's 64 masks hold 133 M pixels)
+DUMP_SEED = 0
 
 
 def hbm_peak():
@@ -135,6 +140,30 @@ def build_workload(name: str, rank: int = 0, pairs: int = 0):
         samples[i, :2000] = rs.randint(0, H, 2000)
         samples[i, 2000:] = rs.randint(0, W, 2000)
     return dict(name=name, W=W, H=H, params=params, B=B, label=label, seq=seq, samples=samples)
+
+
+def dump_outputs(out_dir: str, records: np.ndarray, fixed: np.ndarray) -> None:
+    """Writes one step's outputs, as a caller of Engine.process receives them, to out_dir/<name>.npy: each field of
+    the per-pair records as float64 (records_<field>, records_stats_<field>), and the (pairs, H, W) fixed masks as
+    float32, whole (fixed) when they hold at most DUMP_MASK_SAMPLES pixels, else as a seeded sample of them
+    (fixed_sample, taken at the flat indices stored as float64 in fixed_sample_index)."""
+    out = {}
+    for name in records.dtype.names:
+        if name == 'stats':
+            for sub in records.dtype['stats'].names:
+                out['records_stats_' + sub] = np.asarray(records['stats'][sub], np.float64)
+        else:
+            out['records_' + name] = np.asarray(records[name], np.float64)
+    flat = fixed.reshape(-1)
+    if flat.size <= DUMP_MASK_SAMPLES:
+        out['fixed'] = np.asarray(fixed, np.float32)
+    else:
+        idx = np.unique(np.random.default_rng(DUMP_SEED).integers(0, flat.size, DUMP_MASK_SAMPLES))
+        out['fixed_sample_index'] = idx.astype(np.float64)
+        out['fixed_sample'] = flat[idx].astype(np.float32)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
 
 
 def level_sizes(W, H, params):
@@ -349,6 +378,9 @@ def measure(name, args, steps, world, rank, local, headline):
         elapsed_ms = e0.elapsed_time(e1)
         clocks = sampler.stop(t_host0, t_host1) if (rank == 0 and headline) else None
         launches = eng.launch_count() - launches0
+        if args.dump_outputs and headline and rank == 0:
+            # the last timed step's outputs, before the passes below overwrite them
+            dump_outputs(args.dump_outputs, eng.records_to_numpy(records_d), fixed_d.cpu().numpy())
         # (2) per-kernel-class device times: the same steps again with CUDA events around every launch group
         # (profiling launches kernel by kernel, so it is kept out of the timed region above)
         psteps = max(2, min(steps, 8))
@@ -587,7 +619,13 @@ def main():
     ap.add_argument('--pairs', type=int, default=0, help='frame pairs per step (default: the workload\'s)')
     ap.add_argument('--tune', default=os.environ.get('MAVD_TUNE', ''),
                     help='mavd_tuning fields, e.g. pair_group=8,use_graph=0 (A/B runs; results never depend on them)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default='',
+                    help='write the outputs of the last timed step of the headline workload (rank 0) to DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs needs --impl b200')
     args.warmup = max(args.warmup, 3) if args.impl == 'b200' else args.warmup
     # stdout carries the JSON line and nothing else: keep a private handle on the real stdout for it and point file
     # descriptor 1 at stderr, so that whatever a library prints (NCCL's version banner, worker processes) lands there

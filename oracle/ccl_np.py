@@ -31,14 +31,20 @@ def canonicalise(labels: np.ndarray) -> np.ndarray:
 def stats_from_labels(labels: np.ndarray) -> np.ndarray:
     """(n, 5) int32 rows [left, top, width, height, area] for labels 1..n."""
     n = int(labels.max())
-    out = np.zeros((n, 5), np.int32)
     ys, xs = np.nonzero(labels)
-    lab = labels[ys, xs]
-    for i in range(1, n + 1):
-        sel = lab == i
-        x, y = xs[sel], ys[sel]
-        out[i - 1] = (x.min(), y.min(), x.max() - x.min() + 1, y.max() - y.min() + 1, sel.sum())
-    return out
+    lab = labels[ys, xs].astype(np.int64) - 1
+    # one pass over the foreground for all labels at once: a full-HD noise mask has thousands of components, and a
+    # pass per label over all of its pixels took minutes
+    x0 = np.full(n, np.iinfo(np.int64).max)
+    y0 = np.full(n, np.iinfo(np.int64).max)
+    x1 = np.full(n, -1, np.int64)
+    y1 = np.full(n, -1, np.int64)
+    np.minimum.at(x0, lab, xs)
+    np.minimum.at(y0, lab, ys)
+    np.maximum.at(x1, lab, xs)
+    np.maximum.at(y1, lab, ys)
+    area = np.bincount(lab, minlength=n)
+    return np.stack([x0, y0, x1 - x0 + 1, y1 - y0 + 1, area], axis=1).astype(np.int32).reshape(n, 5)
 
 
 def label_floodfill(mask: np.ndarray) -> np.ndarray:

@@ -63,3 +63,6 @@ def test_ccl_oracles_agree():
         assert stats.shape[0] == lab.max()
         if lab.max():
             assert stats[:, 4].sum() == m.sum()
+        for i in range(lab.max()):
+            ys, xs = np.nonzero(lab == i + 1)
+            assert tuple(stats[i]) == (xs.min(), ys.min(), xs.max() - xs.min() + 1, ys.max() - ys.min() + 1, xs.size)
