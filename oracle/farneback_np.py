@@ -213,21 +213,30 @@ def poly_exp(img: np.ndarray, n: int, sigma: float) -> np.ndarray:
     return R
 
 
+def _border_factors(n: int) -> Tuple[np.ndarray, np.ndarray]:
+    """Per-index factors from the low edge and from the high edge of one axis of length n (1 elsewhere)."""
+    i = np.arange(n)
+    lo = np.where(i < 5, BORDER[np.minimum(i, 4)], F32(1)).astype(F32)
+    hi = np.where(i >= n - 5, BORDER[np.clip(n - i - 1, 0, 4)], F32(1)).astype(F32)
+    return lo, hi
+
+
+def _border_gate(n: int) -> np.ndarray:
+    """cv's (unsigned)(i - 5) >= (unsigned)(n - 10) on one axis.  For n = 8 or 9 the right side wraps to a huge
+    unsigned value, so only i in {3, 4} (n = 8) or {4} (n = 9) pass, although every index lies within 5 of an edge."""
+    i = np.arange(n, dtype=np.int64)
+    return ((i - 5) % 2 ** 32) >= ((n - 10) % 2 ** 32)
+
+
 def border_scale(w: int, h: int) -> np.ndarray:
-    """Product of the per-edge attenuation factors for pixels within 5 of an edge (h, w) f32."""
-    sx = np.ones(w, dtype=F32)
-    sy = np.ones(h, dtype=F32)
-    for d in range(5):
-        if d < w:
-            sx[d] *= BORDER[d]
-        if w - 1 - d >= 0:
-            sx[w - 1 - d] *= BORDER[d]
-        if d < h:
-            sy[d] *= BORDER[d]
-        if h - 1 - d >= 0:
-            sy[h - 1 - d] *= BORDER[d]
-    # cv: scale = bx_left * bx_right * by_top * by_bottom evaluated left to right
-    return (sx[None, :] * sy[:, None]).astype(F32)
+    """FarnebackUpdateMatrices' border attenuation (h, w) f32: pixels that pass cv's gate
+    (unsigned)(x - 5) >= (unsigned)(w - 10) || (unsigned)(y - 5) >= (unsigned)(h - 10) are scaled by
+    ((left * right) * top) * bottom, multiplied in that order in float32; every other pixel by 1."""
+    xl, xr = _border_factors(w)
+    yt, yb = _border_factors(h)
+    sc = ((xl * xr)[None, :] * yt[:, None]).astype(F32) * yb[:, None]
+    gate = _border_gate(w)[None, :] | _border_gate(h)[:, None]
+    return np.where(gate, sc, F32(1)).astype(F32)
 
 
 def update_matrices(R0: np.ndarray, R1: np.ndarray, flow: np.ndarray) -> np.ndarray:
