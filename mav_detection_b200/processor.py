@@ -218,6 +218,7 @@ class Processor:
                     flows[k] = f
                 imu, samples, sky, seg, gt = self._host_inputs(indices, 0)
                 records = self._pinned(0, 'records', (n,), eng_records_dtype())
+                self.focus_of_expansion._eng()                   # its FoE thresholds -> eng.detect_params (shared engine)
                 eng.detect_host(flows, imu, samples, sky=sky, seg=seg, gt_flow=gt, records=records)
                 finish((-1, indices, records, sky, gt is not None, None))
             else:
@@ -234,6 +235,7 @@ class Processor:
                 records = self._pinned(slot, 'records', (n,), eng_records_dtype())
                 flow = self._pinned(slot, 'flow_out', (n, height, width, 2), np.float32) if self.flow_cache is not None \
                     else None
+                self.focus_of_expansion._eng()                   # the call copies detect_params: batches in flight keep theirs
                 eng.submit_host(slot, frames, imu, samples, n_pairs=n, sky=sky, seg=seg, gt_flow=gt, flow_out=flow,
                                 records=records)
                 inflight.append((slot, indices, records, sky, gt is not None, flow))

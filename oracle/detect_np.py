@@ -4,6 +4,14 @@ TEST INFRASTRUCTURE (see oracle/__init__.py).  Each function cites the reference
 lines it follows; tests/golden/make_golden.py checks these restatements against
 the reference modules themselves (imported from /root/reference with stub
 dependencies) and commits the resulting vectors.
+
+Parameters.  `intersections`, `ransac`, `foe_dense`, `masks` and `frame_pipeline` take keyword parameters named after
+the fields of mavd_detect_params (include/mavd.h).  Their defaults are the reference's constants, and a non-default
+value is the reference's expression with that value written in place of the literal.  Pass them as Python floats,
+never as np.float64: NumPy follows NEP 50, so a Python float combined with a float32 array is taken as float32
+(`np.array([2.4], np.float32) < 2.4` is False, `0.5 + 7.7 / mag` stays float32), which is what the reference does on
+its float32 frame (frame_index < 1).  An np.float64 scalar would promote that frame to float64 and change what is
+computed.  The segmentation metrics (`simple_bounding_box`, `tpr_fpr`) take graded uint8 masks as the reference does.
 """
 from __future__ import annotations
 
@@ -89,8 +97,9 @@ def ransac(E: np.ndarray, ransac_threshold: float = 30.0) -> Tuple[float, float]
     return best
 
 
-def foe_dense(flow: np.ndarray, ry: np.ndarray, rx: np.ndarray) -> Tuple[float, float]:
-    return ransac(intersections(flow, ry, rx))
+def foe_dense(flow: np.ndarray, ry: np.ndarray, rx: np.ndarray, magnitude_threshold: float = 2.5,
+              ransac_threshold: float = 30.0) -> Tuple[float, float]:
+    return ransac(intersections(flow, ry, rx, magnitude_threshold), ransac_threshold)
 
 
 def get_phi(flow: np.ndarray, foe: Tuple[float, float], cr_arccos_f32: bool = False) -> np.ndarray:
@@ -119,15 +128,17 @@ def get_phi(flow: np.ndarray, foe: Tuple[float, float], cr_arccos_f32: bool = Fa
     return np.rad2deg(ang)
 
 
-def masks(flow_derot: np.ndarray, phi: np.ndarray, sky: np.ndarray) -> Tuple[np.ndarray, np.ndarray]:
-    """processor.py:307,333-341 -> (total_mask, estimate_fixed), both bool."""
+def masks(flow_derot: np.ndarray, phi: np.ndarray, sky: np.ndarray, dyn_offset: float = 0.25, dyn_base: float = 0.5,
+          dyn_gain: float = 8.0, dyn_min_mag: float = 0.5, fixed_min_mag: float = 1.0,
+          fixed_angle: float = 15.0) -> Tuple[np.ndarray, np.ndarray]:
+    """processor.py:307,333-341 -> (total_mask, estimate_fixed), both bool.  Defaults: the reference's literals."""
     mag = np.linalg.norm(flow_derot, axis=-1)
-    with np.errstate(divide='ignore'):
-        t = 0.5 + 8 / mag
-    amax = phi > (0.25 + t)
-    amin = phi < (0.25 - t)
-    total = (mag > 0.5) * ~sky * np.logical_or(amin, amax)
-    fixed = phi * (mag > 1.0) * ~sky > 15
+    with np.errstate(divide='ignore', invalid='ignore'):
+        t = dyn_base + dyn_gain / mag
+        amax = phi > (dyn_offset + t)
+        amin = phi < (dyn_offset - t)
+        total = (mag > dyn_min_mag) * ~sky * np.logical_or(amin, amax)
+        fixed = phi * (mag > fixed_min_mag) * ~sky > fixed_angle
     return total, fixed
 
 
@@ -143,22 +154,30 @@ def simple_bounding_box(img: np.ndarray) -> Tuple[int, int, int, int]:
     return (int(cols[0]), int(rows[0]), int(cols[-1]), int(rows[-1]))
 
 
+def metric_counts(gt: np.ndarray, mask: np.ndarray) -> Tuple[int, int, int, int]:
+    """The four sums of im_helpers.py:244-252 with img = 255*mask (processor.py:350-351): (positives, negatives,
+    true positives, false positives) for a uint8 segmentation gt."""
+    img = 255 * mask
+    p = np.sum(gt > 127)
+    n = np.sum((255 - gt) > 127)
+    tp = np.sum((gt * img) > 127)
+    fp = np.sum(((255 - gt) * img) > 127)
+    return p, n, tp, fp
+
+
 def tpr_fpr(gt: np.ndarray, mask: np.ndarray) -> Tuple[float, float]:
     """im_helpers.py:244-252 with img = 255*mask (processor.py:350-351)."""
-    img = 255 * mask
+    p, n, tp, fp = metric_counts(gt, mask)
     with np.errstate(divide='ignore', invalid='ignore'):
-        p = np.sum(gt > 127)
-        n = np.sum((255 - gt) > 127)
-        tp = np.sum((gt * img) > 127)
-        fp = np.sum(((255 - gt) * img) > 127)
         return (tp / p, fp / n)
 
 
 def frame_pipeline(frame_index: int, flow_uv: np.ndarray, ang_diff, dt: float, sky: np.ndarray,
-                   ry: np.ndarray, rx: np.ndarray, cr_arccos_f32: bool = False):
-    """processor.py:305-341 for one frame given pre-drawn sample indices."""
+                   ry: np.ndarray, rx: np.ndarray, cr_arccos_f32: bool = False, magnitude_threshold: float = 2.5,
+                   ransac_threshold: float = 30.0, **mask_params):
+    """processor.py:305-341 for one frame given pre-drawn sample indices.  mask_params: the keywords of masks()."""
     fd = derotate(frame_index, flow_uv, ang_diff, dt)
-    foe = foe_dense(fd, ry, rx)
+    foe = foe_dense(fd, ry, rx, magnitude_threshold, ransac_threshold)
     phi = get_phi(fd, foe, cr_arccos_f32)
-    total, fixed = masks(fd, phi, sky)
+    total, fixed = masks(fd, phi, sky, **mask_params)
     return fd, foe, phi, total, fixed
