@@ -9,7 +9,7 @@ from typing import Optional
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, 'csrc', 'libmavd.so')
 
-ABI_VERSION = 2
+ABI_VERSION = 3
 MAVD_OK, MAVD_ERR_INVALID, MAVD_ERR_CUDA, MAVD_ERR_UNSUPPORTED, MAVD_ERR_NOMEM = 0, 1, 2, 3, 4
 N_SAMPLE_PAIRS = 1000
 SAMPLES_PER_FRAME = 4 * N_SAMPLE_PAIRS
@@ -53,11 +53,9 @@ class FrameRecord(C.Structure):
 
 class Tuning(C.Structure):
     """Launch-shape choices (include/mavd.h: mavd_tuning); results never depend on them."""
-    _fields_ = [('overlap', C.c_int32), ('pair_group', C.c_int32), ('r1_staged', C.c_int32), ('iter_fuse', C.c_int32),
-                ('last_fused', C.c_int32), ('mat_coord', C.c_int32), ('mat_r0_first', C.c_int32),
-                ('mat_txlog', C.c_int32), ('pyr_staged', C.c_int32), ('use_graph', C.c_int32),
+    _fields_ = [('mat_coord', C.c_int32), ('pyr_staged', C.c_int32), ('use_graph', C.c_int32),
                 ('polyexp_tma', C.c_int32), ('iter_small_tiles', C.c_int32), ('use_pdl', C.c_int32),
-                ('pyr_sweep', C.c_int32), ('pyr_fuse_h1', C.c_int32), ('reserved', C.c_int32 * 1)]
+                ('pyr_sweep', C.c_int32), ('reserved', C.c_int32 * 1)]
 
 
 class AuxInputs(C.Structure):

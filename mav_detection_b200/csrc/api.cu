@@ -500,28 +500,18 @@ int mavd_destroy(mavd_handle h) {
 void mavd_default_tuning(mavd_tuning* t) {
     if (!t) return;
     memset(t, 0, sizeof(*t));
-    t->overlap = 3;
-    t->pair_group = 4;
-    t->r1_staged = 1;
-    t->iter_fuse = 1;
-    t->last_fused = 1;
     t->mat_coord = 0;
-    t->mat_r0_first = 1;
-    t->mat_txlog = 6;
     t->pyr_staged = 1;
     t->use_graph = 1;
     t->polyexp_tma = 1;
     t->iter_small_tiles = 1;
     t->use_pdl = 1;
     t->pyr_sweep = 1;
-    t->pyr_fuse_h1 = 1;
 }
 
 int mavd_set_tuning(mavd_handle h, const mavd_tuning* t) {
     MAVD_REQUIRE(h && t, MAVD_ERR_INVALID, "set_tuning: NULL argument");
-    MAVD_REQUIRE(t->overlap >= 0 && t->overlap <= 3 && t->pair_group >= 1 && t->mat_coord >= 0 && t->mat_coord <= 2 &&
-                     t->mat_txlog >= 4 && t->mat_txlog <= 8 && t->iter_fuse >= 0 && t->iter_fuse <= 1,
-                 MAVD_ERR_INVALID, "set_tuning: value out of range");
+    MAVD_REQUIRE(t->mat_coord >= 0 && t->mat_coord <= 2, MAVD_ERR_INVALID, "set_tuning: value out of range");
     DeviceGuard dg(h->cfg.device);
     MAVD_CUDA(cudaDeviceSynchronize());
     drop_graphs(h);
@@ -828,7 +818,7 @@ static int detect_run(mavd_handle h, const float* flow, int n, const mavd_detect
     char* stats0 = reinterpret_cast<char*>(d_records) + offsetof(mavd_frame_record, stats);
     // FoE estimation is one CTA per frame; what the residual kernel needs besides the FoE (zeroed statistics, the
     // segmentation maxima, an empty unit list) does not depend on it and runs on the side stream meanwhile
-    const bool fork = h->s_aux != nullptr && h->tune.overlap >= 3 && !h->prof.on;
+    const bool fork = h->s_aux != nullptr && !h->prof.on;
     if (fork) {
         MAVD_CUDA(cudaEventRecord(h->ev_fork, s));
         MAVD_CUDA(cudaStreamWaitEvent(h->s_aux, h->ev_fork, 0));

@@ -224,7 +224,7 @@ __global__ void __launch_bounds__(256) pyr_hsecond_staged_kernel(int W, int Wp, 
 //                window streamed as float4 groups (the staged generic kernel spends 600 instructions per output on
 //                copying spans into shared memory)
 // Per output sample the products are accumulated in the same tap order with the same FMAs as in the generic kernels:
-// the images are bit-identical (test_pyramid_sweep_is_bit_identical).
+// the images are bit-identical (test_pyramid_sweep_equals_the_generic_kernels).
 // ------------------------------------------------------------------------------------------------
 struct HalfPyr {    // level l = 1..6: stride, taps, -(window start of output 0), live outputs per source row
     __host__ __device__ static constexpr int S(int l) { return 1 << l; }
@@ -750,6 +750,8 @@ __device__ __forceinline__ void resize_coord_pow2(int d, float scale, int src, i
     i0 = s;
 }
 
+constexpr int MI_TX = 64, MI_TY = 4;   // matrices_init_kernel block: 64 x 4 pixels
+
 template <int COORD>
 __global__ void __launch_bounds__(256, 8) matrices_init_kernel(const float* __restrict__ R, size_t plane, int w, int h,
                                                            int pitch, size_t R_pair_stride,
@@ -759,19 +761,20 @@ __global__ void __launch_bounds__(256, 8) matrices_init_kernel(const float* __re
                                                            const float* __restrict__ fxa,
                                                            const int* __restrict__ fyi0,
                                                            const float* __restrict__ fya, float up_scale,
-                                                           float* __restrict__ M, double xscale, double yscale,
-                                                           int txlog, int r0_first) {
+                                                           float* __restrict__ M, double xscale, double yscale, int r0_first) {
     pdl_entry();
     // 3-D grid (pairs, tiles_x, tiles_y): blocks are scheduled x-fastest, so the pair index is fastest (same L2 sharing
     // of R between consecutive pairs as in iter_box_tma_kernel) and no thread pays for an integer division: with one
     // pixel per thread the two divisions of a 1-D grid were 55 of the kernel's 400 instructions
-    // block = 2^txlog x 2^(8 - txlog) pixels (64 x 4 by default)
     const int p = blockIdx.x;
-    const int x = (blockIdx.y << txlog) + (threadIdx.x & ((1 << txlog) - 1));
-    const int y = (blockIdx.z << (8 - txlog)) + (threadIdx.x >> txlog);
+    const int x = blockIdx.y * MI_TX + (threadIdx.x & (MI_TX - 1));
+    const int y = blockIdx.z * MI_TY + threadIdx.x / MI_TX;
     if (x >= w || y >= h) return;
     // R0 does not depend on the flow: its five loads go out first and travel with the coarse-flow loads, so that the
-    // second memory round trip of the thread is the R1 gather alone
+    // second memory round trip of the thread is the R1 gather alone.  The host always passes r0_first = 1.  The order
+    // stays a run-time branch because the compile-time form (R0 loaded first, no second load site) is slower: 2.15 vs
+    // 2.05 ms per C2 step (B200, 1000 W).  With the order fixed, ptxas keeps the 64-bit pixel offset live from the R0
+    // loads to the M stores and issues the R1 gather in smaller groups.
     const float* R0 = R + (size_t)p * R_pair_stride;
     R0Px r0;
     if (r0_first) r0 = load_r0_px(R0, (size_t)y * pitch + x, plane);
@@ -816,6 +819,10 @@ __global__ void __launch_bounds__(256, 8) matrices_init_kernel(const float* __re
 // phase is per pixel with x fastest so R0 loads, the R1 gather and the M' stores are coalesced.
 // ------------------------------------------------------------------------------------------------
 constexpr int IT_TX = 64, IT_TY = 32;
+// Consecutive pairs share an R plane (R1 of pair p is R0 of pair p+1): iter_box_tma_kernel interleaves the pairs of a
+// tile in groups of 4 in its CTA order so that the second reader hits L2 (4502 vs 4441 pairs/s ungrouped, 4338 with the
+// whole 64-pair batch interleaved: too many concurrent HBM regions).
+constexpr int IT_PAIR_GROUP = 4;
 
 struct IterArgs {
     const float* Min;
@@ -832,8 +839,6 @@ struct IterArgs {
     int pair_stride;
     const float* gk;        // Gaussian half kernel [m+1] (device) or nullptr
     int n_pairs, tiles_x;   // TMA kernel: 1-D grid (see iter_box_tma_kernel)
-    int group;              // pairs interleaved per tile in the 1-D grid order
-    int last_fused;         // TMA kernel, last iteration: horizontal sums + solve in registers (a.flow must be set)
 };
 
 template <int M_>
@@ -1020,12 +1025,12 @@ __global__ void __launch_bounds__(256, 3) iter_kernel(IterArgs a) {
 // tile plus halo — into shared memory; everything after that happens IN PLACE in that box:
 //   vertical   thread = (plane, column): running 2m+1 sum marching down the column, window in
 //              registers, the sum for row y overwrites row y after its input has been consumed
-//   horizontal half-warp = one row: 4 outputs per thread from 5 float4 reads, written back over
-//              columns 8..71 after a __syncwarp (rows are private to a half-warp)
-//   pixel      x-fastest mapping: 2x2 solve into registers; then a SECOND TMA load puts the five R1 planes
-//              around the tile (displaced by the tile centre's flow) into the same box, and UpdateMatrices
-//              gathers from shared memory (global fallback for footprints outside the box), with
-//              coalesced R0 loads and M' stores
+//   horizontal thread = 4 adjacent pixels of one row: the five planes' sums from 5 float4 reads each and
+//              the 2x2 solve, in registers
+//   pixel      (not the last iteration) the flow vectors pass through shared memory to an x-fastest mapping;
+//              then a SECOND TMA load puts the five R1 planes around the tile (displaced by the tile centre's
+//              flow) into the same box, and UpdateMatrices gathers from shared memory (global fallback for
+//              footprints outside the box), with coalesced R0 loads and M' stores
 // Out-of-image box cells arrive as zeros (TMA fill) and are overwritten with the replicated edge
 // values for border tiles only.
 // ------------------------------------------------------------------------------------------------
@@ -1170,61 +1175,9 @@ __global__ void __launch_bounds__(256, 4) polyexp_tma_kernel(const __grid_consta
     polyexp_passes<N_>(raw0 - (PE_H - n) * PE_RW, t, pc, n, tid, x0, y0, h, pitch, R + (size_t)blockIdx.z * 5 * plane, plane);
 }
 
-// UpdateMatrices with 32-bit index arithmetic; `edge` is tile-uniform (tile within 5 px of a border).
-__device__ __forceinline__ void update_matrices_fast(int x, int y, int w, int h, int pitch, int plane, bool edge,
-                                                     float dx, float dy, const float* __restrict__ R0,
-                                                     const float* __restrict__ R1, float* __restrict__ Mout) {
-    // every address is base + one 32-bit element index: one IMAD.WIDE per address instead of 64-bit add chains
-    const int o = y * pitch + x;
-    const float r0y = __ldg(R0 + o), r0x = __ldg(R0 + (o + plane)), r0yy = __ldg(R0 + (o + 2 * plane)),
-                r0xx = __ldg(R0 + (o + 3 * plane)), r0xy = __ldg(R0 + (o + 4 * plane));
-    float fx = (float)x + dx, fy = (float)y + dy;
-    const float flx = floorf(fx), fly = floorf(fy);
-    const int x1 = (int)fminf(fmaxf(flx, -2.f), 1.0e6f), y1 = (int)fminf(fmaxf(fly, -2.f), 1.0e6f);
-    fx -= flx;
-    fy -= fly;
-    float r2, r3, r4, r5, r6;
-    if ((unsigned)x1 < (unsigned)(w - 1) && (unsigned)y1 < (unsigned)(h - 1)) {
-        const float gx = 1.f - fx, gy = 1.f - fy;
-        const float a00 = gx * gy, a01 = fx * gy, a10 = gx * fy, a11 = fx * fy;
-        const int q0 = y1 * pitch + x1, q1 = q0 + pitch;
-        r2 = a00 * __ldg(R1 + q0) + a01 * __ldg(R1 + q0 + 1) + a10 * __ldg(R1 + q1) + a11 * __ldg(R1 + q1 + 1);
-        r3 = a00 * __ldg(R1 + (q0 + plane)) + a01 * __ldg(R1 + (q0 + plane) + 1) + a10 * __ldg(R1 + (q1 + plane)) +
-             a11 * __ldg(R1 + (q1 + plane) + 1);
-        r4 = a00 * __ldg(R1 + (q0 + 2 * plane)) + a01 * __ldg(R1 + (q0 + 2 * plane) + 1) +
-             a10 * __ldg(R1 + (q1 + 2 * plane)) + a11 * __ldg(R1 + (q1 + 2 * plane) + 1);
-        r5 = a00 * __ldg(R1 + (q0 + 3 * plane)) + a01 * __ldg(R1 + (q0 + 3 * plane) + 1) +
-             a10 * __ldg(R1 + (q1 + 3 * plane)) + a11 * __ldg(R1 + (q1 + 3 * plane) + 1);
-        r6 = a00 * __ldg(R1 + (q0 + 4 * plane)) + a01 * __ldg(R1 + (q0 + 4 * plane) + 1) +
-             a10 * __ldg(R1 + (q1 + 4 * plane)) + a11 * __ldg(R1 + (q1 + 4 * plane) + 1);
-        r4 = (r0yy + r4) * 0.5f;
-        r5 = (r0xx + r5) * 0.5f;
-        r6 = (r0xy + r6) * 0.25f;
-    } else {
-        r2 = r3 = 0.f;
-        r4 = r0yy;
-        r5 = r0xx;
-        r6 = r0xy * 0.5f;
-    }
-    r2 = (r0y - r2) * 0.5f;
-    r3 = (r0x - r3) * 0.5f;
-    r2 += r4 * dy + r6 * dx;
-    r3 += r6 * dy + r5 * dx;
-    if (edge && ((unsigned)(x - 5) >= (unsigned)(w - 10) || (unsigned)(y - 5) >= (unsigned)(h - 10))) {
-        const float sc = (x < 5 ? border_factor(x) : 1.f) * (x >= w - 5 ? border_factor(w - x - 1) : 1.f) *
-                         (y < 5 ? border_factor(y) : 1.f) * (y >= h - 5 ? border_factor(h - y - 1) : 1.f);
-        r2 *= sc; r3 *= sc; r4 *= sc; r5 *= sc; r6 *= sc;
-    }
-    Mout[o] = r4 * r4 + r6 * r6;
-    Mout[o + plane] = (r4 + r5) * r6;
-    Mout[o + 2 * plane] = r5 * r5 + r6 * r6;
-    Mout[o + 3 * plane] = r4 * r2 + r6 * r3;
-    Mout[o + 4 * plane] = r6 * r2 + r5 * r3;
-}
-
 // UpdateMatrices with the R1 footprint read from a shared-memory box [5][RH][RW] whose cell (0, 0) is image pixel
-// (bx, by); footprints that leave the box fall back to global loads.  Same operations, same order as
-// update_matrices_fast: identical results.
+// (bx, by); footprints that leave the box fall back to global loads.  `edge` is tile-uniform (tile within 5 px of a
+// border).  Same operations, same order as update_matrices_px (the generic iter_kernel's): identical results.
 
 __device__ __forceinline__ R0Px load_r0(const float* __restrict__ R0, unsigned o, unsigned plane) {
     R0Px r;
@@ -1294,23 +1247,25 @@ __device__ __forceinline__ void update_matrices_box(int x, int y, int w, int h, 
     st_global_f32(Mout + (o + 4 * plane), r6 * r2 + r5 * r3);
 }
 
-// FUSE (not-last iterations with R1S; default, MAVD_ITER_FUSE=0 selects the staged form): the horizontal sums and the
-// solve are done in registers as in the last iteration and the flow vectors, not the five sums, go through shared
-// memory to reach the x-fastest pixel mapping of the update phase (640 -> 256 wavefronts per tile for that hand-over,
-// one more barrier; same hsum_box, same solve expressions: identical results).  (A variant that parked the flow vectors
-// in the dead raw rows below the vertical sums to save that barrier measured 0.5 % slower and was removed.)
+// Not-last iterations: the horizontal sums and the solve are done in registers as in the last iteration and the flow
+// vectors, not the five sums, go through shared memory to reach the x-fastest pixel mapping of the update phase (640 ->
+// 256 wavefronts per tile for that hand-over, one more barrier: 4.27 vs 4.39 ms per 64-pair step against writing the
+// sums back to the box; same hsum_box, same solve expressions: identical results).  (A variant that parked the flow
+// vectors in the dead raw rows below the vertical sums to save that barrier measured 0.5 % slower and was removed.)
+// R1 is staged in shared memory by the second TMA load: 4.36 vs 4.56 ms per 64-pair step against gathering it from
+// global memory.
 // TY: tile height, 32 by default; 16 for launches whose 32-row tiling would leave SMs idle (single pairs, the coarse
 // levels): twice the CTAs, half the serial work per CTA.  The vertical sums are re-seeded at absolute rows that are
 // multiples of 8 in both tilings and the horizontal groups start at multiples of 4: the results are bit-identical.
 // GAUSS: OPTFLOW_FARNEBACK_GAUSSIAN windows (FarnebackUpdateFlow_GaussianBlur): the vertical pass is the 2m+1-tap
 // filter on the same register window (in place, like the running sums), the horizontal one hsum_gauss; both with the
 // generic kernel's expressions, so the two kernels stay bit-identical.
-template <int M_, bool LAST, int NT, bool R1S, int FUSE = 0, int TY = IT_TY, bool GAUSS = false>
-__global__ void __launch_bounds__(NT, NT == 256 ? 3 : 2) iter_box_tma_kernel(const __grid_constant__ CUtensorMap tmap,
-                                                                             const __grid_constant__ CUtensorMap tmapR,
-                                                                             const __grid_constant__ CUtensorMap tmapRbox,
-                                                                             IterArgs a) {
+template <int M_, bool LAST, int TY, bool GAUSS>
+__global__ void __launch_bounds__(256, 3) iter_box_tma_kernel(const __grid_constant__ CUtensorMap tmap,
+                                                              const __grid_constant__ CUtensorMap tmapR,
+                                                              const __grid_constant__ CUtensorMap tmapRbox, IterArgs a) {
     pdl_entry();
+    constexpr int NT = 256;                 // threads
     constexpr int RW = IT_TX + 16;          // 80 staged columns (halo 8 each side, 16-byte aligned)
     constexpr int RH = TY + 2 * M_;      // staged rows
     constexpr int CH = RH * RW;             // floats per plane box
@@ -1323,18 +1278,18 @@ __global__ void __launch_bounds__(NT, NT == 256 ? 3 : 2) iter_box_tma_kernel(con
     // pairs, and R1 of pair p is R0 of pair p+1 (sequence mode), so every R plane is fetched from HBM once and
     // served to its second reader from L2
     // (the last iteration reads no R: it keeps tile-fastest order, which is better for the M halo reuse)
-    // pairs are interleaved in groups of a.group (not the whole batch: too many concurrent HBM regions otherwise)
+    // pairs are interleaved in groups of IT_PAIR_GROUP
     const int n_tiles = gridDim.x / a.n_pairs;
     int p, tile;
     if (LAST) {
         p = blockIdx.x / n_tiles;
         tile = blockIdx.x - p * n_tiles;
     } else {
-        const int per_group = a.group * n_tiles;
+        const int per_group = IT_PAIR_GROUP * n_tiles;
         const int gidx = blockIdx.x / per_group, rem = blockIdx.x - gidx * per_group;
-        const int gsize = min(a.group, a.n_pairs - gidx * a.group);     // the last group may be short
+        const int gsize = min(IT_PAIR_GROUP, a.n_pairs - gidx * IT_PAIR_GROUP);     // the last group may be short
         tile = rem / gsize;
-        p = gidx * a.group + (rem - tile * gsize);
+        p = gidx * IT_PAIR_GROUP + (rem - tile * gsize);
     }
     const int x0 = (tile % a.tiles_x) * IT_TX, y0 = (tile / a.tiles_x) * TY;
     const int w = a.w, h = a.h, pitch = a.pitch;
@@ -1439,11 +1394,10 @@ __global__ void __launch_bounds__(NT, NT == 256 ? 3 : 2) iter_box_tma_kernel(con
     }
     __syncthreads();
 
-    if (LAST && a.last_fused) {
+    if (LAST) {
         // ---- last iteration: horizontal sums of the five planes and the 2x2 solve in registers ----
         // thread = 4 adjacent pixels of one row: no sums are written back to shared memory, no third barrier, and the
-        // flow leaves as two 16-byte stores (same hsum_box / same solve expressions: results identical to the
-        // staged form below)
+        // flow leaves as two 16-byte stores
         const int q4 = tid & 15, rsub = tid >> 4;
         constexpr int ROWS_PER_IT = NT / 16;
         float2* fl = a.flow + (size_t)p * a.flow_stride;
@@ -1490,159 +1444,105 @@ __global__ void __launch_bounds__(NT, NT == 256 ? 3 : 2) iter_box_tma_kernel(con
         return;
     }
 
-    // ---- horizontal sums, in place: half-warp = one row, thread = 4 outputs ----
-    if (!(FUSE && R1S && !LAST)) {
-        const int q4 = tid & 15, rsub = tid >> 4;
-        constexpr int ROWS_PER_IT = NT / 16;
-#pragma unroll 2
-        for (int it = 0; it < (5 * TY) / ROWS_PER_IT; ++it) {
-            const int task = it * ROWS_PER_IT + rsub;
-            const int c = task / TY, r = task - c * TY;
-            float* row = box + c * CH + r * RW + 4 * q4;
-            float u[20];
-#pragma unroll
-            for (int j = 0; j < 5; ++j) {
-                const float4 v = *reinterpret_cast<const float4*>(row + 4 * j);
-                u[4 * j] = v.x; u[4 * j + 1] = v.y; u[4 * j + 2] = v.z; u[4 * j + 3] = v.w;
-            }
-            float o[4];
-            hsum(u, o);
-            __syncwarp();
-            *reinterpret_cast<float4*>(row + 8) = make_float4(o[0], o[1], o[2], o[3]);
-        }
-        __syncthreads();
-    }
-
-    // ---- per pixel: solve, then UpdateMatrices ----
+    // ---- per pixel: solve, then UpdateMatrices with R1 through shared memory ----
+    // (a) every thread turns the sums of its pixels into flow vectors (registers) and the box is free again;
+    // (b) ONE TMA load brings the 5 planes of R1 around the tile, displaced by the flow of the tile centre,
+    //     into the box; (c) the bilinear gather reads shared memory with immediate offsets (one base address per
+    //     pixel, ~30-cycle latency) instead of 20 global loads.  Pixels whose footprint leaves the box (flow
+    //     differs from the centre's by more than ~5 px) take the global path; values are identical either way.
     const float* R0 = a.R + (size_t)(p * a.pair_stride) * 5 * a.plane;
     const float* R1 = R0 + 5 * a.plane;
-    float* Mout = LAST ? nullptr : a.Mout + (size_t)p * 5 * a.plane;
+    float* Mout = a.Mout + (size_t)p * 5 * a.plane;
     // keep the pair's M' base as ONE 64-bit register pair: the compiler otherwise carries (kernel argument + 64-bit
     // element offset) and rebuilds every store address with a 4-instruction add / shift chain instead of one
     // IMAD.WIDE.U32 on the 32-bit element offset
     asm volatile("" : "+l"(Mout));
-    float2* fl = a.flow ? a.flow + (size_t)p * a.flow_stride : nullptr;
     const bool edge = (x0 < 5) || (y0 < 5) || (x0 + IT_TX > w - 5) || (y0 + TY > h - 5);
     const float scale = a.scale;
-    if (R1S && !LAST) {
-        // ---- R1 through shared memory ----
-        // (a) every thread turns the sums of its pixels into flow vectors (registers) and the box is free again;
-        // (b) ONE TMA load brings the 5 planes of R1 around the tile, displaced by the flow of the tile centre,
-        //     into the box; (c) the bilinear gather reads shared memory with immediate offsets (one base address per
-        //     pixel, ~30-cycle latency) instead of 20 global loads.  Pixels whose footprint leaves the box (flow
-        //     differs from the centre's by more than ~5 px) take the global path; values are identical either way.
-        constexpr int PPT = (IT_TX * TY) / NT;
-        __shared__ int s_org[2];
-        float ffx[PPT], ffy[PPT];
-        if (FUSE) {
-            // (a0) horizontal sums of the five planes + solve for 4 adjacent pixels per task, in registers
-            static_assert(!FUSE || (NT == 256 && TY % 16 == 0), "FUSE assumes 16 rows per pass");
-            const int q4 = tid & 15, rsub = tid >> 4;
-            constexpr int NPASS = TY / 16;
-            float4 gx[NPASS], gy[NPASS];
+    constexpr int PPT = (IT_TX * TY) / NT;
+    __shared__ int s_org[2];
+    float ffx[PPT], ffy[PPT];
+    {
+        // (a0) horizontal sums of the five planes + solve for 4 adjacent pixels per task, in registers
+        static_assert(TY % 16 == 0, "16 rows per pass");
+        const int q4 = tid & 15, rsub = tid >> 4;
+        constexpr int NPASS = TY / 16;
+        float4 gx[NPASS], gy[NPASS];
 #pragma unroll
-            for (int it = 0; it < NPASS; ++it) {
-                const int r = it * 16 + rsub;
-                float o[5][4];
+        for (int it = 0; it < NPASS; ++it) {
+            const int r = it * 16 + rsub;
+            float o[5][4];
 #pragma unroll
-                for (int c = 0; c < 5; ++c) {
-                    const float* row = box + c * CH + r * RW + 4 * q4;
-                    float u[20];
+            for (int c = 0; c < 5; ++c) {
+                const float* row = box + c * CH + r * RW + 4 * q4;
+                float u[20];
 #pragma unroll
-                    for (int j = 0; j < 5; ++j) {
-                        const float4 v = *reinterpret_cast<const float4*>(row + 4 * j);
-                        u[4 * j] = v.x; u[4 * j + 1] = v.y; u[4 * j + 2] = v.z; u[4 * j + 3] = v.w;
-                    }
-                    hsum(u, o[c]);
+                for (int j = 0; j < 5; ++j) {
+                    const float4 v = *reinterpret_cast<const float4*>(row + 4 * j);
+                    u[4 * j] = v.x; u[4 * j + 1] = v.y; u[4 * j + 2] = v.z; u[4 * j + 3] = v.w;
                 }
-                float fx4[4], fy4[4];
-#pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                    const float g11 = o[0][k] * scale, g12 = o[1][k] * scale, g22 = o[2][k] * scale,
-                                h1 = o[3][k] * scale, h2 = o[4][k] * scale;
-                    const float idet = __frcp_rn(g11 * g22 - g12 * g12 + 1e-3f);
-                    fx4[k] = (g11 * h2 - g12 * h1) * idet;
-                    fy4[k] = (g22 * h1 - g12 * h2) * idet;
-                }
-                gx[it] = make_float4(fx4[0], fx4[1], fx4[2], fx4[3]);
-                gy[it] = make_float4(fy4[0], fy4[1], fy4[2], fy4[3]);
+                hsum(u, o[c]);
             }
-            {
-                __syncthreads();                   // every vertical sum has been consumed: the box is free
-                // (a1) the flow vectors through shared memory: [2][32][64] floats at the start of the box
+            float fx4[4], fy4[4];
 #pragma unroll
-                for (int it = 0; it < NPASS; ++it) {
-                    const int o4 = (it * 16 + rsub) * IT_TX + 4 * q4;
-                    *reinterpret_cast<float4*>(box + o4) = gx[it];
-                    *reinterpret_cast<float4*>(box + IT_TX * TY + o4) = gy[it];
-                }
-            }
-            __syncthreads();
-        }
-#pragma unroll
-        for (int j = 0; j < PPT; ++j) {
-            const int idx = j * NT + tid;
-            const int cx = idx & 63, r = idx >> 6;
-            if (FUSE) {
-                ffx[j] = box[idx];
-                ffy[j] = box[IT_TX * TY + idx];
-            } else {
-                const float* sp = box + r * RW + 8 + cx;
-                const float g11 = sp[0] * scale, g12 = sp[CH] * scale, g22 = sp[2 * CH] * scale, h1 = sp[3 * CH] * scale,
-                            h2 = sp[4 * CH] * scale;
+            for (int k = 0; k < 4; ++k) {
+                const float g11 = o[0][k] * scale, g12 = o[1][k] * scale, g22 = o[2][k] * scale,
+                            h1 = o[3][k] * scale, h2 = o[4][k] * scale;
                 const float idet = __frcp_rn(g11 * g22 - g12 * g12 + 1e-3f);
-                ffx[j] = (g11 * h2 - g12 * h1) * idet;
-                ffy[j] = (g22 * h1 - g12 * h2) * idet;
+                fx4[k] = (g11 * h2 - g12 * h1) * idet;
+                fy4[k] = (g22 * h1 - g12 * h2) * idet;
             }
-            if (cx == IT_TX / 2 && r == TY / 2) {
-                // box origin: tile origin displaced by the centre pixel's flow, x a multiple of 4
-                const float cfx = fminf(fmaxf(ffx[j], -1.0e5f), 1.0e5f), cfy = fminf(fmaxf(ffy[j], -1.0e5f), 1.0e5f);
-                s_org[0] = ((x0 + (int)floorf(cfx == cfx ? cfx : 0.f)) & ~3) - 8;
-                s_org[1] = y0 + (int)floorf(cfy == cfy ? cfy : 0.f) - M_;
-            }
+            gx[it] = make_float4(fx4[0], fx4[1], fx4[2], fx4[3]);
+            gy[it] = make_float4(fy4[0], fy4[1], fy4[2], fy4[3]);
         }
-        __syncthreads();                       // all sums consumed, origin published
-        const int bx = s_org[0], by = s_org[1];
-        if (tid == 0) {
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy reads before the async write
-            mbar_expect_tx(&bar, 5 * CH * (uint32_t)sizeof(float));
-            tma_load_3d(box, &tmapRbox, bx, by, (p * a.pair_stride + 1) * 5, &bar);
-        }
-        // R0 of the first pixel is requested before waiting for the box, and R0 of pixel j + 1 while pixel j is being
-        // worked on: the (L2-prefetched) loads are never waited for
-        const int cxp = tid & 63, xp = x0 + cxp;
-        const bool col_ok = xp < w;
-        auto r0_of = [&](int j) {
-            const int y = y0 + ((j * NT + tid) >> 6);
-            return (col_ok && y < h) ? load_r0(R0, (unsigned)(y * pitch + xp), (unsigned)plane) : R0Px{0.f, 0.f, 0.f, 0.f, 0.f};
-        };
-        R0Px cur = r0_of(0);
-        mbar_wait(&bar, 1);
+        __syncthreads();                       // every vertical sum has been consumed: the box is free
+        // (a1) the flow vectors through shared memory: [2][TY][64] floats at the start of the box
 #pragma unroll
-        for (int j = 0; j < PPT; ++j) {     // fully unrolled: ffx / ffy stay in registers
-            const int y = y0 + ((j * NT + tid) >> 6);
-            R0Px nxt = cur;
-            if (j + 1 < PPT) nxt = r0_of(j + 1);
-            if (col_ok && y < h)
-                update_matrices_box<RW, RH>(xp, y, w, h, pitch, (unsigned)plane, edge, ffx[j], ffy[j], cur, R1, Mout, box, bx, by);
-            cur = nxt;
+        for (int it = 0; it < NPASS; ++it) {
+            const int o4 = (it * 16 + rsub) * IT_TX + 4 * q4;
+            *reinterpret_cast<float4*>(box + o4) = gx[it];
+            *reinterpret_cast<float4*>(box + IT_TX * TY + o4) = gy[it];
         }
-        return;
+        __syncthreads();
     }
-#pragma unroll 2
-    for (int j = 0; j < (IT_TX * TY) / NT; ++j) {
+#pragma unroll
+    for (int j = 0; j < PPT; ++j) {
         const int idx = j * NT + tid;
         const int cx = idx & 63, r = idx >> 6;
-        const int x = x0 + cx, y = y0 + r;
-        if (x >= w || y >= h) continue;
-        const float* sp = box + r * RW + 8 + cx;
-        const float g11 = sp[0] * scale, g12 = sp[CH] * scale, g22 = sp[2 * CH] * scale, h1 = sp[3 * CH] * scale,
-                    h2 = sp[4 * CH] * scale;
-        const float idet = __frcp_rn(g11 * g22 - g12 * g12 + 1e-3f);   // MUFU.RCP + one Newton step, no slow-path call
-        const float fx = (g11 * h2 - g12 * h1) * idet;
-        const float fy = (g22 * h1 - g12 * h2) * idet;
-        if (fl) fl[y * a.flow_pitch + x] = make_float2(fx, fy);
-        if (!LAST) update_matrices_fast(x, y, w, h, pitch, plane, edge, fx, fy, R0, R1, Mout);
+        ffx[j] = box[idx];
+        ffy[j] = box[IT_TX * TY + idx];
+        if (cx == IT_TX / 2 && r == TY / 2) {
+            // box origin: tile origin displaced by the centre pixel's flow, x a multiple of 4
+            const float cfx = fminf(fmaxf(ffx[j], -1.0e5f), 1.0e5f), cfy = fminf(fmaxf(ffy[j], -1.0e5f), 1.0e5f);
+            s_org[0] = ((x0 + (int)floorf(cfx == cfx ? cfx : 0.f)) & ~3) - 8;
+            s_org[1] = y0 + (int)floorf(cfy == cfy ? cfy : 0.f) - M_;
+        }
+    }
+    __syncthreads();                           // all flow vectors read, origin published
+    const int bx = s_org[0], by = s_org[1];
+    if (tid == 0) {
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy reads before the async write
+        mbar_expect_tx(&bar, 5 * CH * (uint32_t)sizeof(float));
+        tma_load_3d(box, &tmapRbox, bx, by, (p * a.pair_stride + 1) * 5, &bar);
+    }
+    // R0 of the first pixel is requested before waiting for the box, and R0 of pixel j + 1 while pixel j is being
+    // worked on: the (L2-prefetched) loads are never waited for
+    const int cxp = tid & 63, xp = x0 + cxp;
+    const bool col_ok = xp < w;
+    auto r0_of = [&](int j) {
+        const int y = y0 + ((j * NT + tid) >> 6);
+        return (col_ok && y < h) ? load_r0(R0, (unsigned)(y * pitch + xp), (unsigned)plane) : R0Px{0.f, 0.f, 0.f, 0.f, 0.f};
+    };
+    R0Px cur = r0_of(0);
+    mbar_wait(&bar, 1);
+#pragma unroll
+    for (int j = 0; j < PPT; ++j) {         // fully unrolled: ffx / ffy stay in registers
+        const int y = y0 + ((j * NT + tid) >> 6);
+        R0Px nxt = cur;
+        if (j + 1 < PPT) nxt = r0_of(j + 1);
+        if (col_ok && y < h)
+            update_matrices_box<RW, RH>(xp, y, w, h, pitch, (unsigned)plane, edge, ffx[j], ffy[j], cur, R1, Mout, box, bx, by);
+        cur = nxt;
     }
 }
 
@@ -1672,67 +1572,30 @@ static int launch_iter(const IterArgs& a, dim3 grid, size_t smem, cudaStream_t s
     return MAVD_OK;
 }
 
-template <int M_, bool LAST, int NT, bool R1S, int FUSE = 0, int TY = IT_TY, bool GAUSS = false>
+template <int M_, bool LAST, int TY, bool GAUSS>
 static int launch_iter_tma(const CUtensorMap& map, const CUtensorMap& mapR, const CUtensorMap& mapRbox, const IterArgs& a,
                            dim3 grid, cudaStream_t s, bool pdl) {
     constexpr size_t smem = sizeof(float) * 5 * (TY + 2 * M_) * (IT_TX + 16);
-    MAVD_CUDA((ensure_dynamic_smem<iter_box_tma_kernel<M_, LAST, NT, R1S, FUSE, TY, GAUSS>>(smem)));
-    MAVD_CUDA(launch_chained(pdl, iter_box_tma_kernel<M_, LAST, NT, R1S, FUSE, TY, GAUSS>, grid, NT, smem, s, map, mapR,
-                             mapRbox, a));
+    MAVD_CUDA((ensure_dynamic_smem<iter_box_tma_kernel<M_, LAST, TY, GAUSS>>(smem)));
+    MAVD_CUDA(launch_chained(pdl, iter_box_tma_kernel<M_, LAST, TY, GAUSS>, grid, 256, smem, s, map, mapR, mapRbox, a));
     MAVD_LAUNCHED();
     return MAVD_OK;
 }
 
+// 5 <= m <= 8; with small_tiles the caller built `grid` and the descriptors for 64 x 16 tiles
 template <bool LAST>
-static int launch_iter_tma_m(int m, const mavd_tuning& tune, bool small_tiles, const CUtensorMap& map,
-                             const CUtensorMap& mapR, const CUtensorMap& mapRbox, const IterArgs& a, dim3 grid,
-                             cudaStream_t s, bool pdl) {
-    // R1 staged in shared memory by a second TMA load: 4.36 vs 4.56 ms per 64-pair step (tuning.r1_staged)
-    const bool r1s = tune.r1_staged != 0;
-    // horizontal sums + solve in registers for the not-last iterations too, flow vectors handed to the update phase
-    // through shared memory: iter_full 4.27 vs 4.39 ms per 64-pair step (tuning.iter_fuse)
-    const int fuse = tune.iter_fuse;
-    if (a.gk != nullptr) {  // Gaussian windows: production variants only (the caller checked the tuning), both tile heights
-#define GAUSS_CASE(M)                                                                                                        \
-        case M: return small_tiles ? launch_iter_tma<M, LAST, 256, !LAST, LAST ? 0 : 1, 16, true>(map, mapR, mapRbox, a, grid, s, pdl) \
-                                   : launch_iter_tma<M, LAST, 256, !LAST, LAST ? 0 : 1, IT_TY, true>(map, mapR, mapRbox, a, grid, s, pdl);
-        switch (m) {
-            GAUSS_CASE(5) GAUSS_CASE(6) GAUSS_CASE(7)
-            default: return small_tiles ? launch_iter_tma<8, LAST, 256, !LAST, LAST ? 0 : 1, 16, true>(map, mapR, mapRbox, a, grid, s, pdl)
-                                        : launch_iter_tma<8, LAST, 256, !LAST, LAST ? 0 : 1, IT_TY, true>(map, mapR, mapRbox, a, grid, s, pdl);
-        }
-#undef GAUSS_CASE
-    }
-    if (small_tiles) {      // 64 x 16 tiles (the caller built `grid` and the descriptors for them): production variants only
-        switch (m) {
-            case 5: return launch_iter_tma<5, LAST, 256, !LAST, LAST ? 0 : 1, 16>(map, mapR, mapRbox, a, grid, s, pdl);
-            case 6: return launch_iter_tma<6, LAST, 256, !LAST, LAST ? 0 : 1, 16>(map, mapR, mapRbox, a, grid, s, pdl);
-            case 7: return launch_iter_tma<7, LAST, 256, !LAST, LAST ? 0 : 1, 16>(map, mapR, mapRbox, a, grid, s, pdl);
-            default: return launch_iter_tma<8, LAST, 256, !LAST, LAST ? 0 : 1, 16>(map, mapR, mapRbox, a, grid, s, pdl);
-        }
-    }
-    if (r1s && !LAST && fuse != 0) {
-        switch (m) {
-            case 5: return launch_iter_tma<5, false, 256, true, 1>(map, mapR, mapRbox, a, grid, s, pdl);
-            case 6: return launch_iter_tma<6, false, 256, true, 1>(map, mapR, mapRbox, a, grid, s, pdl);
-            case 7: return launch_iter_tma<7, false, 256, true, 1>(map, mapR, mapRbox, a, grid, s, pdl);
-            default: return launch_iter_tma<8, false, 256, true, 1>(map, mapR, mapRbox, a, grid, s, pdl);
-        }
-    }
-    if (r1s && !LAST) {
-        switch (m) {
-            case 5: return launch_iter_tma<5, LAST, 256, true>(map, mapR, mapRbox, a, grid, s, pdl);
-            case 6: return launch_iter_tma<6, LAST, 256, true>(map, mapR, mapRbox, a, grid, s, pdl);
-            case 7: return launch_iter_tma<7, LAST, 256, true>(map, mapR, mapRbox, a, grid, s, pdl);
-            default: return launch_iter_tma<8, LAST, 256, true>(map, mapR, mapRbox, a, grid, s, pdl);
-        }
-    }
-    switch (m) {
-        case 5: return launch_iter_tma<5, LAST, 256, false>(map, mapR, mapRbox, a, grid, s, pdl);
-        case 6: return launch_iter_tma<6, LAST, 256, false>(map, mapR, mapRbox, a, grid, s, pdl);
-        case 7: return launch_iter_tma<7, LAST, 256, false>(map, mapR, mapRbox, a, grid, s, pdl);
-        default: return launch_iter_tma<8, LAST, 256, false>(map, mapR, mapRbox, a, grid, s, pdl);
-    }
+static int launch_iter_tma_m(int m, bool gauss, bool small_tiles, const CUtensorMap& map, const CUtensorMap& mapR,
+                             const CUtensorMap& mapRbox, const IterArgs& a, dim3 grid, cudaStream_t s, bool pdl) {
+    using Launch = int (*)(const CUtensorMap&, const CUtensorMap&, const CUtensorMap&, const IterArgs&, dim3, cudaStream_t,
+                           bool);
+#define ITER_TMA_M(TY, GAUSS)                                                                                             \
+    { launch_iter_tma<5, LAST, TY, GAUSS>, launch_iter_tma<6, LAST, TY, GAUSS>, launch_iter_tma<7, LAST, TY, GAUSS>,     \
+      launch_iter_tma<8, LAST, TY, GAUSS> }
+    static const Launch table[2][2][4] = {   // [Gaussian window][64 x 16 tiles][m - 5]
+        {ITER_TMA_M(IT_TY, false), ITER_TMA_M(16, false)},
+        {ITER_TMA_M(IT_TY, true), ITER_TMA_M(16, true)}};
+#undef ITER_TMA_M
+    return table[gauss][small_tiles][m - 5](map, mapR, mapRbox, a, grid, s, pdl);
 }
 
 int farneback_run(mavd_handle H, const uint8_t* d_frames, int n_pairs, int pair_stride, float* d_flow,
@@ -1777,7 +1640,6 @@ int farneback_run(mavd_handle H, const uint8_t* d_frames, int n_pairs, int pair_
         // exact power-of-two levels (leading levels of a pyr_scale 0.5 pyramid): one sweep down the frame does their
         // vertical passes, level 1 and 2 get the vectorised horizontal pass (tuning.pyr_sweep; HalfPyr above)
         int nv = 0, nh = 0;
-        bool h1_fused = false;
         if (H->tune.pyr_sweep != 0 && lo == 1 && word_ok) {
             while (nv < VS_MAXLV && 1 + nv <= hi && H->lv[1 + nv].y_half) ++nv;
             while (nh < HP_MAXLV && 1 + nh <= hi && H->lv[1 + nh].x_half) ++nh;
@@ -1805,8 +1667,11 @@ int farneback_run(mavd_handle H, const uint8_t* d_frames, int n_pairs, int pair_
             }
             const dim3 g(ceil_div(words, tb), nb, n_frames);
             const bool pdl = pdl_next(H, lane(st));
-            // level 1's horizontal pass inside the sweep (tuning.pyr_fuse_h1)
-            h1_fused = nh >= 1 && H->tune.pyr_fuse_h1 != 0;
+            // level 1's horizontal pass inside the sweep whenever level 1 is a horizontal decimation too: its vertical
+            // sums never go through HBM (C2 pyramid 0.507 -> 0.468 ms on the B200, profiles/README.md).  Level 1 is not
+            // one when pyr_scale is close to but not 0.5 and only the height halves exactly, e.g. 640 x 200 at 0.498:
+            // level 1 is 319 x 100.
+            const bool h1_fused = nh >= 1;
             if (h1_fused) {
                 const Level& L1 = H->lv[1];
                 vd.img1 = L1.img; vd.img1_stride = L1.plane; vd.pitch1 = L1.pitch;
@@ -1835,7 +1700,8 @@ int farneback_run(mavd_handle H, const uint8_t* d_frames, int n_pairs, int pair_
                                      d_frames, frame_bytes, W, Hh, Wp, word_ok, d));
             MAVD_LAUNCHED();
         }
-        for (int l = h1_fused ? 2 : 1; l <= nh; ++l) {
+        // level 1 here only when the sweep did not run: level 1 is then not a vertical decimation (e.g. an odd height)
+        for (int l = nv >= 1 ? 2 : 1; l <= nh; ++l) {
             const Level& L = H->lv[l];
             HPassW hw;
             memcpy(hw.w, L.xwt, sizeof(hw.w));
@@ -1873,11 +1739,6 @@ int farneback_run(mavd_handle H, const uint8_t* d_frames, int n_pairs, int pair_
         }
         return MAVD_OK;
     };
-    // consecutive pairs share an R plane (R1 of pair p is R0 of pair p+1): interleaving the pairs of a tile in
-    // groups of 4 in the CTA order lets the second reader hit L2 (4502 vs 4441 pairs/s ungrouped, 4338 with the
-    // whole 64-pair batch interleaved: too many concurrent HBM regions)
-    const int pair_group = max(1, min(H->tune.pair_group, n_pairs));
-
     // polynomial expansion of one level for all frames (level 0 reads the u8 frames and blurs on the fly)
     auto expand_level = [&](int li, cudaStream_t st) -> int {
         Level& L = H->lv[li];
@@ -1924,7 +1785,6 @@ int farneback_run(mavd_handle H, const uint8_t* d_frames, int n_pairs, int pair_
         Level& L = H->lv[li];
         {
             ProfScope ps(&H->prof, MAVD_PROF_MATRICES, st);
-            dim3 g(ceil_div(L.w, 64), ceil_div(L.h, 4), n_pairs);
             const bool top = (li == H->n_levels - 1);
             const Level* C = top ? nullptr : &H->lv[li + 1];
             const bool tables = H->tune.mat_coord == 1, no_pow2 = H->tune.mat_coord == 2;
@@ -1932,11 +1792,10 @@ int farneback_run(mavd_handle H, const uint8_t* d_frames, int n_pairs, int pair_
             auto is_pow2 = [](double v) { int e; return v > 0.0 && frexp(v, &e) == 0.5 && e > -20 && e <= 1; };
             const int coord = tables ? MI_COORD_TABLES
                                      : (!no_pow2 && is_pow2(xscale) && is_pow2(yscale)) ? MI_COORD_POW2 : MI_COORD_F64;
-            const int r0_first = H->tune.mat_r0_first, txlog = H->tune.mat_txlog;
-            const dim3 g3(g.z, ceil_div(L.w, 1 << txlog), ceil_div(L.h, 256 >> txlog));       // pair index fastest
+            const dim3 g3(n_pairs, ceil_div(L.w, MI_TX), ceil_div(L.h, MI_TY));       // pair index fastest
 #define MI_ARGS L.R, L.plane, L.w, L.h, L.pitch, (size_t)pair_stride * 5 * L.plane,                                     \
                 top ? nullptr : (const float2*)C->flow, top ? 0 : C->w, top ? 0 : C->h, top ? 0 : C->pitch,             \
-                top ? 0 : C->plane, L.fxi0, L.fxa, L.fyi0, L.fya, (float)(1.0 / fp.pyr_scale), L.M[0], xscale, yscale, txlog, r0_first
+                top ? 0 : C->plane, L.fxi0, L.fxa, L.fyi0, L.fya, (float)(1.0 / fp.pyr_scale), L.M[0], xscale, yscale, 1
             const bool pdl = pdl_next(H, lane(st));
             if (coord == MI_COORD_TABLES) MAVD_CUDA(launch_chained(pdl, matrices_init_kernel<MI_COORD_TABLES>, g3, 256, 0, st, MI_ARGS));
             else if (coord == MI_COORD_POW2) MAVD_CUDA(launch_chained(pdl, matrices_init_kernel<MI_COORD_POW2>, g3, 256, 0, st, MI_ARGS));
@@ -1968,26 +1827,21 @@ int farneback_run(mavd_handle H, const uint8_t* d_frames, int n_pairs, int pair_
             dim3 g(ceil_div(L.w, IT_TX), ceil_div(L.h, IT_TY), n_pairs);
             a.n_pairs = n_pairs;
             a.tiles_x = g.x;
-            a.group = pair_group;
-            a.last_fused = (last && H->tune.last_fused != 0) ? 1 : 0;
             // launches that cannot give every SM its three 64 x 32 tiles (a single pair, the coarse levels) use 64 x 16
-            // tiles: twice the CTAs, half the serial work per CTA (tuning.iter_small_tiles; production variants only)
-            const bool small_tiles = H->tune.iter_small_tiles != 0 && L.has_tmap16 && H->tune.r1_staged != 0 &&
-                                     H->tune.iter_fuse != 0 && H->tune.last_fused != 0 &&
-                                     (long long)g.x * g.y * g.z <= 3LL * 148;
+            // tiles: twice the CTAs, half the serial work per CTA (tuning.iter_small_tiles)
+            const bool small_tiles =
+                H->tune.iter_small_tiles != 0 && L.has_tmap16 && (long long)g.x * g.y * g.z <= 3LL * 148;
             const dim3 g1(small_tiles ? g.x * ceil_div(L.h, 16) * g.z : g.x * g.y * g.z);
             const int RW = IT_TX + 2 * hx, RH = IT_TY + 2 * m;
             const size_t smem = sizeof(float) * ((size_t)RH * RW + (size_t)IT_TY * RW + 5 * IT_TX * IT_TY);
             ProfScope ps(&H->prof, li > 0 ? MAVD_PROF_ITER_COARSE : (last ? MAVD_PROF_ITER_FULL_LAST : MAVD_PROF_ITER_FULL), st);
             int rc;
             const bool pdl = pdl_next(H, lane(st));
-            // Gaussian windows use the TMA kernel's production variants (R1 staged, sums in registers) only
-            const bool prod = H->tune.r1_staged != 0 && H->tune.iter_fuse != 0 && H->tune.last_fused != 0;
-            if ((!gauss || prod) && m >= 5 && m <= 8 && L.has_tmap && !H->force_generic_iter) {
+            if (m >= 5 && m <= 8 && L.has_tmap && !H->force_generic_iter) {
                 const CUtensorMap& mM = small_tiles ? L.tmapM16[cur] : L.tmapM[cur];
                 const CUtensorMap& mRb = small_tiles ? L.tmapRbox16 : L.tmapRbox;
-                rc = last ? launch_iter_tma_m<true>(m, H->tune, small_tiles, mM, L.tmapR, mRb, a, g1, st, pdl)
-                          : launch_iter_tma_m<false>(m, H->tune, small_tiles, mM, L.tmapR, mRb, a, g1, st, pdl);
+                rc = last ? launch_iter_tma_m<true>(m, gauss, small_tiles, mM, L.tmapR, mRb, a, g1, st, pdl)
+                          : launch_iter_tma_m<false>(m, gauss, small_tiles, mM, L.tmapR, mRb, a, g1, st, pdl);
             }
             else if (gauss) rc = last ? launch_iter<true, true>(a, g, smem, st, pdl) : launch_iter<true, false>(a, g, smem, st, pdl);
             else       rc = last ? launch_iter<false, true>(a, g, smem, st, pdl) : launch_iter<false, false>(a, g, smem, st, pdl);
@@ -2001,11 +1855,11 @@ int farneback_run(mavd_handle H, const uint8_t* d_frames, int n_pairs, int pair_
     // The coarse levels (>= 2) are chains of small, latency-bound launches (a 60x34 level is 2 tiles per pair); the
     // expansions of levels 1 and 0 are large and depend only on the frames / pyramid.  Run the coarse chain on a
     // high-priority side stream while the caller's stream does the two big expansions, and join before level 1's
-    // matrices need the level-2 flow.  Stream order as seen by the caller is unchanged.
-    const bool fork = H->n_levels >= 3 && H->s_aux != nullptr && H->tune.overlap != 0;
+    // matrices need the level-2 flow.  The pyramid goes to the side stream too: level 0's expansion reads only the u8
+    // frames.  Stream order as seen by the caller is unchanged.
+    const bool fork = H->n_levels >= 3 && H->s_aux != nullptr;
     const int top_level = H->n_levels - 1;
-    if (fork && H->tune.overlap >= 2) {
-        // the pyramid too goes to the side stream: level 0's expansion reads only the u8 frames
+    if (fork) {
         MAVD_CUDA(cudaEventRecord(H->ev_fork, s));
         MAVD_CUDA(cudaStreamWaitEvent(H->s_aux, H->ev_fork, 0));
         pdl_break(H, lane(H->s_aux));
@@ -2020,22 +1874,6 @@ int farneback_run(mavd_handle H, const uint8_t* d_frames, int n_pairs, int pair_
         MAVD_CUDA(cudaStreamWaitEvent(s, H->ev_pyr, 0));
         pdl_break(H, lane(s));
         TRY_RC(expand_level(1, s));
-        MAVD_CUDA(cudaStreamWaitEvent(s, H->ev_join, 0));
-        pdl_break(H, lane(s));
-        TRY_RC(solve_level(1, s));
-        TRY_RC(solve_level(0, s));
-    } else if (fork) {
-        TRY_RC(build_pyramid(s, 1, top_level));
-        MAVD_CUDA(cudaEventRecord(H->ev_fork, s));
-        MAVD_CUDA(cudaStreamWaitEvent(H->s_aux, H->ev_fork, 0));
-        pdl_break(H, lane(H->s_aux));
-        for (int li = H->n_levels - 1; li >= 2; --li) {
-            TRY_RC(expand_level(li, H->s_aux));
-            TRY_RC(solve_level(li, H->s_aux));
-        }
-        MAVD_CUDA(cudaEventRecord(H->ev_join, H->s_aux));
-        TRY_RC(expand_level(1, s));
-        TRY_RC(expand_level(0, s));
         MAVD_CUDA(cudaStreamWaitEvent(s, H->ev_join, 0));
         pdl_break(H, lane(s));
         TRY_RC(solve_level(1, s));

@@ -34,7 +34,7 @@ def make_imu(n: int, ang: Optional[np.ndarray] = None, dt=None, derotate=None) -
 
 
 def parse_tuning(text: str) -> Dict[str, int]:
-    """'pair_group=8,use_graph=0' -> {'pair_group': 8, 'use_graph': 0} (bench.py --tune, tools/gpu_ab.sh)."""
+    """'pyr_sweep=8,use_graph=0' -> {'pyr_sweep': 8, 'use_graph': 0} (bench.py --tune, tools/gpu_ab.sh)."""
     out: Dict[str, int] = {}
     names = {f[0] for f in Tuning._fields_} - {'reserved'}
     for item in filter(None, (t.strip() for t in text.split(','))):

@@ -50,9 +50,9 @@ def test_ctypes_signatures_have_the_header_arity_and_return_types():
         assert res is restype[ret], '%s: header returns %s' % (name, ret)
 
 
-def test_abi_version_and_defaults(lib):
+def test_abi_version_3_and_defaults(lib):
     from mav_detection_b200 import _lib
-    assert lib.mavd_abi_version() == _lib.ABI_VERSION == 2
+    assert lib.mavd_abi_version() == _lib.ABI_VERSION == 3
     p = _lib.DetectParams()
     lib.mavd_default_detect_params(C.byref(p))
     # focus_of_expansion.py:22-23, processor.py:333-341
@@ -61,14 +61,27 @@ def test_abi_version_and_defaults(lib):
         (0.25, 0.5, 8.0, 0.5, 1.0, 15.0)
 
 
-def test_struct_layouts():
+def test_struct_layouts_of_abi_3():
     from mav_detection_b200 import _lib
     assert C.sizeof(_lib.Imu) == 40
     assert C.sizeof(_lib.FarnebackParams) == 40
     assert C.sizeof(_lib.FrameStats) == 8 * 9 + 16 + 16 + 16
-    assert C.sizeof(_lib.Tuning) == 16 * 4 and C.sizeof(_lib.AuxInputs) == 40
+    assert C.sizeof(_lib.Tuning) == 8 * 4 and C.sizeof(_lib.AuxInputs) == 40
     assert C.sizeof(_lib.FrameRecord) == 16 + 8 + C.sizeof(_lib.FrameStats) + 32 * 5 * 4
     assert np.dtype(_lib.FrameRecord).itemsize == C.sizeof(_lib.FrameRecord)
+
+
+def test_tuning_fields_are_the_header_members():
+    """The ctypes Tuning fields are the mavd_tuning members of include/mavd.h by name, order and array length: a list
+    that drifts from the header can keep the struct's size and then sets the wrong switch without an error."""
+    from mav_detection_b200 import _lib
+    src = open(os.path.join(ROOT, 'include', 'mavd.h')).read()
+    src = re.sub(r'/\*.*?\*/', '', src, flags=re.S)
+    body = re.search(r'typedef struct mavd_tuning \{(.*?)\} mavd_tuning;', src, flags=re.S).group(1)
+    members = re.findall(r'int32_t\s+(\w+)(?:\[(\d+)\])?\s*;', body)
+    assert [(n, int(k or 1)) for n, k in members] == \
+        [(f, getattr(t, '_length_', 1)) for f, t in _lib.Tuning._fields_]
+    assert len(members) == len(re.findall(r';', body))
 
 
 def test_invalid_config_is_a_value_error_without_touching_the_gpu(lib):

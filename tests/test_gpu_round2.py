@@ -257,7 +257,7 @@ def test_processor_batches_the_ground_truth_flow():
     proc.release()
 
 
-def test_graph_replay_equals_direct_launches():
+def test_graph_replay_equals_direct_launches_across_tunings():
     """tuning.use_graph: the captured launch sequence (side stream included) replays the same kernels with the same
     arguments — flows, masks and records are bit-equal to the kernel-by-kernel path, on a user stream and on the
     legacy default stream, first call (capture) and later calls (replay), and after a tuning change."""
@@ -288,7 +288,7 @@ def test_graph_replay_equals_direct_launches():
     assert eng.get_tuning()['use_pdl'] == 1
     gs = eng.graph_stats()
     assert gs['captured'] >= 1 and gs['direct'] == 0, gs
-    eng.set_tuning(pair_group=2, overlap=0, iter_fuse=0, last_fused=0, mat_txlog=5)    # other launch shapes, same results
+    eng.set_tuning(iter_small_tiles=0, polyexp_tma=0, pyr_staged=0)    # other launch shapes, same results
     flow3, fixed3, rec3 = _run_device(eng, seq, n, samples)
     assert np.array_equal(flow3, flow0) and np.array_equal(fixed3, fixed0)
     assert direct_launches > 20
@@ -534,23 +534,27 @@ def test_gaussian_windows_on_the_tma_iteration_kernel(winsize):
     eng.close()
 
 
-@pytest.mark.parametrize('size', [(1920, 1080), (640, 480), (648, 488), (3840, 2160), (2048, 1024), (644, 484)])
-def test_pyramid_sweep_is_bit_identical(size):
+@pytest.mark.parametrize('size', [(1920, 1080), (640, 480), (648, 488), (3840, 2160), (2048, 1024), (644, 484),
+                                  (640, 481), (640, 200, 0.498)])
+def test_pyramid_sweep_equals_the_generic_kernels(size):
     """tuning.pyr_sweep: the exact power-of-two levels of a pyr_scale 0.5 pyramid computed by one sweep down the frame
     (vertical passes) and the vectorised horizontal pass equal the generic kernels' images bit for bit, for every band
     count, on noise frames (every REFLECT_101 border row / column matters); sizes whose coarse levels are not exact
-    decimations (1080 / 16, 484 / 8) mix both kinds of kernels."""
+    decimations (1080 / 16, 484 / 8) mix both kinds of kernels.  An odd height (481) leaves level 1 a horizontal
+    decimation only: no sweep, level 1's horizontal pass on its own.  640 x 200 at pyr_scale 0.498 (levels 319 x 100,
+    159 x 50) is the reverse: the sweep runs without level 1's horizontal pass."""
     import torch
     from mav_detection_b200 import engine
-    W, H = size
+    W, H, pyr_scale = size if len(size) == 3 else size + (0.5,)
     p = dict(engine.SAMPLE_PARAMS)
     p['levels'] = 6
+    p['pyr_scale'] = pyr_scale
     eng = engine.Engine(W, H, p, max_pairs=1)
     rng = np.random.default_rng(W + H)
     frames = torch.from_numpy(rng.integers(0, 256, size=(2, H, W), dtype=np.uint8)).to(eng.device)
 
-    def images(sweep, fuse_h1=1):
-        eng.set_tuning(pyr_sweep=sweep, pyr_fuse_h1=fuse_h1)
+    def images(sweep):
+        eng.set_tuning(pyr_sweep=sweep)
         flow = eng.farneback(frames, pair_stride=2)
         torch.cuda.synchronize()
         eng._keep_alive = (frames, flow)
@@ -559,8 +563,8 @@ def test_pyramid_sweep_is_bit_identical(size):
 
     ref, flow_ref = images(0)
     assert len(ref) >= 4
-    for sweep, fuse_h1 in ((1, 1), (1, 0), (2, 1), (5, 0), (64, 1)):
-        got, flow = images(sweep, fuse_h1)
+    for sweep in (1, 2, 5, 64):
+        got, flow = images(sweep)
         for k, (a, b) in enumerate(zip(ref, got)):
             assert np.array_equal(a, b), (sweep, 1 + k // 2, k % 2, float(np.abs(a - b).max()))
         assert np.array_equal(flow, flow_ref), sweep
