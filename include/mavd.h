@@ -49,6 +49,7 @@ enum {
 #define MAVD_SAMPLES_PER_FRAME (4 * MAVD_N_SAMPLE_PAIRS) /* 2000 row draws then 2000 column draws */
 #define MAVD_MAX_BOXES 32         /* component boxes kept per frame record */
 #define MAVD_HOST_SLOTS 3         /* batches that may be in flight through mavd_submit_host */
+#define MAVD_MAX_DETECTIONS 256   /* largest max_det of a detection table */
 
 /* Arguments of cv2.calcOpticalFlowFarneback as called at src/farneback.py:76-80. */
 typedef struct mavd_farneback_params {
@@ -154,6 +155,19 @@ typedef struct mavd_frame_record {
     mavd_frame_stats stats;
     int32_t boxes[MAVD_MAX_BOXES][5]; /* left, top, width, height, area; raster first-appearance order */
 } mavd_frame_record;
+
+/* One entry of a frame's detection table: an 8-connected component of estimate_fixed (or of the mask given to
+ * mavd_detections).  A table lists the max_det largest components of a frame, ordered by area descending, then label
+ * ascending; entries past min(n_labels, max_det) are all zero.  Every frame's table depends on that frame alone. */
+typedef struct mavd_detection {
+    int32_t label;        /* canonical label as mavd_ccl numbers it (raster first appearance); 0 = unused entry */
+    int32_t box[4];       /* left, top, width, height */
+    int32_t area;
+    int64_t sum_x, sum_y; /* sums of column and row indices over the pixels: centroid = sum / area, exact */
+    double flow_sum[2];   /* sum over the pixels of the derotated flow (mavd_derotate's float64 values; the float32
+                             flow widened when imu.derotate == 0).  Summed with float64 atomics: reproducible to the
+                             rounding of the summation order, not bit for bit */
+} mavd_detection;        /* 56 bytes */
 
 typedef struct mavd_handle_s* mavd_handle;
 
@@ -273,6 +287,13 @@ int mavd_mask_overlay(const uint8_t* d_frame, int32_t channels, const uint8_t* d
 int mavd_ccl(mavd_handle h, const uint8_t* d_mask, int32_t n, int32_t* d_labels, int32_t* d_boxes,
              int32_t max_boxes, int32_t* d_n_labels, void* stream);
 
+/* Detection tables of n masks (H, W) uint8, non-zero = foreground: d_det receives n x max_det mavd_detection,
+ * 1 <= max_det <= MAVD_MAX_DETECTIONS.  d_flow (nullable) is (n, H, W, 2) float32 and then needs h_imu (n entries): each
+ * flow_sum adds mavd_derotate's value of every pixel; without a flow flow_sum is 0.  The first call that asks a handle
+ * for a table allocates (max_pairs x (ceil(W/2) * ceil(H/2) + 1)) int32 of per-label workspace. */
+int mavd_detections(mavd_handle h, const uint8_t* d_mask, int32_t n, const float* d_flow, const mavd_imu* h_imu,
+                    int32_t max_det, mavd_detection* d_det, void* stream);
+
 /* ---- detection from a given flow field, device buffers: derotate -> FoE -> phi/masks -> components ----
  * One iteration of Processor.run_detection (src/processor.py:305-362) per frame, starting from the
  * flow that Dataset.get_flow_uv returns (src/datasets/dataset.py:205-212).  d_total_out / d_fixed_out
@@ -344,6 +365,28 @@ int mavd_submit_host_ex(mavd_handle h, int32_t slot, const uint8_t* h_frames, in
 int mavd_detect_host_ex(mavd_handle h, const float* h_flow, int32_t n, const mavd_imu* h_imu,
                         const mavd_detect_params* prm, const int32_t* h_samples, const mavd_aux_inputs* h_aux,
                         int32_t flags, uint8_t* h_fixed_out, mavd_frame_record* h_records, void* stream);
+
+/* ---- the _ex calls plus each frame's detection table (mavd_detection) of estimate_fixed ----
+ * The _ex calls forward to these with det = NULL.  det: n x max_det entries, a DEVICE pointer for mavd_detect_det /
+ * mavd_process_det and a HOST pointer for mavd_submit_host_det / mavd_detect_host_det (valid after the wait, like the
+ * records); 1 <= max_det <= MAVD_MAX_DETECTIONS when det is non-NULL.  The table comes from the same labelling as
+ * record.boxes (an entry with label <= MAVD_MAX_BOXES has the box and area of boxes[label - 1]); flow_sum sums the
+ * derotated flow of the call (the caller's flow, or the Farneback flow of the pair). */
+int mavd_detect_det(mavd_handle h, const float* d_flow, int32_t n, const mavd_imu* h_imu, const mavd_detect_params* prm,
+                    const int32_t* d_samples, const mavd_aux_inputs* d_aux, uint8_t* d_total_out, uint8_t* d_fixed_out,
+                    mavd_frame_record* d_records, int32_t max_det, mavd_detection* d_det, void* stream);
+int mavd_process_det(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int32_t pair_stride, const mavd_imu* h_imu,
+                     const mavd_detect_params* prm, const int32_t* d_samples, const mavd_aux_inputs* d_aux,
+                     float* d_flow_out, uint8_t* d_total_out, uint8_t* d_fixed_out, mavd_frame_record* d_records,
+                     int32_t max_det, mavd_detection* d_det, void* stream);
+int mavd_submit_host_det(mavd_handle h, int32_t slot, const uint8_t* h_frames, int32_t n_pairs, int32_t pair_stride,
+                         const mavd_imu* h_imu, const mavd_detect_params* prm, const int32_t* h_samples,
+                         const mavd_aux_inputs* h_aux, int32_t flags, float* h_flow_out, uint8_t* h_fixed_out,
+                         mavd_frame_record* h_records, int32_t max_det, mavd_detection* h_det, void* stream);
+int mavd_detect_host_det(mavd_handle h, const float* h_flow, int32_t n, const mavd_imu* h_imu,
+                         const mavd_detect_params* prm, const int32_t* h_samples, const mavd_aux_inputs* h_aux,
+                         int32_t flags, uint8_t* h_fixed_out, mavd_frame_record* h_records, int32_t max_det,
+                         mavd_detection* h_det, void* stream);
 
 /* ---- 1-bit-per-pixel masks on the wire (ground-truth segmentation in, estimate_fixed out) ----
  * Bytes one packed (H, W) mask occupies: ceil(H*W / 8) rounded up to a multiple of 4.  Bit k of byte j is pixel

@@ -15,6 +15,7 @@ N_SAMPLE_PAIRS = 1000
 SAMPLES_PER_FRAME = 4 * N_SAMPLE_PAIRS
 MAX_BOXES = 32
 HOST_SLOTS = 3
+MAX_DETECTIONS = 256
 OPTFLOW_FARNEBACK_GAUSSIAN = 256
 
 
@@ -49,6 +50,12 @@ class FrameStats(C.Structure):
 class FrameRecord(C.Structure):
     _fields_ = [('foe', C.c_double * 2), ('n_intersections', C.c_int32), ('n_labels', C.c_int32),
                 ('stats', FrameStats), ('boxes', (C.c_int32 * 5) * MAX_BOXES)]
+
+
+class Detection(C.Structure):
+    """One entry of a frame's detection table (include/mavd.h: mavd_detection)."""
+    _fields_ = [('label', C.c_int32), ('box', C.c_int32 * 4), ('area', C.c_int32), ('sum_x', C.c_int64),
+                ('sum_y', C.c_int64), ('flow_sum', C.c_double * 2)]
 
 
 class Tuning(C.Structure):
@@ -121,6 +128,15 @@ SIGNATURES = {
                                       _P, C.POINTER(AuxInputs), C.c_int32, _P, _P, _P, _P]),
     'mavd_detect_host_ex': (C.c_int, [_P, _P, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams), _P,
                                       C.POINTER(AuxInputs), C.c_int32, _P, _P, _P]),
+    'mavd_detections': (C.c_int, [_P, _P, C.c_int32, _P, C.POINTER(Imu), C.c_int32, _P, _P]),
+    'mavd_detect_det': (C.c_int, [_P, _P, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams), _P, C.POINTER(AuxInputs),
+                                  _P, _P, _P, C.c_int32, _P, _P]),
+    'mavd_process_det': (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams), _P,
+                                   C.POINTER(AuxInputs), _P, _P, _P, _P, C.c_int32, _P, _P]),
+    'mavd_submit_host_det': (C.c_int, [_P, C.c_int32, _P, C.c_int32, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams),
+                                       _P, C.POINTER(AuxInputs), C.c_int32, _P, _P, _P, C.c_int32, _P, _P]),
+    'mavd_detect_host_det': (C.c_int, [_P, _P, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams), _P,
+                                       C.POINTER(AuxInputs), C.c_int32, _P, _P, C.c_int32, _P, _P]),
     'mavd_packed_mask_bytes': (C.c_int64, [C.c_int32, C.c_int32]),
     'mavd_pack_mask': (C.c_int, [_P, C.c_int32, C.c_int64, _P, _P]),
     'mavd_unpack_mask': (C.c_int, [_P, C.c_int32, C.c_int64, C.c_uint8, _P, _P]),

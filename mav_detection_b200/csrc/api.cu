@@ -751,6 +751,37 @@ int mavd_residual_masks(mavd_handle h, const float* d_flow, int32_t n, const mav
                         d_stats, sizeof(mavd_frame_stats), n64 > 0 ? (h->batch_rot > 0 ? 1 : 2) : 0, n32 > 0, (cudaStream_t)stream);
 }
 
+// A detection table request: max_det in range whenever there is a table.  The per-label workspace is allocated by the
+// first request (outside any graph capture: every caller runs this before run_graphed).
+static int check_det(mavd_handle h, int max_det, const void* det, const char* what) {
+    if (!det) return MAVD_OK;
+    MAVD_REQUIRE(max_det >= 1 && max_det <= MAVD_MAX_DETECTIONS, MAVD_ERR_INVALID, "%s: max_det %d outside 1..%d", what,
+                 max_det, MAVD_MAX_DETECTIONS);
+    MAVD_REQUIRE((reinterpret_cast<uintptr_t>(det) & 7) == 0, MAVD_ERR_INVALID, "%s: detections must be 8-byte aligned",
+                 what);
+    if (h->d_det_area) return MAVD_OK;
+    mavd_handle_full* H = static_cast<mavd_handle_full*>(h);
+    TRY(H->arena.alloc(&H->d_det_area, (size_t)h->cfg.max_pairs * det_lab_stride(h)));
+    TRY(H->arena.alloc(&H->d_det_nlabels, (size_t)h->cfg.max_pairs));
+    H->bytes = H->arena.bytes;
+    return MAVD_OK;
+}
+
+int mavd_detections(mavd_handle h, const uint8_t* d_mask, int32_t n, const float* d_flow, const mavd_imu* h_imu,
+                    int32_t max_det, mavd_detection* d_det, void* stream) {
+    DeviceGuard dg(h ? h->cfg.device : -1);
+    TRY(check_batch(h, n, "detections"));
+    MAVD_REQUIRE(d_det != nullptr, MAVD_ERR_INVALID, "detections: NULL table");
+    MAVD_REQUIRE(!d_flow || h_imu, MAVD_ERR_INVALID, "detections: a flow needs an imu array");
+    TRY(check_det(h, max_det, d_det, "detections"));
+    if (n == 0) return MAVD_OK;
+    MAVD_REQUIRE(d_mask != nullptr, MAVD_ERR_INVALID, "detections: NULL mask");
+    const cudaStream_t s = (cudaStream_t)stream;
+    if (d_flow) TRY(upload_imu(h, h_imu, n, s, nullptr, nullptr));
+    const DetArgs da{d_det, max_det, h->d_det_area, det_lab_stride(h), d_flow, h->d_imu};
+    return ccl_run(h, d_mask, n, nullptr, nullptr, 0, 0, h->d_det_nlabels, sizeof(int32_t), s, false, &da);
+}
+
 int mavd_ccl(mavd_handle h, const uint8_t* d_mask, int32_t n, int32_t* d_labels, int32_t* d_boxes, int32_t max_boxes,
              int32_t* d_n_labels, void* stream) {
     DeviceGuard dg(h ? h->cfg.device : -1);
@@ -814,7 +845,7 @@ static const mavd_aux_inputs kNoAux = {nullptr, 0, nullptr, 0, nullptr};
 
 static int detect_run(mavd_handle h, const float* flow, int n, const mavd_detect_params& p, int n64, int n32,
                       const int32_t* d_samples, const mavd_aux_inputs& aux, uint8_t* d_total_out, uint8_t* fixed,
-                      mavd_frame_record* d_records, cudaStream_t s) {
+                      mavd_frame_record* d_records, int max_det, mavd_detection* d_det, cudaStream_t s) {
     char* stats0 = reinterpret_cast<char*>(d_records) + offsetof(mavd_frame_record, stats);
     // FoE estimation is one CTA per frame; what the residual kernel needs besides the FoE (zeroed statistics, the
     // segmentation maxima, an empty unit list) does not depend on it and runs on the side stream meanwhile
@@ -842,8 +873,9 @@ static int detect_run(mavd_handle h, const float* flow, int n, const mavd_detect
                      n64 > 0 ? (h->batch_rot > 0 ? 1 : 2) : 0, n32 > 0, s, true, aux.gt_flow, fork));
     int32_t* boxes0 = reinterpret_cast<int32_t*>(reinterpret_cast<char*>(d_records) + offsetof(mavd_frame_record, boxes));
     char* nl0 = reinterpret_cast<char*>(d_records) + offsetof(mavd_frame_record, n_labels);
+    const DetArgs da{d_det, max_det, h->d_det_area, det_lab_stride(h), flow, h->d_imu};
     TRY(ccl_run(h, fixed, n, nullptr, boxes0, sizeof(mavd_frame_record) / sizeof(int32_t), MAVD_MAX_BOXES,
-                reinterpret_cast<int32_t*>(nl0), sizeof(mavd_frame_record), s, true));
+                reinterpret_cast<int32_t*>(nl0), sizeof(mavd_frame_record), s, true, d_det ? &da : nullptr));
     MAVD_CUDA(launch_chained(pdl_next(h), records_fill_kernel, ceil_div(n, 128), 128, 0, s, d_records, h->d_foe, h->d_ninter, n));
     MAVD_LAUNCHED();
     return MAVD_OK;
@@ -975,11 +1007,13 @@ int mavd_farneback(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int3
                        ss.s, [&](cudaStream_t s) { return farneback_run(h, d_frames, n_pairs, pair_stride, d_flow, s); });
 }
 
-int mavd_detect_ex(mavd_handle h, const float* d_flow, int32_t n, const mavd_imu* h_imu, const mavd_detect_params* prm,
-                   const int32_t* d_samples, const mavd_aux_inputs* d_aux, uint8_t* d_total_out, uint8_t* d_fixed_out,
-                   mavd_frame_record* d_records, void* stream) {
+int mavd_detect_det(mavd_handle h, const float* d_flow, int32_t n, const mavd_imu* h_imu, const mavd_detect_params* prm,
+                    const int32_t* d_samples, const mavd_aux_inputs* d_aux, uint8_t* d_total_out, uint8_t* d_fixed_out,
+                    mavd_frame_record* d_records, int32_t max_det, mavd_detection* d_det, void* stream) {
     DeviceGuard dg(h ? h->cfg.device : -1);
     TRY(check_batch(h, n, "detect"));
+    TRY(check_det(h, max_det, d_det, "detect"));
+    if (!d_det) max_det = 0;
     if (n == 0) return MAVD_OK;
     MAVD_REQUIRE(d_flow && d_samples && d_records, MAVD_ERR_INVALID, "detect: NULL buffer");
     StreamScope ss(h, stream);
@@ -990,10 +1024,18 @@ int mavd_detect_ex(mavd_handle h, const float* d_flow, int32_t n, const mavd_imu
     TRY(upload_imu(h, h_imu, n, ss.s, &n64, &n32));
     uint8_t* fixed = d_fixed_out ? d_fixed_out : h->d_fixed;
     return run_graphed(h, std::move(KeyBuilder()(int64_t(2))(d_flow)(int64_t(n))(p)(int64_t(n64))(int64_t(h->batch_rot > 0))(int64_t(n32))(d_samples)(aux)
-                                        (d_total_out)(fixed)(d_records).k),
+                                        (d_total_out)(fixed)(d_records)(int64_t(max_det))(d_det).k),
                        ss.s, [&](cudaStream_t s) {
-                           return detect_run(h, d_flow, n, p, n64, n32, d_samples, aux, d_total_out, fixed, d_records, s);
+                           return detect_run(h, d_flow, n, p, n64, n32, d_samples, aux, d_total_out, fixed, d_records,
+                                             max_det, d_det, s);
                        });
+}
+
+int mavd_detect_ex(mavd_handle h, const float* d_flow, int32_t n, const mavd_imu* h_imu, const mavd_detect_params* prm,
+                   const int32_t* d_samples, const mavd_aux_inputs* d_aux, uint8_t* d_total_out, uint8_t* d_fixed_out,
+                   mavd_frame_record* d_records, void* stream) {
+    return mavd_detect_det(h, d_flow, n, h_imu, prm, d_samples, d_aux, d_total_out, d_fixed_out, d_records, 0, nullptr,
+                           stream);
 }
 
 int mavd_detect(mavd_handle h, const float* d_flow, int32_t n, const mavd_imu* h_imu, const mavd_detect_params* prm,
@@ -1004,13 +1046,15 @@ int mavd_detect(mavd_handle h, const float* d_flow, int32_t n, const mavd_imu* h
     return mavd_detect_ex(h, d_flow, n, h_imu, prm, d_samples, &aux, d_total_out, d_fixed_out, d_records, stream);
 }
 
-int mavd_process_ex(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int32_t pair_stride, const mavd_imu* h_imu,
-                    const mavd_detect_params* prm, const int32_t* d_samples, const mavd_aux_inputs* d_aux,
-                    float* d_flow_out, uint8_t* d_total_out, uint8_t* d_fixed_out, mavd_frame_record* d_records,
-                    void* stream) {
+int mavd_process_det(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int32_t pair_stride, const mavd_imu* h_imu,
+                     const mavd_detect_params* prm, const int32_t* d_samples, const mavd_aux_inputs* d_aux,
+                     float* d_flow_out, uint8_t* d_total_out, uint8_t* d_fixed_out, mavd_frame_record* d_records,
+                     int32_t max_det, mavd_detection* d_det, void* stream) {
     DeviceGuard dg(h ? h->cfg.device : -1);
     TRY(check_batch(h, n_pairs, "process"));
     MAVD_REQUIRE(pair_stride == 1 || pair_stride == 2, MAVD_ERR_INVALID, "pair_stride must be 1 or 2");
+    TRY(check_det(h, max_det, d_det, "process"));
+    if (!d_det) max_det = 0;
     if (n_pairs == 0) return MAVD_OK;
     MAVD_REQUIRE(d_frames && d_samples && d_records, MAVD_ERR_INVALID, "process: NULL buffer");
     StreamScope ss(h, stream);
@@ -1023,11 +1067,21 @@ int mavd_process_ex(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int
     TRY(upload_imu(h, h_imu, n_pairs, ss.s, &n64, &n32));
     note_farneback_call(h, d_frames, n_pairs, pair_stride, flow);
     return run_graphed(h, std::move(KeyBuilder()(int64_t(3))(d_frames)(int64_t(n_pairs))(int64_t(pair_stride))(p)(int64_t(n64))(int64_t(h->batch_rot > 0))
-                                        (int64_t(n32))(d_samples)(aux)(flow)(d_total_out)(fixed)(d_records).k),
+                                        (int64_t(n32))(d_samples)(aux)(flow)(d_total_out)(fixed)(d_records)(int64_t(max_det))
+                                        (d_det).k),
                        ss.s, [&](cudaStream_t s) {
                            TRY(farneback_run(h, d_frames, n_pairs, pair_stride, flow, s));
-                           return detect_run(h, flow, n_pairs, p, n64, n32, d_samples, aux, d_total_out, fixed, d_records, s);
+                           return detect_run(h, flow, n_pairs, p, n64, n32, d_samples, aux, d_total_out, fixed, d_records,
+                                             max_det, d_det, s);
                        });
+}
+
+int mavd_process_ex(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int32_t pair_stride, const mavd_imu* h_imu,
+                    const mavd_detect_params* prm, const int32_t* d_samples, const mavd_aux_inputs* d_aux,
+                    float* d_flow_out, uint8_t* d_total_out, uint8_t* d_fixed_out, mavd_frame_record* d_records,
+                    void* stream) {
+    return mavd_process_det(h, d_frames, n_pairs, pair_stride, h_imu, prm, d_samples, d_aux, d_flow_out, d_total_out,
+                            d_fixed_out, d_records, 0, nullptr, stream);
 }
 
 int mavd_process(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int32_t pair_stride, const mavd_imu* h_imu,
@@ -1044,7 +1098,7 @@ int mavd_process(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int32_
 // stream, copy-out stream).
 // ------------------------------------------------------------------------------------------------
 static int ensure_slot(mavd_handle h, int slot, bool want_flow_out, bool want_flow_in, bool want_bits_in, bool want_bits_out,
-                       bool want_gt) {
+                       bool want_gt, bool want_det) {
     mavd_handle_full* H = static_cast<mavd_handle_full*>(h);
     mavd_handle_s::HostSlot& S = H->slot[slot];
     const size_t npx = (size_t)h->cfg.width * h->cfg.height;
@@ -1056,6 +1110,7 @@ static int ensure_slot(mavd_handle h, int slot, bool want_flow_out, bool want_fl
     if (want_bits_in && !S.d_bits_in) TRY(H->arena.alloc(&S.d_bits_in, 2 * B * pb));
     if (want_bits_out && !S.d_bits_out) TRY(H->arena.alloc(&S.d_bits_out, B * pb));
     if (want_gt && !S.d_gt_flow) TRY(H->arena.alloc(&S.d_gt_flow, B * npx * 2));
+    if (want_det && !S.d_det) TRY(H->arena.alloc(&S.d_det, (size_t)B * MAVD_MAX_DETECTIONS));
     if (!H->s_in) MAVD_CUDA(cudaStreamCreateWithFlags(&H->s_in, cudaStreamNonBlocking));
     if (!H->s_out) MAVD_CUDA(cudaStreamCreateWithFlags(&H->s_out, cudaStreamNonBlocking));
     H->bytes = H->arena.bytes;
@@ -1122,12 +1177,15 @@ static int check_aux_strides(mavd_handle h, const mavd_aux_inputs& a, int flags)
     return MAVD_OK;
 }
 
-int mavd_submit_host_ex(mavd_handle h, int32_t slot, const uint8_t* h_frames, int32_t n_pairs, int32_t pair_stride,
-                        const mavd_imu* h_imu, const mavd_detect_params* prm, const int32_t* h_samples,
-                        const mavd_aux_inputs* h_aux, int32_t flags, float* h_flow_out, uint8_t* h_fixed_out,
-                        mavd_frame_record* h_records, void* stream) {
+int mavd_submit_host_det(mavd_handle h, int32_t slot, const uint8_t* h_frames, int32_t n_pairs, int32_t pair_stride,
+                         const mavd_imu* h_imu, const mavd_detect_params* prm, const int32_t* h_samples,
+                         const mavd_aux_inputs* h_aux, int32_t flags, float* h_flow_out, uint8_t* h_fixed_out,
+                         mavd_frame_record* h_records, int32_t max_det, mavd_detection* h_det, void* stream) {
     DeviceGuard dg(h ? h->cfg.device : -1);
     TRY(check_batch(h, n_pairs, "submit_host"));
+    if (h_det)
+        MAVD_REQUIRE(max_det >= 1 && max_det <= MAVD_MAX_DETECTIONS, MAVD_ERR_INVALID,
+                     "submit_host: max_det %d outside 1..%d", max_det, MAVD_MAX_DETECTIONS);
     MAVD_REQUIRE(slot >= 0 && slot < MAVD_HOST_SLOTS, MAVD_ERR_INVALID, "slot %d out of range", slot);
     MAVD_REQUIRE(pair_stride == 1 || pair_stride == 2, MAVD_ERR_INVALID, "pair_stride must be 1 or 2");
     MAVD_REQUIRE(n_pairs >= 1, MAVD_ERR_INVALID, "submit_host: empty batch");
@@ -1139,7 +1197,7 @@ int mavd_submit_host_ex(mavd_handle h, int32_t slot, const uint8_t* h_frames, in
     const size_t pb = (size_t)packed_mask_bytes((int64_t)npx);
     const bool bgr = (flags & MAVD_HOST_BGR) != 0, fixed_packed = (flags & MAVD_HOST_FIXED_PACKED) != 0;
     TRY(ensure_slot(h, slot, h_flow_out != nullptr, false, (flags & (MAVD_HOST_SEG_PACKED | MAVD_HOST_SKY_PACKED)) != 0,
-                    fixed_packed && h_fixed_out, ha.gt_flow != nullptr));
+                    fixed_packed && h_fixed_out, ha.gt_flow != nullptr, h_det != nullptr));
     mavd_handle_s::HostSlot& S = h->slot[slot];
     MAVD_REQUIRE(!S.busy, MAVD_ERR_INVALID, "slot %d is still in flight: call mavd_wait_host first", slot);
     const int n_frames = pair_stride == 1 ? n_pairs + 1 : 2 * n_pairs;
@@ -1166,8 +1224,9 @@ int mavd_submit_host_ex(mavd_handle h, int32_t slot, const uint8_t* h_frames, in
     // the next batch's Farneback, was measured: no gain, the GPU is already full and the work is only re-ordered.)
     MAVD_CUDA(cudaStreamWaitEvent(s, S.ev_in, 0));
     if (!(flags & MAVD_HOST_COPY_ONLY))
-        TRY(mavd_process_ex(h, S.d_frames, n_pairs, pair_stride, h_imu, prm, S.d_samples, &da,
-                            h_flow_out ? S.d_flow : nullptr, nullptr, S.d_fixed, S.d_records, s));
+        TRY(mavd_process_det(h, S.d_frames, n_pairs, pair_stride, h_imu, prm, S.d_samples, &da,
+                             h_flow_out ? S.d_flow : nullptr, nullptr, S.d_fixed, S.d_records, max_det,
+                             h_det ? S.d_det : nullptr, s));
     MAVD_CUDA(cudaEventRecord(S.ev_done, s));
     // copy-out stream
     MAVD_CUDA(cudaStreamWaitEvent(h->s_out, S.ev_done, 0));
@@ -1180,10 +1239,21 @@ int mavd_submit_host_ex(mavd_handle h, int32_t slot, const uint8_t* h_frames, in
     }
     if (h_flow_out)
         MAVD_CUDA(cudaMemcpyAsync(h_flow_out, S.d_flow, sizeof(float) * 2 * npx * n_pairs, cudaMemcpyDeviceToHost, h->s_out));
+    if (h_det)
+        MAVD_CUDA(cudaMemcpyAsync(h_det, S.d_det, sizeof(mavd_detection) * max_det * n_pairs, cudaMemcpyDeviceToHost,
+                                  h->s_out));
     MAVD_CUDA(cudaEventRecord(S.ev_out, h->s_out));
     // the next batch's copy-in must not overwrite staging a kernel still reads: ordered by slot reuse rule
     S.busy = true;
     return MAVD_OK;
+}
+
+int mavd_submit_host_ex(mavd_handle h, int32_t slot, const uint8_t* h_frames, int32_t n_pairs, int32_t pair_stride,
+                        const mavd_imu* h_imu, const mavd_detect_params* prm, const int32_t* h_samples,
+                        const mavd_aux_inputs* h_aux, int32_t flags, float* h_flow_out, uint8_t* h_fixed_out,
+                        mavd_frame_record* h_records, void* stream) {
+    return mavd_submit_host_det(h, slot, h_frames, n_pairs, pair_stride, h_imu, prm, h_samples, h_aux, flags, h_flow_out,
+                                h_fixed_out, h_records, 0, nullptr, stream);
 }
 
 int mavd_submit_host(mavd_handle h, int32_t slot, const uint8_t* h_frames, int32_t n_pairs, int32_t pair_stride,
@@ -1228,11 +1298,15 @@ int mavd_process_host(mavd_handle h, const uint8_t* h_frames, int32_t n_pairs, i
     return mavd_wait_host(h, 0);
 }
 
-int mavd_detect_host_ex(mavd_handle h, const float* h_flow, int32_t n, const mavd_imu* h_imu,
-                        const mavd_detect_params* prm, const int32_t* h_samples, const mavd_aux_inputs* h_aux,
-                        int32_t flags, uint8_t* h_fixed_out, mavd_frame_record* h_records, void* stream) {
+int mavd_detect_host_det(mavd_handle h, const float* h_flow, int32_t n, const mavd_imu* h_imu,
+                         const mavd_detect_params* prm, const int32_t* h_samples, const mavd_aux_inputs* h_aux,
+                         int32_t flags, uint8_t* h_fixed_out, mavd_frame_record* h_records, int32_t max_det,
+                         mavd_detection* h_det, void* stream) {
     DeviceGuard dg(h ? h->cfg.device : -1);
     TRY(check_batch(h, n, "detect_host"));
+    if (h_det)
+        MAVD_REQUIRE(max_det >= 1 && max_det <= MAVD_MAX_DETECTIONS, MAVD_ERR_INVALID,
+                     "detect_host: max_det %d outside 1..%d", max_det, MAVD_MAX_DETECTIONS);
     if (n == 0) return MAVD_OK;
     MAVD_REQUIRE(h_flow && h_samples && h_records, MAVD_ERR_INVALID, "detect_host: NULL buffer");
     MAVD_REQUIRE((flags & MAVD_HOST_BGR) == 0, MAVD_ERR_INVALID, "detect_host: MAVD_HOST_BGR has no meaning here");
@@ -1244,7 +1318,7 @@ int mavd_detect_host_ex(mavd_handle h, const float* h_flow, int32_t n, const mav
     const bool fixed_packed = (flags & MAVD_HOST_FIXED_PACKED) != 0;
     TRY(mavd_wait_host(h, 0));
     TRY(ensure_slot(h, 0, false, true, (flags & (MAVD_HOST_SEG_PACKED | MAVD_HOST_SKY_PACKED)) != 0,
-                    fixed_packed && h_fixed_out, ha.gt_flow != nullptr));
+                    fixed_packed && h_fixed_out, ha.gt_flow != nullptr, h_det != nullptr));
     mavd_handle_s::HostSlot& S = h->slot[0];
     StreamScope ss(h, stream);
     cudaStream_t s = ss.s;
@@ -1253,8 +1327,11 @@ int mavd_detect_host_ex(mavd_handle h, const float* h_flow, int32_t n, const mav
     mavd_aux_inputs da;
     TRY(stage_aux(h, S, ha, flags, n, s, &da));
     if (!(flags & MAVD_HOST_COPY_ONLY))
-        TRY(mavd_detect_ex(h, S.d_flow_in, n, h_imu, prm, S.d_samples, &da, nullptr, S.d_fixed, S.d_records, s));
+        TRY(mavd_detect_det(h, S.d_flow_in, n, h_imu, prm, S.d_samples, &da, nullptr, S.d_fixed, S.d_records, max_det,
+                            h_det ? S.d_det : nullptr, s));
     MAVD_CUDA(cudaMemcpyAsync(h_records, S.d_records, sizeof(mavd_frame_record) * n, cudaMemcpyDeviceToHost, s));
+    if (h_det)
+        MAVD_CUDA(cudaMemcpyAsync(h_det, S.d_det, sizeof(mavd_detection) * max_det * n, cudaMemcpyDeviceToHost, s));
     if (h_fixed_out && fixed_packed) {
         TRY(pack_mask_run(S.d_fixed, n, (int64_t)npx, S.d_bits_out, s));
         MAVD_CUDA(cudaMemcpyAsync(h_fixed_out, S.d_bits_out, pb * n, cudaMemcpyDeviceToHost, s));
@@ -1263,6 +1340,13 @@ int mavd_detect_host_ex(mavd_handle h, const float* h_flow, int32_t n, const mav
     }
     MAVD_CUDA(cudaStreamSynchronize(s));
     return MAVD_OK;
+}
+
+int mavd_detect_host_ex(mavd_handle h, const float* h_flow, int32_t n, const mavd_imu* h_imu,
+                        const mavd_detect_params* prm, const int32_t* h_samples, const mavd_aux_inputs* h_aux,
+                        int32_t flags, uint8_t* h_fixed_out, mavd_frame_record* h_records, void* stream) {
+    return mavd_detect_host_det(h, h_flow, n, h_imu, prm, h_samples, h_aux, flags, h_fixed_out, h_records, 0, nullptr,
+                                stream);
 }
 
 int mavd_detect_host(mavd_handle h, const float* h_flow, int32_t n, const mavd_imu* h_imu, const mavd_detect_params* prm,

@@ -215,6 +215,9 @@ struct mavd_handle_s {
     uint8_t* d_total = nullptr;     // [max_pairs][H][W]
     uint8_t* d_fixed = nullptr;
     float* d_flow = nullptr;        // [max_pairs][H][W][2] (when the caller does not want the flow)
+    // detection tables (allocated by the first call that asks for one: mavd_workspace_bytes is unchanged otherwise)
+    int32_t* d_det_area = nullptr;  // [max_pairs][det_lab_stride]: area per label, then -(slot + 1) of a selected label
+    int32_t* d_det_nlabels = nullptr;   // [max_pairs] label counts of mavd_detections
     // host-path staging: MAVD_HOST_SLOTS independent sets of device buffers + the streams/events that let
     // the H2D of one batch, the compute of the previous one and the D2H of the one before overlap
     struct HostSlot {
@@ -231,6 +234,7 @@ struct mavd_handle_s {
         uint8_t* d_bits_out = nullptr;  // [max_pairs][packed bytes]: estimate_fixed packed for the way back
         float* d_gt_flow = nullptr;     // [max_pairs][H][W][2] ground-truth flow (allocated on first use)
         float* d_flow = nullptr;        // [max_pairs][H][W][2] flow of the batch (allocated on first request)
+        mavd_detection* d_det = nullptr;    // [max_pairs][MAVD_MAX_DETECTIONS] detection tables (allocated on first request)
         cudaEvent_t ev_in = nullptr, ev_done = nullptr, ev_out = nullptr;
         bool busy = false;
     } slot[MAVD_HOST_SLOTS];
@@ -322,6 +326,18 @@ int magnitude_run(const void* d_flow, int is_f64, int64_t n, void* d_out, cudaSt
 int simple_bbox_run(const uint8_t* d_img, int w, int h, int c, int32_t* d_out5, cudaStream_t s);
 int tpr_fpr_run(const uint8_t* d_gt, const int64_t* d_img, int64_t n, int64_t* d_counts4, cudaStream_t s);
 int flow_vis_run(const float* d_flow, int64_t n, uint8_t* d_bgr, uint32_t* d_scratch3, cudaStream_t s);
+// Detection table of ccl_run: the max_det largest components of each frame (include/mavd.h: mavd_detection).
+struct DetArgs {
+    mavd_detection* det;     // [n][max_det]
+    int max_det;
+    int32_t* lab_area;       // h->d_det_area
+    int lab_stride;          // det_lab_stride(h)
+    const float* flow;       // nullable: (n, H, W, 2) float32, derotated per pixel as mavd_derotate does
+    const mavd_imu* imu;     // device, n entries (with flow)
+};
+// labels a frame can hold under 8-connectivity (one per 2 x 2 block at most), plus the unused label 0
+static inline int det_lab_stride(mavd_handle h) { return ((h->cfg.width + 1) / 2) * ((h->cfg.height + 1) / 2) + 1; }
 int ccl_run(mavd_handle h, const uint8_t* d_mask, int n, int32_t* d_labels, int32_t* d_boxes, size_t boxes_stride,
-            int max_boxes, int32_t* d_n_labels, size_t nlabels_stride_bytes, cudaStream_t s, bool list_ready = false);
+            int max_boxes, int32_t* d_n_labels, size_t nlabels_stride_bytes, cudaStream_t s, bool list_ready = false,
+            const DetArgs* det = nullptr);
 }  // namespace mavd

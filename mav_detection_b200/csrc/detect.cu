@@ -1795,6 +1795,338 @@ __global__ void ccl_boxes_final_kernel(int32_t* boxes, size_t boxes_stride, int 
     else { p[2] = p[2] - p[0] + 1; p[3] = p[3] - p[1] + 1; }
 }
 
+// ------------------------------------------------------------------------------------------------
+// Detection tables (mavd_detection): the max_det largest components of every frame, from the same unit list, forest
+// and rank array that give the record's boxes.
+//   zero    the per-label areas of labels 1..n_labels
+//   area    pass A: area of every label, runs of one label folded in registers (the BoxAcc pattern)
+//   select  one CTA per frame: exact top max_det by (area desc, label asc) — radix select of the cut-off area over
+//           10-bit digits, ties at the cut taken in label order — then lab_area[label] = -(slot + 1) for the selected
+//           labels and every table entry initialised
+//   stats   pass B: box, area, index sums and derotated flow of the selected labels only
+//   final   box corners -> width / height
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) det_area_zero_kernel(int32_t* __restrict__ lab_area, int lab_stride,
+                                                            const char* nlabels_base, size_t nlabels_stride) {
+    pdl_entry();
+    const int f = blockIdx.y;
+    const int nl = *reinterpret_cast<const int32_t*>(nlabels_base + (size_t)f * nlabels_stride);
+    int32_t* A = lab_area + (size_t)f * lab_stride;
+    for (int l = blockIdx.x * blockDim.x + threadIdx.x; l <= nl; l += gridDim.x * blockDim.x) A[l] = 0;
+}
+
+// label of every run start of the unit (0 elsewhere) and the label of the unit's first run (warp-uniform)
+__device__ __forceinline__ int unit_labels(const UnitRuns& R, const int* parent, const int* __restrict__ rank, size_t base,
+                                           int ub, int lab[4]) {
+    const int lane = threadIdx.x & 31;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+        lab[j] = 0;
+        if ((R.S.w[j] >> lane) & 1u) lab[j] = rank[base + parent[base + ub + 32 * j + lane]];
+    }
+    const int s0 = first_set_at_or_above(R.S, 0);
+    int l0 = 0;
+#pragma unroll
+    for (int jj = 0; jj < 4; ++jj) {
+        const int v = __shfl_sync(0xffffffffu, lab[jj], s0 & 31);
+        if ((s0 >> 5) == jj) l0 = v;
+    }
+    return l0;
+}
+
+template <int VEC>
+__global__ void __launch_bounds__(256) det_area_kernel(const uint8_t* __restrict__ mask, const int* parent,
+                                                       const int* __restrict__ rank, int w, int npx, CclList L,
+                                                       int32_t* __restrict__ lab_area, int lab_stride) {
+    pdl_entry();
+    const int warps = gridDim.x * 8, gw = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    const int cnt = *L.count;
+    int acc_f = -1, acc_l = 0, acc_area = 0;       // the (frame, label) whose area the warp holds in registers
+    for (int q = gw; q < cnt; q += warps) {
+        const int e = L.entries[q];
+        const int f = e / L.n_units, u = e - f * L.n_units, ub = u * CCL_UNIT;
+        const size_t base = (size_t)f * npx;
+        UnitRuns R;
+        R.M = ccl_load_bits<VEC>(mask + base, ub, npx);
+        R.RS = row_starts(ub, w, R.x0);
+        unit_runs(R);
+        int lab[4];
+        const int l0 = unit_labels(R, parent, rank, base, ub, lab);
+        if (f != acc_f || l0 != acc_l) {
+            if (acc_f >= 0 && lane == 0) atomicAdd(lab_area + (size_t)acc_f * lab_stride + acc_l, acc_area);
+            acc_f = f; acc_l = l0; acc_area = 0;
+        }
+        int mine = 0;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            if (!((R.S.w[j] >> lane) & 1u)) continue;
+            const int t = 32 * j + lane;
+            const int len = first_set_at_or_above(R.E, t) - t + 1;
+            if (lab[j] == l0) mine += len;
+            else atomicAdd(lab_area + (size_t)f * lab_stride + lab[j], len);
+        }
+        acc_area += __reduce_add_sync(0xffffffffu, mine);
+    }
+    if (acc_f >= 0 && lane == 0) atomicAdd(lab_area + (size_t)acc_f * lab_stride + acc_l, acc_area);
+}
+
+// exclusive prefix of v over the 1024 threads of the block; *total receives the sum (wtot: 33 ints of shared memory,
+// free again when the function returns)
+__device__ __forceinline__ int block_excl_scan_1024(int v, int* wtot, int* total) {
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    int incl = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int t = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += t;
+    }
+    if (lane == 31) wtot[wid] = incl;
+    __syncthreads();
+    if (wid == 0) {
+        const int wv = wtot[lane];
+        int wi = wv;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int t = __shfl_up_sync(0xffffffffu, wi, o);
+            if (lane >= o) wi += t;
+        }
+        wtot[lane] = wi - wv;
+        if (lane == 31) wtot[32] = wi;
+    }
+    __syncthreads();
+    const int r = wtot[wid] + incl - v;
+    *total = wtot[32];
+    __syncthreads();
+    return r;
+}
+
+__global__ void __launch_bounds__(1024) det_select_kernel(int32_t* __restrict__ lab_area, int lab_stride,
+                                                          const char* nlabels_base, size_t nlabels_stride,
+                                                          mavd_detection* __restrict__ det, int max_det) {
+    pdl_entry();
+    __shared__ int hist[1024];
+    __shared__ int wtot[33];
+    __shared__ int sel_lab[MAVD_MAX_DETECTIONS], sel_area[MAVD_MAX_DETECTIONS];
+    __shared__ int s_digit, s_above, s_cnt;
+    const int f = blockIdx.x, tid = threadIdx.x;
+    const int nl = *reinterpret_cast<const int32_t*>(nlabels_base + (size_t)f * nlabels_stride);
+    int32_t* A = lab_area + (size_t)f * lab_stride;
+    // every label with area > cut is taken, and the first take_eq labels with area == cut; with at most max_det labels
+    // all are taken (every label has an area >= 1)
+    int cut = 0, take_eq = 0;
+    if (nl > max_det) {
+        int prefix = 0, hi_mask = 0, rem = max_det;   // rem-th largest area among the labels that match the prefix
+        for (int shift = 20; shift >= 0; shift -= 10) {    // areas < 2^28 (16384^2 pixels)
+            hist[tid] = 0;
+            __syncthreads();
+            for (int l = 1 + tid; l <= nl; l += 1024) {
+                const int a = A[l];
+                if ((a & hi_mask) == prefix) atomicAdd(&hist[(a >> shift) & 1023], 1);
+            }
+            __syncthreads();
+            // thread t looks at digit 1023 - t: inclusive prefix = labels with that digit or a larger one
+            const int c = hist[1023 - tid];
+            int tot;
+            const int ex = block_excl_scan_1024(c, wtot, &tot);
+            if (ex < rem && ex + c >= rem) { s_digit = 1023 - tid; s_above = ex; }
+            __syncthreads();
+            prefix |= s_digit << shift;
+            hi_mask |= 1023 << shift;
+            rem -= s_above;
+            __syncthreads();
+        }
+        cut = prefix;
+        take_eq = rem;
+    }
+    if (tid == 0) s_cnt = 0;
+    __syncthreads();
+    int eq_seen = 0;
+    for (int b = 1; b <= nl; b += 1024) {
+        const int l = b + tid;
+        const int a = l <= nl ? A[l] : 0;
+        const bool eq = a == cut && a > 0;
+        int tot;
+        const int r = block_excl_scan_1024(eq ? 1 : 0, wtot, &tot);
+        if (a > cut || (eq && eq_seen + r < take_eq)) {
+            const int pos = atomicAdd(&s_cnt, 1);
+            sel_lab[pos] = l;
+            sel_area[pos] = a;
+        }
+        eq_seen += tot;
+    }
+    __syncthreads();
+    const int cnt = s_cnt;     // == min(nl, max_det)
+    mavd_detection* D = det + (size_t)f * max_det;
+    for (int i = tid; i < max_det; i += 1024) {
+        if (i < cnt) {
+            const int a = sel_area[i], l = sel_lab[i];
+            int r = 0;
+            for (int k = 0; k < cnt; ++k) r += sel_area[k] > a || (sel_area[k] == a && sel_lab[k] < l);
+            mavd_detection& d = D[r];
+            d.label = l;
+            d.box[0] = 0x7fffffff; d.box[1] = 0x7fffffff; d.box[2] = -1; d.box[3] = -1;
+            d.area = 0;
+            d.sum_x = 0; d.sum_y = 0;
+            d.flow_sum[0] = 0.0; d.flow_sum[1] = 0.0;
+            A[l] = -(r + 1);
+        }
+        if (i >= cnt) {
+            mavd_detection& d = D[i];
+            d.label = 0;
+            d.box[0] = d.box[1] = d.box[2] = d.box[3] = 0;
+            d.area = 0;
+            d.sum_x = 0; d.sum_y = 0;
+            d.flow_sum[0] = 0.0; d.flow_sum[1] = 0.0;
+        }
+    }
+}
+
+// Statistics of one table entry accumulated by a warp (runs of the entry the unit starts with) before one flush.
+struct DetAcc {
+    int f = -1, slot = -1;
+    int x0 = 0x7fffffff, y0 = 0x7fffffff, x1 = -1, y1 = -1, area = 0;
+    long long sx = 0, sy = 0;
+    double fx = 0.0, fy = 0.0;
+};
+
+__device__ __forceinline__ void det_flush(DetAcc& acc, mavd_detection* det, int max_det) {
+    if (acc.f >= 0 && acc.area > 0 && (threadIdx.x & 31) == 0) {
+        mavd_detection* d = det + (size_t)acc.f * max_det + acc.slot;
+        atomicMin(&d->box[0], acc.x0); atomicMin(&d->box[1], acc.y0);
+        atomicMax(&d->box[2], acc.x1); atomicMax(&d->box[3], acc.y1);
+        atomicAdd(&d->area, acc.area);
+        atomicAdd(reinterpret_cast<unsigned long long*>(&d->sum_x), (unsigned long long)acc.sx);
+        atomicAdd(reinterpret_cast<unsigned long long*>(&d->sum_y), (unsigned long long)acc.sy);
+        atomicAdd(&d->flow_sum[0], acc.fx);
+        atomicAdd(&d->flow_sum[1], acc.fy);
+    }
+    acc = DetAcc();
+}
+
+__device__ __forceinline__ double warp_sum_f64(double v) {
+#pragma unroll
+    for (int o = 16; o >= 1; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
+
+template <int VEC>
+__global__ void __launch_bounds__(256) det_stats_kernel(const uint8_t* __restrict__ mask, const int* parent,
+                                                        const int* __restrict__ rank, int w, int h, int npx, CclList L,
+                                                        const int32_t* __restrict__ lab_area, int lab_stride,
+                                                        const float* __restrict__ flow, const mavd_imu* __restrict__ imu,
+                                                        mavd_detection* det, int max_det) {
+    pdl_entry();
+    const int warps = gridDim.x * 8, gw = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    const unsigned FULL = 0xffffffffu;
+    const int cnt = *L.count;
+    DetAcc acc;
+    int derot_f = -1;
+    Derot D{};
+    for (int q = gw; q < cnt; q += warps) {
+        const int e = L.entries[q];
+        const int f = e / L.n_units, u = e - f * L.n_units, ub = u * CCL_UNIT;
+        const size_t base = (size_t)f * npx;
+        UnitRuns R;
+        R.M = ccl_load_bits<VEC>(mask + base, ub, npx);
+        R.RS = row_starts(ub, w, R.x0);
+        unit_runs(R);
+        int lab[4], sl[4];
+        const int l0 = unit_labels(R, parent, rank, base, ub, lab);
+        bool any = false;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            sl[j] = -1;
+            if (lab[j] > 0) {
+                const int v = lab_area[(size_t)f * lab_stride + lab[j]];
+                if (v < 0) sl[j] = -v - 1;
+            }
+            any |= sl[j] >= 0;
+        }
+        if (!__any_sync(FULL, any)) continue;                 // no selected component in this unit
+        const int m0 = lab_area[(size_t)f * lab_stride + l0];
+        const int slot0 = m0 < 0 ? -m0 - 1 : -1;             // the entry the warp accumulates in registers
+        if (slot0 >= 0 && (f != acc.f || slot0 != acc.slot)) {
+            det_flush(acc, det, max_det);
+            acc.f = f; acc.slot = slot0;
+        }
+        int ax0 = 0x7fffffff, ay0 = 0x7fffffff, ax1 = -1, ay1 = -1, aarea = 0, asx = 0, asy = 0;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            if (sl[j] < 0) continue;
+            const int t = 32 * j + lane, g = ub + t;
+            const int len = first_set_at_or_above(R.E, t) - t + 1;
+            const int y = g / w, xs = g - y * w, xe = xs + len - 1;
+            const int sx = len * xs + len * (len - 1) / 2, sy = len * y;    // < 128 * 16384: no overflow
+            if (sl[j] == slot0) {
+                ax0 = min(ax0, xs); ay0 = min(ay0, y); ax1 = max(ax1, xe); ay1 = max(ay1, y);
+                aarea += len; asx += sx; asy += sy;
+            } else {
+                mavd_detection* d = det + (size_t)f * max_det + sl[j];
+                atomicMin(&d->box[0], xs); atomicMin(&d->box[1], y); atomicMax(&d->box[2], xe); atomicMax(&d->box[3], y);
+                atomicAdd(&d->area, len);
+                atomicAdd(reinterpret_cast<unsigned long long*>(&d->sum_x), (unsigned long long)sx);
+                atomicAdd(reinterpret_cast<unsigned long long*>(&d->sum_y), (unsigned long long)sy);
+            }
+        }
+        double fx = 0.0, fy = 0.0;
+        if (flow) {
+            if (f != derot_f) { D = make_derot(imu[f], w, h); derot_f = f; }
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                const int t = 32 * j + lane;
+                const bool on = (R.M.w[j] >> lane) & 1u;
+                const int s = on ? last_set_at_or_below(R.S, t) : 0;
+                int ps = -1;
+#pragma unroll
+                for (int jj = 0; jj < 4; ++jj) {
+                    const int v = __shfl_sync(FULL, sl[jj], s & 31);
+                    if ((s >> 5) == jj) ps = v;
+                }
+                if (!on || ps < 0) continue;
+                const int g = ub + t, y = g / w, x = g - y * w;
+                const float* p = flow + 2 * (base + g);
+                double v0 = (double)__ldg(p), v1 = (double)__ldg(p + 1);
+                if (D.on) {
+                    double r0, r1;
+                    derot_at(D, x, y, r0, r1);
+                    v0 = __dsub_rn(v0, r0);
+                    v1 = __dsub_rn(v1, r1);
+                }
+                if (ps == slot0) {
+                    fx = __dadd_rn(fx, v0);
+                    fy = __dadd_rn(fy, v1);
+                } else {
+                    mavd_detection* d = det + (size_t)f * max_det + ps;
+                    atomicAdd(&d->flow_sum[0], v0);
+                    atomicAdd(&d->flow_sum[1], v1);
+                }
+            }
+        }
+        if (slot0 >= 0) {
+            acc.x0 = min(acc.x0, __reduce_min_sync(FULL, ax0)); acc.y0 = min(acc.y0, __reduce_min_sync(FULL, ay0));
+            acc.x1 = max(acc.x1, __reduce_max_sync(FULL, ax1)); acc.y1 = max(acc.y1, __reduce_max_sync(FULL, ay1));
+            acc.area += __reduce_add_sync(FULL, aarea);
+            acc.sx += __reduce_add_sync(FULL, asx);
+            acc.sy += __reduce_add_sync(FULL, asy);
+            if (flow) {
+                acc.fx += warp_sum_f64(fx);
+                acc.fy += warp_sum_f64(fy);
+            }
+        }
+    }
+    det_flush(acc, det, max_det);
+}
+
+__global__ void det_final_kernel(mavd_detection* det, int total) {
+    pdl_entry();
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= total) return;
+    mavd_detection& d = det[i];
+    if (d.label == 0) return;
+    d.box[2] = d.box[2] - d.box[0] + 1;
+    d.box[3] = d.box[3] - d.box[1] + 1;
+}
+
 // scratch behind the rank array: [count (4 ints)] [unit_cnt: max_pairs x n_units] [entries: max_pairs x n_units]
 int ccl_n_units(mavd_handle H) { return ceil_div(H->cfg.width * H->cfg.height, CCL_UNIT); }
 static int* ccl_count_ptr(mavd_handle H) { return H->d_scan + (size_t)H->cfg.max_pairs * H->cfg.width * H->cfg.height; }
@@ -1821,7 +2153,7 @@ int ccl_list_reset(mavd_handle H, int n, cudaStream_t s, int lane) {
 template <int VEC>
 static int ccl_launch(mavd_handle H, const uint8_t* d_mask, int n, int* parent, int32_t* labels_out, int32_t* d_boxes,
                       size_t boxes_stride, int max_boxes, int32_t* d_n_labels, size_t nlabels_stride, cudaStream_t s,
-                      bool list_ready) {
+                      bool list_ready, const DetArgs* det) {
     const int w = H->cfg.width, h = H->cfg.height, npx = w * h;
     const int n_units = ccl_n_units(H);
     int* rank = H->d_scan;                     // [n][npx], written and read at roots only
@@ -1864,20 +2196,39 @@ static int ccl_launch(mavd_handle H, const uint8_t* d_mask, int n, int* parent, 
                                  boxes_stride, max_boxes, n));
         MAVD_LAUNCHED();
     }
+    if (det) {
+        const char* nl = reinterpret_cast<const char*>(d_n_labels);
+        MAVD_CUDA(launch_chained(pdl_next(H), det_area_zero_kernel, dim3(ceil_div(det->lab_stride, 256 * 8), n), 256, 0, s,
+                                 det->lab_area, det->lab_stride, nl, nlabels_stride));
+        MAVD_LAUNCHED();
+        MAVD_CUDA(launch_chained(pdl_next(H), det_area_kernel<VEC>, CCL_GRID, 256, 0, s, d_mask, parent, rank, w, npx, L,
+                                 det->lab_area, det->lab_stride));
+        MAVD_LAUNCHED();
+        MAVD_CUDA(launch_chained(pdl_next(H), det_select_kernel, n, 1024, 0, s, det->lab_area, det->lab_stride, nl,
+                                 nlabels_stride, det->det, det->max_det));
+        MAVD_LAUNCHED();
+        MAVD_CUDA(launch_chained(pdl_next(H), det_stats_kernel<VEC>, CCL_GRID, 256, 0, s, d_mask, parent, rank, w, h, npx, L,
+                                 det->lab_area, det->lab_stride, det->flow, det->imu, det->det, det->max_det));
+        MAVD_LAUNCHED();
+        MAVD_CUDA(launch_chained(pdl_next(H), det_final_kernel, ceil_div(n * det->max_det, 128), 128, 0, s, det->det,
+                                 n * det->max_det));
+        MAVD_LAUNCHED();
+    }
     return MAVD_OK;
 }
 
 // d_labels: the caller's label image (also used as the union-find array), or NULL when only the
 // component count / boxes are wanted (the handle's scratch then holds the union-find array).
 // list_ready: the producer of the mask already appended its occupied units (ccl_list_reset before it ran).
+// det (nullable): also the detection table of every frame (DetArgs, common.cuh).
 int ccl_run(mavd_handle H, const uint8_t* d_mask, int n, int32_t* d_labels, int32_t* d_boxes, size_t boxes_stride,
-            int max_boxes, int32_t* d_n_labels, size_t nlabels_stride, cudaStream_t s, bool list_ready) {
+            int max_boxes, int32_t* d_n_labels, size_t nlabels_stride, cudaStream_t s, bool list_ready, const DetArgs* det) {
     ProfScope ps(&H->prof, MAVD_PROF_CCL, s);
     const int w = H->cfg.width;
     int* parent = d_labels ? d_labels : H->d_labels;
     const bool vec4 = (w % 4 == 0) && ((reinterpret_cast<uintptr_t>(d_mask) & 3) == 0);
-    if (vec4) return ccl_launch<4>(H, d_mask, n, parent, d_labels, d_boxes, boxes_stride, max_boxes, d_n_labels, nlabels_stride, s, list_ready);
-    return ccl_launch<1>(H, d_mask, n, parent, d_labels, d_boxes, boxes_stride, max_boxes, d_n_labels, nlabels_stride, s, list_ready);
+    if (vec4) return ccl_launch<4>(H, d_mask, n, parent, d_labels, d_boxes, boxes_stride, max_boxes, d_n_labels, nlabels_stride, s, list_ready, det);
+    return ccl_launch<1>(H, d_mask, n, parent, d_labels, d_boxes, boxes_stride, max_boxes, d_n_labels, nlabels_stride, s, list_ready, det);
 }
 
 }  // namespace mavd

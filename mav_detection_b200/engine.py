@@ -10,7 +10,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import AuxInputs, Config, DetectParams, FarnebackParams, FrameRecord, FrameStats, Imu, Tuning, check
+from ._lib import AuxInputs, Config, DetectParams, Detection, FarnebackParams, FrameRecord, FrameStats, Imu, Tuning, check
 
 # cv2.calcOpticalFlowFarneback arguments used by the reference (src/farneback.py:78-80)
 REFERENCE_PARAMS = dict(pyr_scale=0.4, levels=1, winsize=12, iterations=10, poly_n=8, poly_sigma=1.2, flags=0)
@@ -19,6 +19,7 @@ SAMPLE_PARAMS = dict(pyr_scale=0.5, levels=5, winsize=15, iterations=3, poly_n=5
 
 RECORD_DTYPE = np.dtype(FrameRecord)
 STATS_DTYPE = np.dtype(FrameStats)
+DETECTION_DTYPE = np.dtype(Detection)
 
 
 def make_imu(n: int, ang: Optional[np.ndarray] = None, dt=None, derotate=None) -> C.Array:
@@ -357,14 +358,57 @@ class Engine:
                                 cnt.data_ptr(), self._stream()))
         return labels, boxes, cnt
 
+    def _det_count(self, max_det) -> int:
+        if isinstance(max_det, bool) or not isinstance(max_det, (int, np.integer)) or \
+                not 1 <= int(max_det) <= _lib.MAX_DETECTIONS:
+            raise ValueError('max_det must be an int in 1..%d' % _lib.MAX_DETECTIONS)
+        return int(max_det)
+
+    def _det_host(self, det: Optional[np.ndarray], n: int) -> Tuple[int, Optional[int]]:
+        """(max_det, pointer) of a host detection table: (n, max_det) DETECTION_DTYPE, C-contiguous (pinned for the
+        copy to be asynchronous)."""
+        if det is None:
+            return 0, None
+        if not isinstance(det, np.ndarray) or det.dtype != DETECTION_DTYPE or det.ndim != 2 or det.shape[0] < n or \
+                not det.flags['C_CONTIGUOUS']:
+            raise ValueError('detections must be a C-contiguous (n, max_det) array of DETECTION_DTYPE')
+        return self._det_count(det.shape[1]), det.ctypes.data
+
+    def detections(self, mask: torch.Tensor, flow: Optional[torch.Tensor] = None, imu=None,
+                   max_det: int = 32) -> torch.Tensor:
+        """Detection table of every (H, W) mask of an (n, H, W) uint8/bool CUDA tensor (non-zero = foreground): the
+        max_det largest 8-connected components by (area desc, label asc).  With a float32 (n, H, W, 2) flow and its imu
+        array, flow_sum is the derotated flow summed over each component.  Returns an (n, max_det, itemsize) uint8
+        CUDA tensor of mavd_detection (detections_to_numpy)."""
+        max_det = self._det_count(max_det)
+        if mask.dtype not in (torch.uint8, torch.bool) or not mask.is_cuda or not mask.is_contiguous() or \
+                tuple(mask.shape[1:]) != (self.height, self.width):
+            raise ValueError('mask must be a contiguous CUDA uint8/bool tensor (n, %d, %d)' % (self.height, self.width))
+        n = mask.shape[0]
+        if flow is not None:
+            if self._flow_kind(flow) != 0 or flow.shape[0] != n:
+                raise ValueError('flow must be float32 (%d, %d, %d, 2)' % (n, self.height, self.width))
+            if imu is None:
+                raise ValueError('a flow needs its imu array')
+        out = torch.empty((n, max_det, DETECTION_DTYPE.itemsize), dtype=torch.uint8, device=self.device)
+        check(self.lib.mavd_detections(self._h, mask.data_ptr(), n, _ptr(flow), imu, max_det, out.data_ptr(),
+                                       self._stream()))
+        return out
+
+    @staticmethod
+    def detections_to_numpy(det: torch.Tensor) -> np.ndarray:
+        """(n, max_det, itemsize) uint8 tensor -> (n, max_det) DETECTION_DTYPE array."""
+        return det.cpu().numpy().view(DETECTION_DTYPE)[..., 0]
+
     # -- whole path ----------------------------------------------------------------------------
     def process(self, frames: torch.Tensor, imu, samples: torch.Tensor, n_pairs: Optional[int] = None,
                 pair_stride: int = 1, sky: Optional[torch.Tensor] = None, seg: Optional[torch.Tensor] = None,
                 flow_out: Optional[torch.Tensor] = None, total_out: Optional[torch.Tensor] = None,
                 fixed_out: Optional[torch.Tensor] = None, records: Optional[torch.Tensor] = None,
-                gt_flow: Optional[torch.Tensor] = None) -> torch.Tensor:
+                gt_flow: Optional[torch.Tensor] = None, detections: Optional[int] = None):
         """Farneback -> derotate -> FoE -> phi/masks -> components, device buffers in and out.
-        Returns the (n_pairs, sizeof(mavd_frame_record)) uint8 CUDA tensor of records."""
+        Returns the (n_pairs, sizeof(mavd_frame_record)) uint8 CUDA tensor of records; with detections = max_det,
+        (records, the (n_pairs, max_det, itemsize) uint8 CUDA tensor of each pair's detection table)."""
         if n_pairs is None:
             n_pairs = frames.shape[0] - 1 if pair_stride == 1 else frames.shape[0] // 2
         self._check_frames(frames, n_pairs, pair_stride)
@@ -372,6 +416,14 @@ class Engine:
         if records is None:
             records = torch.empty((n_pairs, RECORD_DTYPE.itemsize), dtype=torch.uint8, device=self.device)
         aux = self._aux(sky, seg, gt_flow, n_pairs)
+        if detections is not None:
+            max_det = self._det_count(detections)
+            det = torch.empty((n_pairs, max_det, DETECTION_DTYPE.itemsize), dtype=torch.uint8, device=self.device)
+            check(self.lib.mavd_process_det(self._h, frames.data_ptr(), n_pairs, pair_stride, imu,
+                                            C.byref(self.detect_params), samples.data_ptr(), C.byref(aux),
+                                            _ptr(flow_out), _ptr(total_out), _ptr(fixed_out), records.data_ptr(),
+                                            max_det, det.data_ptr(), self._stream()))
+            return records, det
         check(self.lib.mavd_process_ex(self._h, frames.data_ptr(), n_pairs, pair_stride, imu,
                                        C.byref(self.detect_params), samples.data_ptr(), C.byref(aux),
                                        _ptr(flow_out), _ptr(total_out), _ptr(fixed_out), records.data_ptr(),
@@ -381,8 +433,9 @@ class Engine:
     def detect(self, flow: torch.Tensor, imu, samples: torch.Tensor, sky: Optional[torch.Tensor] = None,
                seg: Optional[torch.Tensor] = None, total_out: Optional[torch.Tensor] = None,
                fixed_out: Optional[torch.Tensor] = None, records: Optional[torch.Tensor] = None,
-               gt_flow: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """derotate -> FoE -> phi/masks -> components from a given float32 flow (the Dataset.get_flow_uv seam)."""
+               gt_flow: Optional[torch.Tensor] = None, detections: Optional[int] = None):
+        """derotate -> FoE -> phi/masks -> components from a given float32 flow (the Dataset.get_flow_uv seam).
+        detections = max_det: returns (records, detection tables) as process does."""
         n = flow.shape[0]
         if flow.dtype != torch.float32 or not flow.is_cuda or not flow.is_contiguous() or \
                 tuple(flow.shape[1:]) != (self.height, self.width, 2):
@@ -391,6 +444,13 @@ class Engine:
         if records is None:
             records = torch.empty((n, RECORD_DTYPE.itemsize), dtype=torch.uint8, device=self.device)
         aux = self._aux(sky, seg, gt_flow, n)
+        if detections is not None:
+            max_det = self._det_count(detections)
+            det = torch.empty((n, max_det, DETECTION_DTYPE.itemsize), dtype=torch.uint8, device=self.device)
+            check(self.lib.mavd_detect_det(self._h, flow.data_ptr(), n, imu, C.byref(self.detect_params),
+                                           samples.data_ptr(), C.byref(aux), _ptr(total_out), _ptr(fixed_out),
+                                           records.data_ptr(), max_det, det.data_ptr(), self._stream()))
+            return records, det
         check(self.lib.mavd_detect_ex(self._h, flow.data_ptr(), n, imu, C.byref(self.detect_params), samples.data_ptr(),
                                       C.byref(aux), _ptr(total_out), _ptr(fixed_out), records.data_ptr(),
                                       self._stream()))
@@ -435,22 +495,30 @@ class Engine:
                     flow_out: Optional[np.ndarray] = None, fixed_out: Optional[np.ndarray] = None,
                     records: Optional[np.ndarray] = None, gt_flow: Optional[np.ndarray] = None,
                     seg_packed: bool = False, sky_packed: bool = False, fixed_packed: bool = False,
-                    copy_only: bool = False) -> np.ndarray:
+                    copy_only: bool = False, detections: Optional[np.ndarray] = None) -> np.ndarray:
         """Asynchronous process_host: returns at once; the outputs are valid after wait_host(slot).  Keeping
         up to _lib.HOST_SLOTS batches in flight overlaps the host<->device copies with the compute.
         seg_packed / sky_packed: the masks are given at 1 bit per pixel (pack_mask_host); fixed_packed: fixed_out
-        receives (n, packed_mask_bytes) bits; copy_only: move the bytes but skip the compute (host-feed ceiling)."""
+        receives (n, packed_mask_bytes) bits; copy_only: move the bytes but skip the compute (host-feed ceiling);
+        detections: an (n, max_det) DETECTION_DTYPE host array (pinned) that receives each pair's detection table."""
         n_pairs, records = self._host_args(frames, samples, n_pairs, pair_stride, flow_out, fixed_out, records,
                                            fixed_packed)
         aux = self._aux(sky, seg, gt_flow, n_pairs, host=True, sky_packed=sky_packed, seg_packed=seg_packed)
         flags = (_lib.HOST_BGR if frames.ndim == 4 else 0) | (_lib.HOST_SEG_PACKED if seg_packed else 0) | \
             (_lib.HOST_SKY_PACKED if sky_packed else 0) | (_lib.HOST_FIXED_PACKED if fixed_packed else 0) | \
             (_lib.HOST_COPY_ONLY if copy_only else 0)
-        check(self.lib.mavd_submit_host_ex(self._h, slot, _hp(frames), n_pairs, pair_stride, imu,
-                                           C.byref(self.detect_params), _hp(samples), C.byref(aux), flags,
-                                           _hp(flow_out), _hp(fixed_out), records.ctypes.data, self._stream()))
+        max_det, det = self._det_host(detections, n_pairs)
+        if det is None:
+            check(self.lib.mavd_submit_host_ex(self._h, slot, _hp(frames), n_pairs, pair_stride, imu,
+                                               C.byref(self.detect_params), _hp(samples), C.byref(aux), flags,
+                                               _hp(flow_out), _hp(fixed_out), records.ctypes.data, self._stream()))
+        else:
+            check(self.lib.mavd_submit_host_det(self._h, slot, _hp(frames), n_pairs, pair_stride, imu,
+                                                C.byref(self.detect_params), _hp(samples), C.byref(aux), flags,
+                                                _hp(flow_out), _hp(fixed_out), records.ctypes.data, max_det, det,
+                                                self._stream()))
         # keep the host buffers alive until the wait
-        self._inflight[slot] = (frames, imu, samples, sky, seg, gt_flow, flow_out, fixed_out, records)
+        self._inflight[slot] = (frames, imu, samples, sky, seg, gt_flow, flow_out, fixed_out, records, detections)
         return records
 
     def wait_host(self, slot: int) -> None:
@@ -460,9 +528,10 @@ class Engine:
     def detect_host(self, flow: np.ndarray, imu, samples: np.ndarray, sky: Optional[np.ndarray] = None,
                     seg: Optional[np.ndarray] = None, fixed_out: Optional[np.ndarray] = None,
                     records: Optional[np.ndarray] = None, gt_flow: Optional[np.ndarray] = None,
-                    seg_packed: bool = False, sky_packed: bool = False, fixed_packed: bool = False) -> np.ndarray:
+                    seg_packed: bool = False, sky_packed: bool = False, fixed_packed: bool = False,
+                    detections: Optional[np.ndarray] = None) -> np.ndarray:
         """Detection from a HOST float32 flow (n, H, W, 2): what Processor.run_detection does with
-        Dataset.get_flow_uv (processor.py:305-362)."""
+        Dataset.get_flow_uv (processor.py:305-362).  detections: as in submit_host."""
         if flow.dtype != np.float32 or tuple(flow.shape[1:]) != (self.height, self.width, 2) or \
                 not flow.flags['C_CONTIGUOUS']:
             raise ValueError('flow must be C-contiguous float32 (n, %d, %d, 2)' % (self.height, self.width))
@@ -470,9 +539,15 @@ class Engine:
         aux = self._aux(sky, seg, gt_flow, n, host=True, sky_packed=sky_packed, seg_packed=seg_packed)
         flags = (_lib.HOST_SEG_PACKED if seg_packed else 0) | (_lib.HOST_SKY_PACKED if sky_packed else 0) | \
             (_lib.HOST_FIXED_PACKED if fixed_packed else 0)
-        check(self.lib.mavd_detect_host_ex(self._h, flow.ctypes.data, n, imu, C.byref(self.detect_params),
-                                           _hp(samples), C.byref(aux), flags, _hp(fixed_out), records.ctypes.data,
-                                           self._stream()))
+        max_det, det = self._det_host(detections, n)
+        if det is None:
+            check(self.lib.mavd_detect_host_ex(self._h, flow.ctypes.data, n, imu, C.byref(self.detect_params),
+                                               _hp(samples), C.byref(aux), flags, _hp(fixed_out), records.ctypes.data,
+                                               self._stream()))
+        else:
+            check(self.lib.mavd_detect_host_det(self._h, flow.ctypes.data, n, imu, C.byref(self.detect_params),
+                                                _hp(samples), C.byref(aux), flags, _hp(fixed_out), records.ctypes.data,
+                                                max_det, det, self._stream()))
         return records
 
     @staticmethod

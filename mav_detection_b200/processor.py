@@ -15,7 +15,7 @@ from __future__ import annotations
 
 import json
 import os
-from typing import Any, Dict, List, Optional, Tuple
+from typing import Any, Dict, List, NamedTuple, Optional, Tuple
 
 import numpy as np
 
@@ -46,12 +46,35 @@ def to_gray(frame: np.ndarray) -> np.ndarray:
     raise ValueError('frames must be (H, W) gray or (H, W, 3) BGR uint8')
 
 
+class Detection(NamedTuple):
+    """One component of a frame's estimate_fixed mask (include/mavd.h: mavd_detection): box (left, top, width,
+    height), area in pixels, centroid (x, y) and the mean derotated flow (u, v) over its pixels."""
+    label: int
+    box: Tuple[int, int, int, int]
+    area: int
+    centroid: Tuple[float, float]
+    flow: Tuple[float, float]
+
+
+def detections_from_table(table: np.ndarray) -> List[Detection]:
+    """The used entries of one frame's (max_det,) DETECTION_DTYPE table, largest component first."""
+    out = []
+    for d in table:
+        if d['label'] == 0:
+            break
+        a = int(d['area'])
+        out.append(Detection(int(d['label']), tuple(int(v) for v in d['box']), a,
+                             (int(d['sum_x']) / a, int(d['sum_y']) / a),
+                             (float(d['flow_sum'][0]) / a, float(d['flow_sum'][1]) / a)))
+    return out
+
+
 class Processor:
     """Acts as detector over one sequence (the dataset-conversion half of the reference class is out of scope)."""
 
     def __init__(self, config: RunConfig, flow_source: str = 'dataset', batch_frames: int = 8,
                  farneback_params: Optional[Dict] = None, engine: Any = None, write_results: bool = True,
-                 flow_cache: Any = None) -> None:
+                 flow_cache: Any = None, max_detections: int = 0) -> None:
         if flow_source not in ('dataset', 'farneback'):
             raise ValueError("flow_source must be 'dataset' or 'farneback'")
         self.config = config
@@ -66,6 +89,12 @@ class Processor:
         # flow_source 'farneback' + flow_cache (a flow_cache.FloCache): every computed flow field is also written as
         # <cache dir>/<frame index:06d>.flo, the files Dataset.get_flow_uv reads (datasets/dataset.py:205-212)
         self.flow_cache = flow_cache
+        # max_detections > 0: run_detection also lists each frame's max_detections largest components of
+        # estimate_fixed in self.detections[frame index] (Detection objects, largest first)
+        self.max_detections = int(max_detections)
+        if not 0 <= self.max_detections <= 256:
+            raise ValueError('max_detections must be in 0..256')
+        self.detections: Dict[int, List[Detection]] = dict()
         width, height = self.dataset.capture_size
         if engine is None:
             from . import engine as engine_mod
@@ -187,16 +216,24 @@ class Processor:
         eng = self.engine
         width, height = self.dataset.capture_size
         B = self.batch_frames
-        inflight: List[tuple] = []   # (slot, indices, records, sky, gt?, flow)
+        inflight: List[tuple] = []   # (slot, indices, records, sky, gt?, flow, detection tables)
         slot = 0
+        D = self.max_detections
+
+        def det_tables(s: int, n: int) -> Optional[np.ndarray]:
+            from .engine import DETECTION_DTYPE
+            return self._pinned(s, 'detections', (n, D), DETECTION_DTYPE) if D else None
 
         def finish(entry) -> None:
-            s, indices, records, sky, has_gt, flow = entry
+            s, indices, records, sky, has_gt, flow, det = entry
             if s >= 0:
                 eng.wait_host(s)
             if flow is not None:
                 for k, i in enumerate(indices):           # frame_step_size may skip indices: one file per frame
                     self.flow_cache.put_batch(i, flow[k:k + 1])
+            if det is not None:
+                for k, i in enumerate(indices):
+                    self.detections[i] = detections_from_table(det[k])
             for k, i in enumerate(indices):
                 fr = self._frame_result(i, records[k], sky[k], has_gt)
                 self.detection_results[i] = fr
@@ -218,9 +255,10 @@ class Processor:
                     flows[k] = f
                 imu, samples, sky, seg, gt = self._host_inputs(indices, 0)
                 records = self._pinned(0, 'records', (n,), eng_records_dtype())
+                det = det_tables(0, n)
                 self.focus_of_expansion._eng()                   # its FoE thresholds -> eng.detect_params (shared engine)
-                eng.detect_host(flows, imu, samples, sky=sky, seg=seg, gt_flow=gt, records=records)
-                finish((-1, indices, records, sky, gt is not None, None))
+                eng.detect_host(flows, imu, samples, sky=sky, seg=seg, gt_flow=gt, records=records, detections=det)
+                finish((-1, indices, records, sky, gt is not None, None, det))
             else:
                 # flow(i) = Farneback(frame i, frame i+1); consecutive batches share one frame
                 if len(inflight) == HOST_SLOTS - 1:
@@ -235,10 +273,11 @@ class Processor:
                 records = self._pinned(slot, 'records', (n,), eng_records_dtype())
                 flow = self._pinned(slot, 'flow_out', (n, height, width, 2), np.float32) if self.flow_cache is not None \
                     else None
+                det = det_tables(slot, n)
                 self.focus_of_expansion._eng()                   # the call copies detect_params: batches in flight keep theirs
                 eng.submit_host(slot, frames, imu, samples, n_pairs=n, sky=sky, seg=seg, gt_flow=gt, flow_out=flow,
-                                records=records)
-                inflight.append((slot, indices, records, sky, gt is not None, flow))
+                                records=records, detections=det)
+                inflight.append((slot, indices, records, sky, gt is not None, flow, det))
                 slot = (slot + 1) % HOST_SLOTS
             self.frame_index = indices[-1] + self.frame_step_size
             n10 = int(self.dataset.N / 10)
