@@ -169,6 +169,34 @@ typedef struct mavd_detection {
                              rounding of the summation order, not bit for bit */
 } mavd_detection;        /* 56 bytes */
 
+/* Arguments of cv2.goodFeaturesToTrack(image, maxCorners, qualityLevel, minDistance, mask, blockSize, gradientSize)
+ * (Shi-Tomasi corners; the Harris detector is not supported). */
+typedef struct mavd_gftt_params {
+    int32_t max_corners;     /* corners written per frame (>= 0); the count returned is never limited */
+    double quality_level;    /* > 0 */
+    double min_distance;     /* >= 0 */
+    int32_t block_size;      /* 1..31 */
+    int32_t gradient_size;   /* 3 */
+} mavd_gftt_params;
+
+/* cv2 flag and termination-criteria values of mavd_lk_params */
+#define MAVD_LK_GET_MIN_EIGENVALS 8 /* cv2.OPTFLOW_LK_GET_MIN_EIGENVALS: err = the window's minimum eigenvalue */
+#define MAVD_LK_MAX_LEVEL 16        /* largest max_level accepted (levels smaller than the window are never used) */
+#define MAVD_TERM_COUNT 1           /* cv2.TERM_CRITERIA_COUNT */
+#define MAVD_TERM_EPS 2             /* cv2.TERM_CRITERIA_EPS */
+
+/* Arguments of cv2.calcOpticalFlowPyrLK(prev, next, prevPts, None, winSize, maxLevel, criteria, flags,
+ * minEigThreshold).  OPTFLOW_USE_INITIAL_FLOW is not supported. */
+typedef struct mavd_lk_params {
+    int32_t win_w, win_h;     /* 3..63 each */
+    int32_t max_level;        /* 0..MAVD_LK_MAX_LEVEL */
+    int32_t criteria_type;    /* MAVD_TERM_COUNT | MAVD_TERM_EPS bits: without COUNT 30 iterations, without EPS 0.01 */
+    int32_t criteria_count;   /* clamped to 0..100 */
+    double criteria_eps;      /* clamped to 0..10 */
+    int32_t flags;            /* 0 or MAVD_LK_GET_MIN_EIGENVALS */
+    double min_eig_threshold;
+} mavd_lk_params;
+
 typedef struct mavd_handle_s* mavd_handle;
 
 /* ---- library ---- */
@@ -387,6 +415,26 @@ int mavd_detect_host_det(mavd_handle h, const float* h_flow, int32_t n, const ma
                          const mavd_detect_params* prm, const int32_t* h_samples, const mavd_aux_inputs* h_aux,
                          int32_t flags, uint8_t* h_fixed_out, mavd_frame_record* h_records, int32_t max_det,
                          mavd_detection* h_det, void* stream);
+
+/* ---- sparse features: cv2.goodFeaturesToTrack and cv2.calcOpticalFlowPyrLK (the LucasKanade class's calls) ----
+ * mavd_good_features_to_track: Shi-Tomasi corners of n_frames dense (H, W) uint8 frames (n_frames <= 2 * max_pairs).
+ * d_corners: n_frames x max_corners x 2 float32 (x, y) in cv2's order; d_count[i] is frame i's corner count WITHOUT a
+ * limit, and min(count, max_corners) entries are written (the rest of the row is zero).  d_mask (nullable): (H, W) uint8,
+ * mask_stride bytes between frames (0 = one mask for every frame).  d_eig (nullable): n_frames x (H, W) float32
+ * cv2.cornerMinEigenVal images, bit for bit.  d_corners may be NULL when max_corners is 0.
+ * The first call allocates the corner workspace: about 50 bytes per pixel for 16 frames. */
+int mavd_good_features_to_track(mavd_handle h, const uint8_t* d_frames, int32_t n_frames, const mavd_gftt_params* prm,
+                                const uint8_t* d_mask, int64_t mask_stride, float* d_corners, int32_t* d_count,
+                                float* d_eig, void* stream);
+/* mavd_pyr_lk: pair p tracks d_prev_pts[p] (n_points x 2 float32) from frame p*pair_stride to frame p*pair_stride+1
+ * (pair_stride 1 or 2, as in mavd_farneback).  d_n_points (nullable): n_pairs int32 counts, points past a pair's count
+ * are not tracked (next (0, 0), status 0, err 0); mavd_good_features_to_track's d_count feeds it directly.
+ * d_next_pts: n_pairs x n_points x 2 float32, d_status: uint8, d_err: float32 (cv2's err; 0 where cv2 leaves it
+ * unset).  Non-finite points get status 0 and err 0.  The first call allocates the pyramid workspace: about 6 bytes per
+ * pixel per frame (2 * max_pairs frames). */
+int mavd_pyr_lk(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int32_t pair_stride, const mavd_lk_params* prm,
+                const float* d_prev_pts, int32_t n_points, const int32_t* d_n_points, float* d_next_pts,
+                uint8_t* d_status, float* d_err, void* stream);
 
 /* ---- 1-bit-per-pixel masks on the wire (ground-truth segmentation in, estimate_fixed out) ----
  * Bytes one packed (H, W) mask occupies: ceil(H*W / 8) rounded up to a multiple of 4.  Bit k of byte j is pixel

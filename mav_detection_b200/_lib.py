@@ -17,6 +17,9 @@ MAX_BOXES = 32
 HOST_SLOTS = 3
 MAX_DETECTIONS = 256
 OPTFLOW_FARNEBACK_GAUSSIAN = 256
+LK_GET_MIN_EIGENVALS = 8
+LK_MAX_LEVEL = 16
+TERM_COUNT, TERM_EPS = 1, 2
 
 
 class FarnebackParams(C.Structure):
@@ -56,6 +59,19 @@ class Detection(C.Structure):
     """One entry of a frame's detection table (include/mavd.h: mavd_detection)."""
     _fields_ = [('label', C.c_int32), ('box', C.c_int32 * 4), ('area', C.c_int32), ('sum_x', C.c_int64),
                 ('sum_y', C.c_int64), ('flow_sum', C.c_double * 2)]
+
+
+class GfttParams(C.Structure):
+    """Arguments of cv2.goodFeaturesToTrack (include/mavd.h: mavd_gftt_params)."""
+    _fields_ = [('max_corners', C.c_int32), ('quality_level', C.c_double), ('min_distance', C.c_double),
+                ('block_size', C.c_int32), ('gradient_size', C.c_int32)]
+
+
+class LkParams(C.Structure):
+    """Arguments of cv2.calcOpticalFlowPyrLK (include/mavd.h: mavd_lk_params)."""
+    _fields_ = [('win_w', C.c_int32), ('win_h', C.c_int32), ('max_level', C.c_int32), ('criteria_type', C.c_int32),
+                ('criteria_count', C.c_int32), ('criteria_eps', C.c_double), ('flags', C.c_int32),
+                ('min_eig_threshold', C.c_double)]
 
 
 class Tuning(C.Structure):
@@ -137,6 +153,9 @@ SIGNATURES = {
                                        _P, C.POINTER(AuxInputs), C.c_int32, _P, _P, _P, C.c_int32, _P, _P]),
     'mavd_detect_host_det': (C.c_int, [_P, _P, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams), _P,
                                        C.POINTER(AuxInputs), C.c_int32, _P, _P, C.c_int32, _P, _P]),
+    'mavd_good_features_to_track': (C.c_int, [_P, _P, C.c_int32, C.POINTER(GfttParams), _P, C.c_int64, _P, _P, _P,
+                                               _P]),
+    'mavd_pyr_lk': (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(LkParams), _P, C.c_int32, _P, _P, _P, _P, _P]),
     'mavd_packed_mask_bytes': (C.c_int64, [C.c_int32, C.c_int32]),
     'mavd_pack_mask': (C.c_int, [_P, C.c_int32, C.c_int64, _P, _P]),
     'mavd_unpack_mask': (C.c_int, [_P, C.c_int32, C.c_int64, C.c_uint8, _P, _P]),

@@ -8,7 +8,7 @@ import subprocess
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 INCLUDE = os.path.join(os.path.dirname(HERE), 'include')
-SOURCES = ['api.cu', 'farneback.cu', 'detect.cu']
+SOURCES = ['api.cu', 'farneback.cu', 'detect.cu', 'sparse.cu']
 OUT = os.path.join(CSRC, 'libmavd.so')
 
 

@@ -782,6 +782,100 @@ int mavd_detections(mavd_handle h, const uint8_t* d_mask, int32_t n, const float
     return ccl_run(h, d_mask, n, nullptr, nullptr, 0, 0, h->d_det_nlabels, sizeof(int32_t), s, false, &da);
 }
 
+// The corner workspace of mavd::gftt_chunk() frames, carved from one allocation made by the first corner call.
+static GfttWork gftt_work(mavd_handle h) {
+    const int W = h->cfg.width, Hh = h->cfg.height, G = gftt_chunk();
+    const size_t npx = (size_t)W * Hh;
+    char* p = (char*)h->sp_gftt;
+    GfttWork w;
+    w.rows = (double*)p;                  p += sizeof(double) * 3 * npx * G;
+    w.keys = (unsigned long long*)p;      p += sizeof(unsigned long long) * gftt_key_cap(W, Hh) * G;
+    w.cov = (float3*)p;                   p += sizeof(float3) * npx * G;
+    w.eig = (float*)p;                    p += sizeof(float) * npx * G;
+    w.grid = (int*)p;                     p += sizeof(int) * gftt_grid_cap(W, Hh) * G;
+    w.maxv = (uint32_t*)p;                p += sizeof(uint32_t) * G;
+    w.n_cand = (int*)p;
+    return w;
+}
+
+static size_t gftt_work_bytes(mavd_handle h) {
+    const int W = h->cfg.width, Hh = h->cfg.height, G = gftt_chunk();
+    const size_t npx = (size_t)W * Hh;
+    return (sizeof(double) * 3 * npx + sizeof(unsigned long long) * gftt_key_cap(W, Hh) + sizeof(float3) * npx +
+            sizeof(float) * npx + sizeof(int) * gftt_grid_cap(W, Hh) + sizeof(uint32_t) + sizeof(int)) * G;
+}
+
+int mavd_good_features_to_track(mavd_handle h, const uint8_t* d_frames, int32_t n_frames, const mavd_gftt_params* prm,
+                                const uint8_t* d_mask, int64_t mask_stride, float* d_corners, int32_t* d_count,
+                                float* d_eig, void* stream) {
+    DeviceGuard dg(h ? h->cfg.device : -1);
+    MAVD_REQUIRE(h != nullptr && prm != nullptr, MAVD_ERR_INVALID, "good_features_to_track: NULL argument");
+    const mavd_gftt_params p = *prm;
+    MAVD_REQUIRE(n_frames >= 0 && n_frames <= h->max_frames, MAVD_ERR_INVALID,
+                 "good_features_to_track: %d frames exceed the handle's %d", n_frames, h->max_frames);
+    MAVD_REQUIRE(!std::isnan(p.quality_level) && !std::isnan(p.min_distance), MAVD_ERR_INVALID,
+                 "good_features_to_track: NaN parameter");
+    MAVD_REQUIRE(p.max_corners >= 0, MAVD_ERR_INVALID, "good_features_to_track: max_corners %d < 0", p.max_corners);
+    MAVD_REQUIRE(mask_stride >= 0, MAVD_ERR_INVALID, "good_features_to_track: negative mask stride");
+    MAVD_REQUIRE(p.block_size >= 1 && p.block_size <= 31, MAVD_ERR_UNSUPPORTED,
+                 "good_features_to_track: block_size %d outside 1..31", p.block_size);
+    MAVD_REQUIRE(p.gradient_size == 3, MAVD_ERR_UNSUPPORTED, "good_features_to_track: gradient_size must be 3");
+    MAVD_REQUIRE(p.quality_level > 0, MAVD_ERR_UNSUPPORTED, "good_features_to_track: quality_level must be > 0");
+    MAVD_REQUIRE(p.min_distance >= 0 && std::isfinite(p.min_distance), MAVD_ERR_UNSUPPORTED,
+                 "good_features_to_track: min_distance must be finite and >= 0");
+    MAVD_REQUIRE(std::isfinite(p.quality_level), MAVD_ERR_UNSUPPORTED, "good_features_to_track: infinite quality_level");
+    if (n_frames == 0) return MAVD_OK;
+    MAVD_REQUIRE(d_frames && d_count && (d_corners || p.max_corners == 0), MAVD_ERR_INVALID,
+                 "good_features_to_track: NULL buffer");
+    if (!h->sp_gftt) {
+        mavd_handle_full* H = static_cast<mavd_handle_full*>(h);
+        char* base = nullptr;
+        TRY(H->arena.alloc(&base, gftt_work_bytes(h)));
+        H->sp_gftt = base;
+        H->bytes = H->arena.bytes;
+    }
+    return gftt_run(h, gftt_work(h), d_frames, n_frames, p, d_mask, d_mask ? mask_stride : 0, d_corners, d_count, d_eig,
+                    (cudaStream_t)stream);
+}
+
+int mavd_pyr_lk(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int32_t pair_stride, const mavd_lk_params* prm,
+                const float* d_prev_pts, int32_t n_points, const int32_t* d_n_points, float* d_next_pts,
+                uint8_t* d_status, float* d_err, void* stream) {
+    DeviceGuard dg(h ? h->cfg.device : -1);
+    MAVD_REQUIRE(h != nullptr && prm != nullptr, MAVD_ERR_INVALID, "pyr_lk: NULL argument");
+    const mavd_lk_params p = *prm;
+    MAVD_REQUIRE(n_pairs >= 0 && n_pairs <= h->cfg.max_pairs, MAVD_ERR_INVALID, "pyr_lk: batch %d exceeds max_pairs %d",
+                 n_pairs, h->cfg.max_pairs);
+    MAVD_REQUIRE(pair_stride == 1 || pair_stride == 2, MAVD_ERR_INVALID, "pair_stride must be 1 or 2");
+    MAVD_REQUIRE(n_points >= 0 && n_points <= (1 << 24), MAVD_ERR_INVALID, "pyr_lk: n_points %d outside 0..2^24",
+                 n_points);
+    MAVD_REQUIRE(!std::isnan(p.criteria_eps) && !std::isnan(p.min_eig_threshold), MAVD_ERR_INVALID,
+                 "pyr_lk: NaN parameter");
+    MAVD_REQUIRE(p.win_w >= 3 && p.win_w <= 63 && p.win_h >= 3 && p.win_h <= 63, MAVD_ERR_UNSUPPORTED,
+                 "pyr_lk: window %d x %d outside 3..63", p.win_w, p.win_h);
+    MAVD_REQUIRE(p.max_level >= 0 && p.max_level <= MAVD_LK_MAX_LEVEL, MAVD_ERR_UNSUPPORTED,
+                 "pyr_lk: max_level %d outside 0..%d", p.max_level, MAVD_LK_MAX_LEVEL);
+    MAVD_REQUIRE(p.flags == 0 || p.flags == MAVD_LK_GET_MIN_EIGENVALS, MAVD_ERR_UNSUPPORTED,
+                 "pyr_lk: flags %d not supported (0 or MAVD_LK_GET_MIN_EIGENVALS)", p.flags);
+    MAVD_REQUIRE((p.criteria_type & ~(MAVD_TERM_COUNT | MAVD_TERM_EPS)) == 0, MAVD_ERR_UNSUPPORTED,
+                 "pyr_lk: criteria_type %d not supported", p.criteria_type);
+    if (n_pairs == 0 || n_points == 0) return MAVD_OK;
+    MAVD_REQUIRE(d_frames && d_prev_pts && d_next_pts && d_status && d_err, MAVD_ERR_INVALID, "pyr_lk: NULL buffer");
+    if (!h->sp_pyr) {
+        mavd_handle_full* H = static_cast<mavd_handle_full*>(h);
+        const int W = h->cfg.width, Hh = h->cfg.height;
+        uint8_t* pyr = nullptr;
+        short2* der = nullptr;
+        TRY(H->arena.alloc(&pyr, (size_t)h->max_frames * lk_pyr_frame_bytes(W, Hh)));
+        TRY(H->arena.alloc(&der, (size_t)h->max_frames * lk_der_frame_elems(W, Hh)));
+        H->sp_pyr = pyr;
+        H->sp_der = der;
+        H->bytes = H->arena.bytes;
+    }
+    return lk_run(h, h->sp_pyr, h->sp_der, d_frames, n_pairs, pair_stride, p, d_prev_pts, n_points, d_n_points,
+                  d_next_pts, d_status, d_err, (cudaStream_t)stream);
+}
+
 int mavd_ccl(mavd_handle h, const uint8_t* d_mask, int32_t n, int32_t* d_labels, int32_t* d_boxes, int32_t max_boxes,
              int32_t* d_n_labels, void* stream) {
     DeviceGuard dg(h ? h->cfg.device : -1);

@@ -218,6 +218,10 @@ struct mavd_handle_s {
     // detection tables (allocated by the first call that asks for one: mavd_workspace_bytes is unchanged otherwise)
     int32_t* d_det_area = nullptr;  // [max_pairs][det_lab_stride]: area per label, then -(slot + 1) of a selected label
     int32_t* d_det_nlabels = nullptr;   // [max_pairs] label counts of mavd_detections
+    // sparse features (allocated by the first call that needs them: mavd_workspace_bytes is unchanged otherwise)
+    void* sp_gftt = nullptr;        // corner workspace of mavd::gftt_chunk() frames (sparse.cu: gftt_run)
+    uint8_t* sp_pyr = nullptr;      // [max_frames] pyramid levels 1.. of mavd_pyr_lk
+    short2* sp_der = nullptr;       // [max_frames] int16 Scharr derivatives of every level
     // host-path staging: MAVD_HOST_SLOTS independent sets of device buffers + the streams/events that let
     // the H2D of one batch, the compute of the previous one and the D2H of the one before overlap
     struct HostSlot {
@@ -340,4 +344,25 @@ static inline int det_lab_stride(mavd_handle h) { return ((h->cfg.width + 1) / 2
 int ccl_run(mavd_handle h, const uint8_t* d_mask, int n, int32_t* d_labels, int32_t* d_boxes, size_t boxes_stride,
             int max_boxes, int32_t* d_n_labels, size_t nlabels_stride_bytes, cudaStream_t s, bool list_ready = false,
             const DetArgs* det = nullptr);
+// sparse.cu: corners and pyramidal Lucas-Kanade
+struct GfttWork {
+    float3* cov;                    // [chunk][H][W] products of the Sobel derivatives
+    double* rows;                   // [chunk][H][W][3] row sums of the block
+    float* eig;                     // [chunk][H][W] when the caller wants no eig image
+    unsigned long long* keys;       // [chunk][gftt_key_cap] candidates
+    int* grid;                      // [chunk][gftt_grid_cap] accepted corners by cell
+    uint32_t* maxv;                 // [chunk]
+    int* n_cand;                    // [chunk]
+};
+size_t gftt_key_cap(int W, int H);
+size_t gftt_grid_cap(int W, int H);
+int gftt_chunk();
+int gftt_run(mavd_handle h, const GfttWork& ws, const uint8_t* d_frames, int n, const mavd_gftt_params& p,
+             const uint8_t* d_mask, int64_t mask_stride, float* d_corners, int32_t* d_count, float* d_eig,
+             cudaStream_t s);
+size_t lk_pyr_frame_bytes(int W, int H);
+size_t lk_der_frame_elems(int W, int H);
+int lk_run(mavd_handle h, uint8_t* pyr, short2* der, const uint8_t* d_frames, int n_pairs, int pair_stride,
+           const mavd_lk_params& p, const float* d_prev, int n_points, const int32_t* d_n_points, float* d_next,
+           uint8_t* d_status, float* d_err, cudaStream_t s);
 }  // namespace mavd

@@ -400,6 +400,65 @@ class Engine:
         """(n, max_det, itemsize) uint8 tensor -> (n, max_det) DETECTION_DTYPE array."""
         return det.cpu().numpy().view(DETECTION_DTYPE)[..., 0]
 
+    # -- sparse features -------------------------------------------------------------------------
+    def _check_u8_frames(self, frames: torch.Tensor, n: int, what: str) -> None:
+        if frames.dtype != torch.uint8 or not frames.is_cuda or not frames.is_contiguous() or frames.dim() != 3 or \
+                tuple(frames.shape[1:]) != (self.height, self.width) or frames.shape[0] < n:
+            raise ValueError('%s must be a contiguous CUDA uint8 tensor (>= %d, %d, %d)' % (what, n, self.height,
+                                                                                            self.width))
+
+    def good_features(self, frames: torch.Tensor, max_corners: int, quality_level: float, min_distance: float,
+                      block_size: int = 3, mask: Optional[torch.Tensor] = None, want_eig: bool = False):
+        """cv2.goodFeaturesToTrack(frame, max_corners, quality_level, min_distance, mask, block_size) for every frame
+        of an (n, H, W) uint8 CUDA tensor.  Returns (corners (n, max_corners, 2) float32, counts (n,) int32[, eig
+        (n, H, W) float32]).  counts are not limited by max_corners; frame i's corners are corners[i, :min(count,
+        max_corners)] in cv2's order.  mask: (H, W) for every frame or (n, H, W), uint8 or bool."""
+        n = frames.shape[0]
+        self._check_u8_frames(frames, n, 'frames')
+        prm = _lib.GfttParams(int(max_corners), float(quality_level), float(min_distance), int(block_size), 3)
+        stride = 0
+        if mask is not None:
+            if mask.dtype not in (torch.uint8, torch.bool) or not mask.is_cuda or not mask.is_contiguous() or \
+                    tuple(mask.shape[-2:]) != (self.height, self.width) or mask.dim() not in (2, 3) or \
+                    (mask.dim() == 3 and mask.shape[0] != n):
+                raise ValueError('mask must be a contiguous CUDA uint8/bool tensor (H, W) or (n, H, W)')
+            stride = self.width * self.height if mask.dim() == 3 else 0
+        corners = torch.zeros((n, max(int(max_corners), 0), 2), dtype=torch.float32, device=self.device)
+        counts = torch.zeros((n,), dtype=torch.int32, device=self.device)
+        eig = torch.empty((n, self.height, self.width), dtype=torch.float32, device=self.device) if want_eig else None
+        check(self.lib.mavd_good_features_to_track(self._h, frames.data_ptr(), n, C.byref(prm), _ptr(mask), stride,
+                                                   corners.data_ptr() if corners.numel() else None, counts.data_ptr(),
+                                                   _ptr(eig), self._stream()))
+        return (corners, counts, eig) if want_eig else (corners, counts)
+
+    def pyr_lk(self, frames: torch.Tensor, prev_pts: torch.Tensor, n_points: Optional[torch.Tensor] = None,
+               pair_stride: int = 1, win: Tuple[int, int] = (21, 21), max_level: int = 3,
+               criteria: Tuple[int, int, float] = (_lib.TERM_COUNT | _lib.TERM_EPS, 30, 0.01), flags: int = 0,
+               min_eig_threshold: float = 1e-4):
+        """cv2.calcOpticalFlowPyrLK(prev, next, prevPts, None, win, max_level, criteria, flags, min_eig_threshold) for
+        every pair: pair p tracks prev_pts[p] ((n_pairs, N, 2) float32 CUDA) from frame p*pair_stride to the next
+        frame.  n_points: optional (n_pairs,) int32 counts (good_features' counts).  Returns (next_pts (n_pairs, N, 2)
+        float32, status (n_pairs, N) uint8, err (n_pairs, N) float32)."""
+        if prev_pts.dtype != torch.float32 or not prev_pts.is_cuda or not prev_pts.is_contiguous() or \
+                prev_pts.dim() != 3 or prev_pts.shape[2] != 2:
+            raise ValueError('prev_pts must be a contiguous CUDA float32 tensor (n_pairs, N, 2)')
+        n_pairs, n = prev_pts.shape[0], prev_pts.shape[1]
+        if pair_stride not in (1, 2):
+            raise ValueError('pair_stride must be 1 or 2')
+        self._check_u8_frames(frames, (n_pairs - 1) * pair_stride + 2 if n_pairs else 0, 'frames')
+        if n_points is not None and (n_points.dtype != torch.int32 or not n_points.is_cuda or
+                                     not n_points.is_contiguous() or n_points.shape[0] < n_pairs):
+            raise ValueError('n_points must be a contiguous CUDA int32 tensor (>= n_pairs,)')
+        prm = _lib.LkParams(int(win[0]), int(win[1]), int(max_level), int(criteria[0]), int(criteria[1]),
+                            float(criteria[2]), int(flags), float(min_eig_threshold))
+        nxt = torch.empty_like(prev_pts)
+        status = torch.empty((n_pairs, n), dtype=torch.uint8, device=self.device)
+        err = torch.empty((n_pairs, n), dtype=torch.float32, device=self.device)
+        check(self.lib.mavd_pyr_lk(self._h, frames.data_ptr(), n_pairs, pair_stride, C.byref(prm), prev_pts.data_ptr(),
+                                   n, _ptr(n_points), nxt.data_ptr(), status.data_ptr(), err.data_ptr(),
+                                   self._stream()))
+        return nxt, status, err
+
     # -- whole path ----------------------------------------------------------------------------
     def process(self, frames: torch.Tensor, imu, samples: torch.Tensor, n_pairs: Optional[int] = None,
                 pair_stride: int = 1, sky: Optional[torch.Tensor] = None, seg: Optional[torch.Tensor] = None,
