@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define MAVD_ABI_VERSION 3
+#define MAVD_ABI_VERSION 4
 
 enum {
     MAVD_OK = 0,
@@ -126,7 +126,7 @@ typedef struct mavd_aux_inputs {
     const float* gt_flow;
 } mavd_aux_inputs;
 
-/* flags of mavd_submit_host_ex / mavd_detect_host_ex */
+/* flags of mavd_submit_host / mavd_detect_host */
 #define MAVD_HOST_BGR 1           /* h_frames are (H, W, 3) BGR frames, converted to gray on the device */
 #define MAVD_HOST_SEG_PACKED 2    /* aux.seg is 1 bit per pixel (bit set = 255), mavd_packed_mask_bytes per frame */
 #define MAVD_HOST_SKY_PACKED 4    /* aux.sky is 1 bit per pixel (bit set = sky) */
@@ -322,99 +322,59 @@ int mavd_ccl(mavd_handle h, const uint8_t* d_mask, int32_t n, int32_t* d_labels,
 int mavd_detections(mavd_handle h, const uint8_t* d_mask, int32_t n, const float* d_flow, const mavd_imu* h_imu,
                     int32_t max_det, mavd_detection* d_det, void* stream);
 
-/* ---- detection from a given flow field, device buffers: derotate -> FoE -> phi/masks -> components ----
- * One iteration of Processor.run_detection (src/processor.py:305-362) per frame, starting from the
- * flow that Dataset.get_flow_uv returns (src/datasets/dataset.py:205-212).  d_total_out / d_fixed_out
- * nullable.  d_records: n mavd_frame_record. */
-int mavd_detect(mavd_handle h, const float* d_flow, int32_t n, const mavd_imu* h_imu,
-                const mavd_detect_params* prm, const int32_t* d_samples, const uint8_t* d_sky, int64_t sky_stride,
-                const uint8_t* d_seg, int64_t seg_stride, uint8_t* d_total_out, uint8_t* d_fixed_out,
-                mavd_frame_record* d_records, void* stream);
+/* ---- detection calls: one iteration of Processor.run_detection (src/processor.py:305-362) per frame ----
+ * Arguments common to the four calls below:
+ *  - aux (nullable = no optional input): sky, segmentation and ground-truth flow (mavd_aux_inputs), DEVICE pointers
+ *    for mavd_detect / mavd_process and HOST pointers for mavd_submit_host / mavd_detect_host.  A ground-truth flow
+ *    keeps datasets that carry one (SimData: src/processor.py:309-310,344,359) at one call per batch.
+ *  - records: n mavd_frame_record.
+ *  - det (nullable = no table): each frame's detection table of estimate_fixed, n x max_det mavd_detection (8-byte
+ *    aligned on the device), with 1 <= max_det <= MAVD_MAX_DETECTIONS; max_det is ignored when det is NULL.  For the
+ *    host calls the tables are valid after the wait, like the records.  The table comes from the same labelling as
+ *    record.boxes (an entry with label <= MAVD_MAX_BOXES has the box and area of boxes[label - 1]); flow_sum sums the
+ *    derotated flow of the call (the caller's flow, or the Farneback flow of the pair).
+ *  - flags (host calls): MAVD_HOST_* above.  With MAVD_HOST_SEG_PACKED / MAVD_HOST_SKY_PACKED the segmentation / sky
+ *    masks cross the bus at 1 bit per pixel and are expanded on the device; with MAVD_HOST_FIXED_PACKED the
+ *    estimate_fixed masks are packed on the device and return at 1 bit per pixel (numpy.packbits(mask.ravel(),
+ *    bitorder='little') per frame, padded to mavd_packed_mask_bytes).  Sample indices are range-checked on the host.
+ *    Host buffers should be pinned for the copies to be asynchronous. */
 
-/* ---- whole path, device buffers: flow -> derotate -> FoE -> phi/masks -> components ----
- * mavd_farneback followed by mavd_detect.  d_flow_out / d_fixed_out / d_total_out nullable. */
-int mavd_process(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int32_t pair_stride,
-                 const mavd_imu* h_imu, const mavd_detect_params* prm, const int32_t* d_samples,
-                 const uint8_t* d_sky, int64_t sky_stride, const uint8_t* d_seg, int64_t seg_stride,
-                 float* d_flow_out, uint8_t* d_total_out, uint8_t* d_fixed_out,
-                 mavd_frame_record* d_records, void* stream);
+/* Detection from a given DEVICE flow field: derotate -> FoE -> phi/masks -> components, starting from the flow that
+ * Dataset.get_flow_uv returns (src/datasets/dataset.py:205-212).  d_total_out / d_fixed_out nullable. */
+int mavd_detect(mavd_handle h, const float* d_flow, int32_t n, const mavd_imu* h_imu, const mavd_detect_params* prm,
+                const int32_t* d_samples, const mavd_aux_inputs* d_aux, uint8_t* d_total_out, uint8_t* d_fixed_out,
+                mavd_frame_record* d_records, int32_t max_det, mavd_detection* d_det, void* stream);
 
-/* ---- whole path, HOST buffers (the end-to-end call): copies frames/samples/sky/seg in, runs
- * mavd_process, copies the records (and, when non-NULL, estimate_fixed masks and flow) back.
- * Host buffers should be pinned for the copies to be asynchronous; the call returns after the
- * results have landed (it synchronises). */
-int mavd_process_host(mavd_handle h, const uint8_t* h_frames, int32_t n_pairs, int32_t pair_stride,
-                      const mavd_imu* h_imu, const mavd_detect_params* prm, const int32_t* h_samples,
-                      const uint8_t* h_sky, int64_t sky_stride, const uint8_t* h_seg, int64_t seg_stride,
-                      float* h_flow_out, uint8_t* h_fixed_out, mavd_frame_record* h_records, void* stream);
+/* Whole path, DEVICE buffers: mavd_farneback followed by mavd_detect.  d_flow_out / d_total_out / d_fixed_out
+ * nullable. */
+int mavd_process(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int32_t pair_stride, const mavd_imu* h_imu,
+                 const mavd_detect_params* prm, const int32_t* d_samples, const mavd_aux_inputs* d_aux,
+                 float* d_flow_out, uint8_t* d_total_out, uint8_t* d_fixed_out, mavd_frame_record* d_records,
+                 int32_t max_det, mavd_detection* d_det, void* stream);
 
-/* The same, split into an asynchronous submit and a wait so that a caller can keep up to
- * MAVD_HOST_SLOTS batches in flight: batch k+1's host->device copies run on a copy stream while batch k
- * computes on `stream` and batch k-1's results return on a third stream.  `slot` in [0, MAVD_HOST_SLOTS)
- * names the staging buffers used; a slot must be waited on before it is submitted again.  All host
- * buffers of a submit must stay valid (and unmodified) until its wait returns. */
+/* Whole path, HOST buffers (the end-to-end call), split into an asynchronous submit and a wait so that a caller can
+ * keep up to MAVD_HOST_SLOTS batches in flight: batch k+1's host->device copies run on a copy stream while batch k
+ * computes on `stream` and batch k-1's results (records, and when non-NULL the estimate_fixed masks, the flow and the
+ * detection tables) return on a third stream.  `slot` in [0, MAVD_HOST_SLOTS) names the staging buffers used; a slot
+ * must be waited on before it is submitted again.  All host buffers of a submit must stay valid (and unmodified)
+ * until its wait returns.  A blocking call is mavd_wait_host(h, 0); mavd_submit_host(h, 0, ...);
+ * mavd_wait_host(h, 0).
+ * With MAVD_HOST_BGR, h_frames are (H, W, 3) uint8 BGR frames as cv2.VideoCapture.read() / Dataset.get_frame()
+ * deliver them (src/farneback.py:73, src/datasets/dataset.py:223-230): they are copied as they are and converted to
+ * gray on the device on the copy-in stream (mavd_bgr2gray == cv2.cvtColor(COLOR_BGR2GRAY), src/farneback.py:74). */
 int mavd_submit_host(mavd_handle h, int32_t slot, const uint8_t* h_frames, int32_t n_pairs, int32_t pair_stride,
                      const mavd_imu* h_imu, const mavd_detect_params* prm, const int32_t* h_samples,
-                     const uint8_t* h_sky, int64_t sky_stride, const uint8_t* h_seg, int64_t seg_stride,
-                     float* h_flow_out, uint8_t* h_fixed_out, mavd_frame_record* h_records, void* stream);
+                     const mavd_aux_inputs* h_aux, int32_t flags, float* h_flow_out, uint8_t* h_fixed_out,
+                     mavd_frame_record* h_records, int32_t max_det, mavd_detection* h_det, void* stream);
 int mavd_wait_host(mavd_handle h, int32_t slot);
-/* The same with (H, W, 3) uint8 BGR frames as cv2.VideoCapture.read() / Dataset.get_frame() deliver them
- * (src/farneback.py:73, src/datasets/dataset.py:223-230): the frames are copied as they are and converted to gray on
- * the device on the copy-in stream (mavd_bgr2gray == cv2.cvtColor(COLOR_BGR2GRAY), src/farneback.py:74). */
-int mavd_submit_host_bgr(mavd_handle h, int32_t slot, const uint8_t* h_bgr_frames, int32_t n_pairs, int32_t pair_stride,
-                         const mavd_imu* h_imu, const mavd_detect_params* prm, const int32_t* h_samples,
-                         const uint8_t* h_sky, int64_t sky_stride, const uint8_t* h_seg, int64_t seg_stride,
-                         float* h_flow_out, uint8_t* h_fixed_out, mavd_frame_record* h_records, void* stream);
 
-/* Detection from a HOST flow field (n x H x W x 2 float32), the Dataset.get_flow_uv seam end to end. */
+/* Detection from a HOST flow field (n x H x W x 2 float32), the Dataset.get_flow_uv seam end to end.  Waits for
+ * slot 0, uses its staging buffers on `stream` alone, and returns after the results have landed (it synchronises).
+ * MAVD_HOST_BGR is rejected. */
 int mavd_detect_host(mavd_handle h, const float* h_flow, int32_t n, const mavd_imu* h_imu,
-                     const mavd_detect_params* prm, const int32_t* h_samples, const uint8_t* h_sky,
-                     int64_t sky_stride, const uint8_t* h_seg, int64_t seg_stride, uint8_t* h_fixed_out,
-                     mavd_frame_record* h_records, void* stream);
-
-/* ---- the same calls with every optional per-frame input in one struct (ground-truth flow included) ----
- * mavd_detect / mavd_process / mavd_submit_host / mavd_detect_host forward to these.  One device call per batch also
- * for datasets that carry a ground-truth flow (SimData: src/processor.py:309-310,344,359). */
-int mavd_detect_ex(mavd_handle h, const float* d_flow, int32_t n, const mavd_imu* h_imu, const mavd_detect_params* prm,
-                   const int32_t* d_samples, const mavd_aux_inputs* d_aux, uint8_t* d_total_out, uint8_t* d_fixed_out,
-                   mavd_frame_record* d_records, void* stream);
-int mavd_process_ex(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int32_t pair_stride, const mavd_imu* h_imu,
-                    const mavd_detect_params* prm, const int32_t* d_samples, const mavd_aux_inputs* d_aux,
-                    float* d_flow_out, uint8_t* d_total_out, uint8_t* d_fixed_out, mavd_frame_record* d_records,
-                    void* stream);
-/* flags: MAVD_HOST_* above.  With MAVD_HOST_SEG_PACKED / MAVD_HOST_SKY_PACKED the segmentation / sky masks cross the
- * bus at 1 bit per pixel and are expanded on the device on the copy-in stream; with MAVD_HOST_FIXED_PACKED the
- * estimate_fixed masks are packed on the copy-out stream and return at 1 bit per pixel (numpy.packbits(mask.ravel(),
- * bitorder='little') per frame, padded to mavd_packed_mask_bytes).  Sample indices are range-checked on the host. */
-int mavd_submit_host_ex(mavd_handle h, int32_t slot, const uint8_t* h_frames, int32_t n_pairs, int32_t pair_stride,
-                        const mavd_imu* h_imu, const mavd_detect_params* prm, const int32_t* h_samples,
-                        const mavd_aux_inputs* h_aux, int32_t flags, float* h_flow_out, uint8_t* h_fixed_out,
-                        mavd_frame_record* h_records, void* stream);
-int mavd_detect_host_ex(mavd_handle h, const float* h_flow, int32_t n, const mavd_imu* h_imu,
-                        const mavd_detect_params* prm, const int32_t* h_samples, const mavd_aux_inputs* h_aux,
-                        int32_t flags, uint8_t* h_fixed_out, mavd_frame_record* h_records, void* stream);
-
-/* ---- the _ex calls plus each frame's detection table (mavd_detection) of estimate_fixed ----
- * The _ex calls forward to these with det = NULL.  det: n x max_det entries, a DEVICE pointer for mavd_detect_det /
- * mavd_process_det and a HOST pointer for mavd_submit_host_det / mavd_detect_host_det (valid after the wait, like the
- * records); 1 <= max_det <= MAVD_MAX_DETECTIONS when det is non-NULL.  The table comes from the same labelling as
- * record.boxes (an entry with label <= MAVD_MAX_BOXES has the box and area of boxes[label - 1]); flow_sum sums the
- * derotated flow of the call (the caller's flow, or the Farneback flow of the pair). */
-int mavd_detect_det(mavd_handle h, const float* d_flow, int32_t n, const mavd_imu* h_imu, const mavd_detect_params* prm,
-                    const int32_t* d_samples, const mavd_aux_inputs* d_aux, uint8_t* d_total_out, uint8_t* d_fixed_out,
-                    mavd_frame_record* d_records, int32_t max_det, mavd_detection* d_det, void* stream);
-int mavd_process_det(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int32_t pair_stride, const mavd_imu* h_imu,
-                     const mavd_detect_params* prm, const int32_t* d_samples, const mavd_aux_inputs* d_aux,
-                     float* d_flow_out, uint8_t* d_total_out, uint8_t* d_fixed_out, mavd_frame_record* d_records,
-                     int32_t max_det, mavd_detection* d_det, void* stream);
-int mavd_submit_host_det(mavd_handle h, int32_t slot, const uint8_t* h_frames, int32_t n_pairs, int32_t pair_stride,
-                         const mavd_imu* h_imu, const mavd_detect_params* prm, const int32_t* h_samples,
-                         const mavd_aux_inputs* h_aux, int32_t flags, float* h_flow_out, uint8_t* h_fixed_out,
-                         mavd_frame_record* h_records, int32_t max_det, mavd_detection* h_det, void* stream);
-int mavd_detect_host_det(mavd_handle h, const float* h_flow, int32_t n, const mavd_imu* h_imu,
-                         const mavd_detect_params* prm, const int32_t* h_samples, const mavd_aux_inputs* h_aux,
-                         int32_t flags, uint8_t* h_fixed_out, mavd_frame_record* h_records, int32_t max_det,
-                         mavd_detection* h_det, void* stream);
+                     const mavd_detect_params* prm, const int32_t* h_samples, const mavd_aux_inputs* h_aux,
+                     int32_t flags, uint8_t* h_fixed_out, mavd_frame_record* h_records, int32_t max_det,
+                     mavd_detection* h_det, void* stream);
 
 /* ---- sparse features: cv2.goodFeaturesToTrack and cv2.calcOpticalFlowPyrLK (the LucasKanade class's calls) ----
  * mavd_good_features_to_track: Shi-Tomasi corners of n_frames dense (H, W) uint8 frames (n_frames <= 2 * max_pairs).

@@ -9,7 +9,7 @@ from typing import Optional
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, 'csrc', 'libmavd.so')
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 MAVD_OK, MAVD_ERR_INVALID, MAVD_ERR_CUDA, MAVD_ERR_UNSUPPORTED, MAVD_ERR_NOMEM = 0, 1, 2, 3, 4
 N_SAMPLE_PAIRS = 1000
 SAMPLES_PER_FRAME = 4 * N_SAMPLE_PAIRS
@@ -123,36 +123,16 @@ SIGNATURES = {
     'mavd_residual_masks': (C.c_int, [_P, _P, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams), _P,
                                       _P, C.c_int64, _P, C.c_int64, _P, _P, _P, _P, _P]),
     'mavd_ccl': (C.c_int, [_P, _P, C.c_int32, _P, _P, C.c_int32, _P, _P]),
-    'mavd_process': (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams), _P,
-                               _P, C.c_int64, _P, C.c_int64, _P, _P, _P, _P, _P]),
-    'mavd_process_host': (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams), _P,
-                                    _P, C.c_int64, _P, C.c_int64, _P, _P, _P, _P]),
-    'mavd_detect': (C.c_int, [_P, _P, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams), _P, _P, C.c_int64, _P, C.c_int64,
-                              _P, _P, _P, _P]),
-    'mavd_submit_host': (C.c_int, [_P, C.c_int32, _P, C.c_int32, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams), _P,
-                                   _P, C.c_int64, _P, C.c_int64, _P, _P, _P, _P]),
-    'mavd_submit_host_bgr': (C.c_int, [_P, C.c_int32, _P, C.c_int32, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams), _P,
-                                       _P, C.c_int64, _P, C.c_int64, _P, _P, _P, _P]),
-    'mavd_wait_host': (C.c_int, [_P, C.c_int32]),
-    'mavd_detect_host': (C.c_int, [_P, _P, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams), _P, _P, C.c_int64, _P,
-                                   C.c_int64, _P, _P, _P]),
-    'mavd_detect_ex': (C.c_int, [_P, _P, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams), _P, C.POINTER(AuxInputs),
-                                 _P, _P, _P, _P]),
-    'mavd_process_ex': (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams), _P,
-                                  C.POINTER(AuxInputs), _P, _P, _P, _P, _P]),
-    'mavd_submit_host_ex': (C.c_int, [_P, C.c_int32, _P, C.c_int32, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams),
-                                      _P, C.POINTER(AuxInputs), C.c_int32, _P, _P, _P, _P]),
-    'mavd_detect_host_ex': (C.c_int, [_P, _P, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams), _P,
-                                      C.POINTER(AuxInputs), C.c_int32, _P, _P, _P]),
     'mavd_detections': (C.c_int, [_P, _P, C.c_int32, _P, C.POINTER(Imu), C.c_int32, _P, _P]),
-    'mavd_detect_det': (C.c_int, [_P, _P, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams), _P, C.POINTER(AuxInputs),
-                                  _P, _P, _P, C.c_int32, _P, _P]),
-    'mavd_process_det': (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams), _P,
-                                   C.POINTER(AuxInputs), _P, _P, _P, _P, C.c_int32, _P, _P]),
-    'mavd_submit_host_det': (C.c_int, [_P, C.c_int32, _P, C.c_int32, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams),
-                                       _P, C.POINTER(AuxInputs), C.c_int32, _P, _P, _P, C.c_int32, _P, _P]),
-    'mavd_detect_host_det': (C.c_int, [_P, _P, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams), _P,
-                                       C.POINTER(AuxInputs), C.c_int32, _P, _P, C.c_int32, _P, _P]),
+    'mavd_detect': (C.c_int, [_P, _P, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams), _P, C.POINTER(AuxInputs),
+                              _P, _P, _P, C.c_int32, _P, _P]),
+    'mavd_process': (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams), _P,
+                               C.POINTER(AuxInputs), _P, _P, _P, _P, C.c_int32, _P, _P]),
+    'mavd_submit_host': (C.c_int, [_P, C.c_int32, _P, C.c_int32, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams),
+                                   _P, C.POINTER(AuxInputs), C.c_int32, _P, _P, _P, C.c_int32, _P, _P]),
+    'mavd_wait_host': (C.c_int, [_P, C.c_int32]),
+    'mavd_detect_host': (C.c_int, [_P, _P, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams), _P,
+                                   C.POINTER(AuxInputs), C.c_int32, _P, _P, C.c_int32, _P, _P]),
     'mavd_good_features_to_track': (C.c_int, [_P, _P, C.c_int32, C.POINTER(GfttParams), _P, C.c_int64, _P, _P, _P,
                                                _P]),
     'mavd_pyr_lk': (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(LkParams), _P, C.c_int32, _P, _P, _P, _P, _P]),

@@ -437,7 +437,7 @@ int mavd_create(const mavd_config* cfg, mavd_handle* out) {
     C_TRY(A.alloc(&H->d_flow, B * npx * 2));
     for (int k = 0; k < MAVD_HOST_SLOTS; ++k) {
         mavd_handle_s::HostSlot& S = H->slot[k];
-        // slot 0 is always there (mavd_process_host); further slots appear on their first submit
+        // slot 0 is always there (mavd_detect_host stages through it); further slots appear on their first submit
         if (k == 0) C_TRY(alloc_slot(A, S, F, B, npx));
     }
     C_TRY(A.alloc(&H->d_stats_tmp, B));
@@ -1101,9 +1101,9 @@ int mavd_farneback(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int3
                        ss.s, [&](cudaStream_t s) { return farneback_run(h, d_frames, n_pairs, pair_stride, d_flow, s); });
 }
 
-int mavd_detect_det(mavd_handle h, const float* d_flow, int32_t n, const mavd_imu* h_imu, const mavd_detect_params* prm,
-                    const int32_t* d_samples, const mavd_aux_inputs* d_aux, uint8_t* d_total_out, uint8_t* d_fixed_out,
-                    mavd_frame_record* d_records, int32_t max_det, mavd_detection* d_det, void* stream) {
+int mavd_detect(mavd_handle h, const float* d_flow, int32_t n, const mavd_imu* h_imu, const mavd_detect_params* prm,
+                const int32_t* d_samples, const mavd_aux_inputs* d_aux, uint8_t* d_total_out, uint8_t* d_fixed_out,
+                mavd_frame_record* d_records, int32_t max_det, mavd_detection* d_det, void* stream) {
     DeviceGuard dg(h ? h->cfg.device : -1);
     TRY(check_batch(h, n, "detect"));
     TRY(check_det(h, max_det, d_det, "detect"));
@@ -1125,25 +1125,10 @@ int mavd_detect_det(mavd_handle h, const float* d_flow, int32_t n, const mavd_im
                        });
 }
 
-int mavd_detect_ex(mavd_handle h, const float* d_flow, int32_t n, const mavd_imu* h_imu, const mavd_detect_params* prm,
-                   const int32_t* d_samples, const mavd_aux_inputs* d_aux, uint8_t* d_total_out, uint8_t* d_fixed_out,
-                   mavd_frame_record* d_records, void* stream) {
-    return mavd_detect_det(h, d_flow, n, h_imu, prm, d_samples, d_aux, d_total_out, d_fixed_out, d_records, 0, nullptr,
-                           stream);
-}
-
-int mavd_detect(mavd_handle h, const float* d_flow, int32_t n, const mavd_imu* h_imu, const mavd_detect_params* prm,
-                const int32_t* d_samples, const uint8_t* d_sky, int64_t sky_stride, const uint8_t* d_seg,
-                int64_t seg_stride, uint8_t* d_total_out, uint8_t* d_fixed_out, mavd_frame_record* d_records,
-                void* stream) {
-    const mavd_aux_inputs aux = {d_sky, sky_stride, d_seg, seg_stride, nullptr};
-    return mavd_detect_ex(h, d_flow, n, h_imu, prm, d_samples, &aux, d_total_out, d_fixed_out, d_records, stream);
-}
-
-int mavd_process_det(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int32_t pair_stride, const mavd_imu* h_imu,
-                     const mavd_detect_params* prm, const int32_t* d_samples, const mavd_aux_inputs* d_aux,
-                     float* d_flow_out, uint8_t* d_total_out, uint8_t* d_fixed_out, mavd_frame_record* d_records,
-                     int32_t max_det, mavd_detection* d_det, void* stream) {
+int mavd_process(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int32_t pair_stride, const mavd_imu* h_imu,
+                 const mavd_detect_params* prm, const int32_t* d_samples, const mavd_aux_inputs* d_aux,
+                 float* d_flow_out, uint8_t* d_total_out, uint8_t* d_fixed_out, mavd_frame_record* d_records,
+                 int32_t max_det, mavd_detection* d_det, void* stream) {
     DeviceGuard dg(h ? h->cfg.device : -1);
     TRY(check_batch(h, n_pairs, "process"));
     MAVD_REQUIRE(pair_stride == 1 || pair_stride == 2, MAVD_ERR_INVALID, "pair_stride must be 1 or 2");
@@ -1168,23 +1153,6 @@ int mavd_process_det(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, in
                            return detect_run(h, flow, n_pairs, p, n64, n32, d_samples, aux, d_total_out, fixed, d_records,
                                              max_det, d_det, s);
                        });
-}
-
-int mavd_process_ex(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int32_t pair_stride, const mavd_imu* h_imu,
-                    const mavd_detect_params* prm, const int32_t* d_samples, const mavd_aux_inputs* d_aux,
-                    float* d_flow_out, uint8_t* d_total_out, uint8_t* d_fixed_out, mavd_frame_record* d_records,
-                    void* stream) {
-    return mavd_process_det(h, d_frames, n_pairs, pair_stride, h_imu, prm, d_samples, d_aux, d_flow_out, d_total_out,
-                            d_fixed_out, d_records, 0, nullptr, stream);
-}
-
-int mavd_process(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int32_t pair_stride, const mavd_imu* h_imu,
-                 const mavd_detect_params* prm, const int32_t* d_samples, const uint8_t* d_sky, int64_t sky_stride,
-                 const uint8_t* d_seg, int64_t seg_stride, float* d_flow_out, uint8_t* d_total_out,
-                 uint8_t* d_fixed_out, mavd_frame_record* d_records, void* stream) {
-    const mavd_aux_inputs aux = {d_sky, sky_stride, d_seg, seg_stride, nullptr};
-    return mavd_process_ex(h, d_frames, n_pairs, pair_stride, h_imu, prm, d_samples, &aux, d_flow_out, d_total_out,
-                           d_fixed_out, d_records, stream);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1271,27 +1239,53 @@ static int check_aux_strides(mavd_handle h, const mavd_aux_inputs& a, int flags)
     return MAVD_OK;
 }
 
-int mavd_submit_host_det(mavd_handle h, int32_t slot, const uint8_t* h_frames, int32_t n_pairs, int32_t pair_stride,
-                         const mavd_imu* h_imu, const mavd_detect_params* prm, const int32_t* h_samples,
-                         const mavd_aux_inputs* h_aux, int32_t flags, float* h_flow_out, uint8_t* h_fixed_out,
-                         mavd_frame_record* h_records, int32_t max_det, mavd_detection* h_det, void* stream) {
+// The arguments of a host-buffer call, all checked before anything is allocated or copied.  An empty batch reads no
+// buffer.
+static int check_host_args(mavd_handle h, const char* what, int n, const void* h_in, const int32_t* h_samples,
+                           const mavd_frame_record* h_records, const mavd_aux_inputs& ha, int flags, int max_det,
+                           const mavd_detection* h_det) {
+    if (h_det)
+        MAVD_REQUIRE(max_det >= 1 && max_det <= MAVD_MAX_DETECTIONS, MAVD_ERR_INVALID, "%s: max_det %d outside 1..%d",
+                     what, max_det, MAVD_MAX_DETECTIONS);
+    if (n == 0) return MAVD_OK;
+    MAVD_REQUIRE(h_in && h_samples && h_records, MAVD_ERR_INVALID, "%s: NULL buffer", what);
+    TRY(check_aux_strides(h, ha, flags));
+    return check_samples(h_samples, n, h->cfg.width, h->cfg.height);
+}
+
+// copy a batch's records, detection tables (when asked for) and estimate_fixed masks (packed first with
+// MAVD_HOST_FIXED_PACKED) from the slot's device buffers to the caller's host buffers on stream s
+static int copy_out(mavd_handle h, mavd_handle_s::HostSlot& S, int n, int flags, uint8_t* h_fixed_out,
+                    mavd_frame_record* h_records, int max_det, mavd_detection* h_det, cudaStream_t s) {
+    const size_t npx = (size_t)h->cfg.width * h->cfg.height;
+    MAVD_CUDA(cudaMemcpyAsync(h_records, S.d_records, sizeof(mavd_frame_record) * n, cudaMemcpyDeviceToHost, s));
+    if (h_det)
+        MAVD_CUDA(cudaMemcpyAsync(h_det, S.d_det, sizeof(mavd_detection) * max_det * n, cudaMemcpyDeviceToHost, s));
+    if (h_fixed_out && (flags & MAVD_HOST_FIXED_PACKED)) {
+        const size_t pb = (size_t)packed_mask_bytes((int64_t)npx);
+        TRY(pack_mask_run(S.d_fixed, n, (int64_t)npx, S.d_bits_out, s));
+        MAVD_CUDA(cudaMemcpyAsync(h_fixed_out, S.d_bits_out, pb * n, cudaMemcpyDeviceToHost, s));
+    } else if (h_fixed_out) {
+        MAVD_CUDA(cudaMemcpyAsync(h_fixed_out, S.d_fixed, npx * n, cudaMemcpyDeviceToHost, s));
+    }
+    return MAVD_OK;
+}
+
+int mavd_submit_host(mavd_handle h, int32_t slot, const uint8_t* h_frames, int32_t n_pairs, int32_t pair_stride,
+                     const mavd_imu* h_imu, const mavd_detect_params* prm, const int32_t* h_samples,
+                     const mavd_aux_inputs* h_aux, int32_t flags, float* h_flow_out, uint8_t* h_fixed_out,
+                     mavd_frame_record* h_records, int32_t max_det, mavd_detection* h_det, void* stream) {
     DeviceGuard dg(h ? h->cfg.device : -1);
     TRY(check_batch(h, n_pairs, "submit_host"));
-    if (h_det)
-        MAVD_REQUIRE(max_det >= 1 && max_det <= MAVD_MAX_DETECTIONS, MAVD_ERR_INVALID,
-                     "submit_host: max_det %d outside 1..%d", max_det, MAVD_MAX_DETECTIONS);
     MAVD_REQUIRE(slot >= 0 && slot < MAVD_HOST_SLOTS, MAVD_ERR_INVALID, "slot %d out of range", slot);
     MAVD_REQUIRE(pair_stride == 1 || pair_stride == 2, MAVD_ERR_INVALID, "pair_stride must be 1 or 2");
     MAVD_REQUIRE(n_pairs >= 1, MAVD_ERR_INVALID, "submit_host: empty batch");
-    MAVD_REQUIRE(h_frames && h_samples && h_records, MAVD_ERR_INVALID, "submit_host: NULL buffer");
     const mavd_aux_inputs ha = h_aux ? *h_aux : kNoAux;
-    TRY(check_aux_strides(h, ha, flags));
-    TRY(check_samples(h_samples, n_pairs, h->cfg.width, h->cfg.height));
+    TRY(check_host_args(h, "submit_host", n_pairs, h_frames, h_samples, h_records, ha, flags, max_det, h_det));
     const size_t npx = (size_t)h->cfg.width * h->cfg.height;
-    const size_t pb = (size_t)packed_mask_bytes((int64_t)npx);
-    const bool bgr = (flags & MAVD_HOST_BGR) != 0, fixed_packed = (flags & MAVD_HOST_FIXED_PACKED) != 0;
+    const bool bgr = (flags & MAVD_HOST_BGR) != 0;
     TRY(ensure_slot(h, slot, h_flow_out != nullptr, false, (flags & (MAVD_HOST_SEG_PACKED | MAVD_HOST_SKY_PACKED)) != 0,
-                    fixed_packed && h_fixed_out, ha.gt_flow != nullptr, h_det != nullptr));
+                    (flags & MAVD_HOST_FIXED_PACKED) && h_fixed_out, ha.gt_flow != nullptr, h_det != nullptr));
     mavd_handle_s::HostSlot& S = h->slot[slot];
     MAVD_REQUIRE(!S.busy, MAVD_ERR_INVALID, "slot %d is still in flight: call mavd_wait_host first", slot);
     const int n_frames = pair_stride == 1 ? n_pairs + 1 : 2 * n_pairs;
@@ -1318,54 +1312,19 @@ int mavd_submit_host_det(mavd_handle h, int32_t slot, const uint8_t* h_frames, i
     // the next batch's Farneback, was measured: no gain, the GPU is already full and the work is only re-ordered.)
     MAVD_CUDA(cudaStreamWaitEvent(s, S.ev_in, 0));
     if (!(flags & MAVD_HOST_COPY_ONLY))
-        TRY(mavd_process_det(h, S.d_frames, n_pairs, pair_stride, h_imu, prm, S.d_samples, &da,
-                             h_flow_out ? S.d_flow : nullptr, nullptr, S.d_fixed, S.d_records, max_det,
-                             h_det ? S.d_det : nullptr, s));
+        TRY(mavd_process(h, S.d_frames, n_pairs, pair_stride, h_imu, prm, S.d_samples, &da,
+                         h_flow_out ? S.d_flow : nullptr, nullptr, S.d_fixed, S.d_records, max_det,
+                         h_det ? S.d_det : nullptr, s));
     MAVD_CUDA(cudaEventRecord(S.ev_done, s));
     // copy-out stream
     MAVD_CUDA(cudaStreamWaitEvent(h->s_out, S.ev_done, 0));
-    MAVD_CUDA(cudaMemcpyAsync(h_records, S.d_records, sizeof(mavd_frame_record) * n_pairs, cudaMemcpyDeviceToHost, h->s_out));
-    if (h_fixed_out && fixed_packed) {
-        TRY(pack_mask_run(S.d_fixed, n_pairs, (int64_t)npx, S.d_bits_out, h->s_out));
-        MAVD_CUDA(cudaMemcpyAsync(h_fixed_out, S.d_bits_out, pb * n_pairs, cudaMemcpyDeviceToHost, h->s_out));
-    } else if (h_fixed_out) {
-        MAVD_CUDA(cudaMemcpyAsync(h_fixed_out, S.d_fixed, npx * n_pairs, cudaMemcpyDeviceToHost, h->s_out));
-    }
+    TRY(copy_out(h, S, n_pairs, flags, h_fixed_out, h_records, max_det, h_det, h->s_out));
     if (h_flow_out)
         MAVD_CUDA(cudaMemcpyAsync(h_flow_out, S.d_flow, sizeof(float) * 2 * npx * n_pairs, cudaMemcpyDeviceToHost, h->s_out));
-    if (h_det)
-        MAVD_CUDA(cudaMemcpyAsync(h_det, S.d_det, sizeof(mavd_detection) * max_det * n_pairs, cudaMemcpyDeviceToHost,
-                                  h->s_out));
     MAVD_CUDA(cudaEventRecord(S.ev_out, h->s_out));
     // the next batch's copy-in must not overwrite staging a kernel still reads: ordered by slot reuse rule
     S.busy = true;
     return MAVD_OK;
-}
-
-int mavd_submit_host_ex(mavd_handle h, int32_t slot, const uint8_t* h_frames, int32_t n_pairs, int32_t pair_stride,
-                        const mavd_imu* h_imu, const mavd_detect_params* prm, const int32_t* h_samples,
-                        const mavd_aux_inputs* h_aux, int32_t flags, float* h_flow_out, uint8_t* h_fixed_out,
-                        mavd_frame_record* h_records, void* stream) {
-    return mavd_submit_host_det(h, slot, h_frames, n_pairs, pair_stride, h_imu, prm, h_samples, h_aux, flags, h_flow_out,
-                                h_fixed_out, h_records, 0, nullptr, stream);
-}
-
-int mavd_submit_host(mavd_handle h, int32_t slot, const uint8_t* h_frames, int32_t n_pairs, int32_t pair_stride,
-                     const mavd_imu* h_imu, const mavd_detect_params* prm, const int32_t* h_samples,
-                     const uint8_t* h_sky, int64_t sky_stride, const uint8_t* h_seg, int64_t seg_stride,
-                     float* h_flow_out, uint8_t* h_fixed_out, mavd_frame_record* h_records, void* stream) {
-    const mavd_aux_inputs aux = {h_sky, sky_stride, h_seg, seg_stride, nullptr};
-    return mavd_submit_host_ex(h, slot, h_frames, n_pairs, pair_stride, h_imu, prm, h_samples, &aux, 0, h_flow_out,
-                               h_fixed_out, h_records, stream);
-}
-
-int mavd_submit_host_bgr(mavd_handle h, int32_t slot, const uint8_t* h_bgr_frames, int32_t n_pairs, int32_t pair_stride,
-                         const mavd_imu* h_imu, const mavd_detect_params* prm, const int32_t* h_samples,
-                         const uint8_t* h_sky, int64_t sky_stride, const uint8_t* h_seg, int64_t seg_stride,
-                         float* h_flow_out, uint8_t* h_fixed_out, mavd_frame_record* h_records, void* stream) {
-    const mavd_aux_inputs aux = {h_sky, sky_stride, h_seg, seg_stride, nullptr};
-    return mavd_submit_host_ex(h, slot, h_bgr_frames, n_pairs, pair_stride, h_imu, prm, h_samples, &aux, MAVD_HOST_BGR,
-                               h_flow_out, h_fixed_out, h_records, stream);
 }
 
 int mavd_wait_host(mavd_handle h, int32_t slot) {
@@ -1379,40 +1338,20 @@ int mavd_wait_host(mavd_handle h, int32_t slot) {
     return MAVD_OK;
 }
 
-int mavd_process_host(mavd_handle h, const uint8_t* h_frames, int32_t n_pairs, int32_t pair_stride,
-                      const mavd_imu* h_imu, const mavd_detect_params* prm, const int32_t* h_samples,
-                      const uint8_t* h_sky, int64_t sky_stride, const uint8_t* h_seg, int64_t seg_stride,
-                      float* h_flow_out, uint8_t* h_fixed_out, mavd_frame_record* h_records, void* stream) {
-    DeviceGuard dg(h ? h->cfg.device : -1);
-    TRY(check_batch(h, n_pairs, "process_host"));
-    if (n_pairs == 0) return MAVD_OK;
-    TRY(mavd_wait_host(h, 0));
-    TRY(mavd_submit_host(h, 0, h_frames, n_pairs, pair_stride, h_imu, prm, h_samples, h_sky, sky_stride, h_seg,
-                         seg_stride, h_flow_out, h_fixed_out, h_records, stream));
-    return mavd_wait_host(h, 0);
-}
-
-int mavd_detect_host_det(mavd_handle h, const float* h_flow, int32_t n, const mavd_imu* h_imu,
-                         const mavd_detect_params* prm, const int32_t* h_samples, const mavd_aux_inputs* h_aux,
-                         int32_t flags, uint8_t* h_fixed_out, mavd_frame_record* h_records, int32_t max_det,
-                         mavd_detection* h_det, void* stream) {
+int mavd_detect_host(mavd_handle h, const float* h_flow, int32_t n, const mavd_imu* h_imu,
+                     const mavd_detect_params* prm, const int32_t* h_samples, const mavd_aux_inputs* h_aux,
+                     int32_t flags, uint8_t* h_fixed_out, mavd_frame_record* h_records, int32_t max_det,
+                     mavd_detection* h_det, void* stream) {
     DeviceGuard dg(h ? h->cfg.device : -1);
     TRY(check_batch(h, n, "detect_host"));
-    if (h_det)
-        MAVD_REQUIRE(max_det >= 1 && max_det <= MAVD_MAX_DETECTIONS, MAVD_ERR_INVALID,
-                     "detect_host: max_det %d outside 1..%d", max_det, MAVD_MAX_DETECTIONS);
-    if (n == 0) return MAVD_OK;
-    MAVD_REQUIRE(h_flow && h_samples && h_records, MAVD_ERR_INVALID, "detect_host: NULL buffer");
-    MAVD_REQUIRE((flags & MAVD_HOST_BGR) == 0, MAVD_ERR_INVALID, "detect_host: MAVD_HOST_BGR has no meaning here");
     const mavd_aux_inputs ha = h_aux ? *h_aux : kNoAux;
-    TRY(check_aux_strides(h, ha, flags));
-    TRY(check_samples(h_samples, n, h->cfg.width, h->cfg.height));
+    TRY(check_host_args(h, "detect_host", n, h_flow, h_samples, h_records, ha, flags, max_det, h_det));
+    if (n == 0) return MAVD_OK;
+    MAVD_REQUIRE((flags & MAVD_HOST_BGR) == 0, MAVD_ERR_INVALID, "detect_host: MAVD_HOST_BGR has no meaning here");
     const size_t npx = (size_t)h->cfg.width * h->cfg.height;
-    const size_t pb = (size_t)packed_mask_bytes((int64_t)npx);
-    const bool fixed_packed = (flags & MAVD_HOST_FIXED_PACKED) != 0;
     TRY(mavd_wait_host(h, 0));
     TRY(ensure_slot(h, 0, false, true, (flags & (MAVD_HOST_SEG_PACKED | MAVD_HOST_SKY_PACKED)) != 0,
-                    fixed_packed && h_fixed_out, ha.gt_flow != nullptr, h_det != nullptr));
+                    (flags & MAVD_HOST_FIXED_PACKED) && h_fixed_out, ha.gt_flow != nullptr, h_det != nullptr));
     mavd_handle_s::HostSlot& S = h->slot[0];
     StreamScope ss(h, stream);
     cudaStream_t s = ss.s;
@@ -1421,33 +1360,11 @@ int mavd_detect_host_det(mavd_handle h, const float* h_flow, int32_t n, const ma
     mavd_aux_inputs da;
     TRY(stage_aux(h, S, ha, flags, n, s, &da));
     if (!(flags & MAVD_HOST_COPY_ONLY))
-        TRY(mavd_detect_det(h, S.d_flow_in, n, h_imu, prm, S.d_samples, &da, nullptr, S.d_fixed, S.d_records, max_det,
-                            h_det ? S.d_det : nullptr, s));
-    MAVD_CUDA(cudaMemcpyAsync(h_records, S.d_records, sizeof(mavd_frame_record) * n, cudaMemcpyDeviceToHost, s));
-    if (h_det)
-        MAVD_CUDA(cudaMemcpyAsync(h_det, S.d_det, sizeof(mavd_detection) * max_det * n, cudaMemcpyDeviceToHost, s));
-    if (h_fixed_out && fixed_packed) {
-        TRY(pack_mask_run(S.d_fixed, n, (int64_t)npx, S.d_bits_out, s));
-        MAVD_CUDA(cudaMemcpyAsync(h_fixed_out, S.d_bits_out, pb * n, cudaMemcpyDeviceToHost, s));
-    } else if (h_fixed_out) {
-        MAVD_CUDA(cudaMemcpyAsync(h_fixed_out, S.d_fixed, npx * n, cudaMemcpyDeviceToHost, s));
-    }
+        TRY(mavd_detect(h, S.d_flow_in, n, h_imu, prm, S.d_samples, &da, nullptr, S.d_fixed, S.d_records, max_det,
+                        h_det ? S.d_det : nullptr, s));
+    TRY(copy_out(h, S, n, flags, h_fixed_out, h_records, max_det, h_det, s));
     MAVD_CUDA(cudaStreamSynchronize(s));
     return MAVD_OK;
-}
-
-int mavd_detect_host_ex(mavd_handle h, const float* h_flow, int32_t n, const mavd_imu* h_imu,
-                        const mavd_detect_params* prm, const int32_t* h_samples, const mavd_aux_inputs* h_aux,
-                        int32_t flags, uint8_t* h_fixed_out, mavd_frame_record* h_records, void* stream) {
-    return mavd_detect_host_det(h, h_flow, n, h_imu, prm, h_samples, h_aux, flags, h_fixed_out, h_records, 0, nullptr,
-                                stream);
-}
-
-int mavd_detect_host(mavd_handle h, const float* h_flow, int32_t n, const mavd_imu* h_imu, const mavd_detect_params* prm,
-                     const int32_t* h_samples, const uint8_t* h_sky, int64_t sky_stride, const uint8_t* h_seg,
-                     int64_t seg_stride, uint8_t* h_fixed_out, mavd_frame_record* h_records, void* stream) {
-    const mavd_aux_inputs aux = {h_sky, sky_stride, h_seg, seg_stride, nullptr};
-    return mavd_detect_host_ex(h, h_flow, n, h_imu, prm, h_samples, &aux, 0, h_fixed_out, h_records, stream);
 }
 
 int64_t mavd_packed_mask_bytes(int32_t width, int32_t height) {

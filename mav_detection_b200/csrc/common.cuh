@@ -226,7 +226,7 @@ struct mavd_handle_s {
     // the H2D of one batch, the compute of the previous one and the D2H of the one before overlap
     struct HostSlot {
         uint8_t* d_frames = nullptr;    // [max_frames][H][W]
-        uint8_t* d_bgr = nullptr;       // [max_frames][H][W][3], mavd_submit_host_bgr only (allocated on first use)
+        uint8_t* d_bgr = nullptr;       // [max_frames][H][W][3], MAVD_HOST_BGR submits only (allocated on first use)
         int32_t* d_samples = nullptr;   // [max_pairs][4000]
         uint8_t* d_sky = nullptr;       // [max_pairs][H][W]
         uint8_t* d_seg = nullptr;

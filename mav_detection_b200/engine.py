@@ -364,6 +364,14 @@ class Engine:
             raise ValueError('max_det must be an int in 1..%d' % _lib.MAX_DETECTIONS)
         return int(max_det)
 
+    def _det_device(self, detections: Optional[int], n: int) -> Tuple[int, Optional[torch.Tensor]]:
+        """(max_det, table) for a device call asked for `detections` entries per frame: an (n, max_det, itemsize) uint8
+        CUDA tensor, or (0, None) for no table."""
+        if detections is None:
+            return 0, None
+        max_det = self._det_count(detections)
+        return max_det, torch.empty((n, max_det, DETECTION_DTYPE.itemsize), dtype=torch.uint8, device=self.device)
+
     def _det_host(self, det: Optional[np.ndarray], n: int) -> Tuple[int, Optional[int]]:
         """(max_det, pointer) of a host detection table: (n, max_det) DETECTION_DTYPE, C-contiguous (pinned for the
         copy to be asynchronous)."""
@@ -475,19 +483,11 @@ class Engine:
         if records is None:
             records = torch.empty((n_pairs, RECORD_DTYPE.itemsize), dtype=torch.uint8, device=self.device)
         aux = self._aux(sky, seg, gt_flow, n_pairs)
-        if detections is not None:
-            max_det = self._det_count(detections)
-            det = torch.empty((n_pairs, max_det, DETECTION_DTYPE.itemsize), dtype=torch.uint8, device=self.device)
-            check(self.lib.mavd_process_det(self._h, frames.data_ptr(), n_pairs, pair_stride, imu,
-                                            C.byref(self.detect_params), samples.data_ptr(), C.byref(aux),
-                                            _ptr(flow_out), _ptr(total_out), _ptr(fixed_out), records.data_ptr(),
-                                            max_det, det.data_ptr(), self._stream()))
-            return records, det
-        check(self.lib.mavd_process_ex(self._h, frames.data_ptr(), n_pairs, pair_stride, imu,
-                                       C.byref(self.detect_params), samples.data_ptr(), C.byref(aux),
-                                       _ptr(flow_out), _ptr(total_out), _ptr(fixed_out), records.data_ptr(),
-                                       self._stream()))
-        return records
+        max_det, det = self._det_device(detections, n_pairs)
+        check(self.lib.mavd_process(self._h, frames.data_ptr(), n_pairs, pair_stride, imu, C.byref(self.detect_params),
+                                    samples.data_ptr(), C.byref(aux), _ptr(flow_out), _ptr(total_out), _ptr(fixed_out),
+                                    records.data_ptr(), max_det, _ptr(det), self._stream()))
+        return records if det is None else (records, det)
 
     def detect(self, flow: torch.Tensor, imu, samples: torch.Tensor, sky: Optional[torch.Tensor] = None,
                seg: Optional[torch.Tensor] = None, total_out: Optional[torch.Tensor] = None,
@@ -503,17 +503,11 @@ class Engine:
         if records is None:
             records = torch.empty((n, RECORD_DTYPE.itemsize), dtype=torch.uint8, device=self.device)
         aux = self._aux(sky, seg, gt_flow, n)
-        if detections is not None:
-            max_det = self._det_count(detections)
-            det = torch.empty((n, max_det, DETECTION_DTYPE.itemsize), dtype=torch.uint8, device=self.device)
-            check(self.lib.mavd_detect_det(self._h, flow.data_ptr(), n, imu, C.byref(self.detect_params),
-                                           samples.data_ptr(), C.byref(aux), _ptr(total_out), _ptr(fixed_out),
-                                           records.data_ptr(), max_det, det.data_ptr(), self._stream()))
-            return records, det
-        check(self.lib.mavd_detect_ex(self._h, flow.data_ptr(), n, imu, C.byref(self.detect_params), samples.data_ptr(),
-                                      C.byref(aux), _ptr(total_out), _ptr(fixed_out), records.data_ptr(),
-                                      self._stream()))
-        return records
+        max_det, det = self._det_device(detections, n)
+        check(self.lib.mavd_detect(self._h, flow.data_ptr(), n, imu, C.byref(self.detect_params), samples.data_ptr(),
+                                   C.byref(aux), _ptr(total_out), _ptr(fixed_out), records.data_ptr(), max_det,
+                                   _ptr(det), self._stream()))
+        return records if det is None else (records, det)
 
     def _host_args(self, frames, samples, n_pairs, pair_stride, flow_out, fixed_out, records, fixed_packed=False):
         if n_pairs is None:
@@ -567,15 +561,9 @@ class Engine:
             (_lib.HOST_SKY_PACKED if sky_packed else 0) | (_lib.HOST_FIXED_PACKED if fixed_packed else 0) | \
             (_lib.HOST_COPY_ONLY if copy_only else 0)
         max_det, det = self._det_host(detections, n_pairs)
-        if det is None:
-            check(self.lib.mavd_submit_host_ex(self._h, slot, _hp(frames), n_pairs, pair_stride, imu,
-                                               C.byref(self.detect_params), _hp(samples), C.byref(aux), flags,
-                                               _hp(flow_out), _hp(fixed_out), records.ctypes.data, self._stream()))
-        else:
-            check(self.lib.mavd_submit_host_det(self._h, slot, _hp(frames), n_pairs, pair_stride, imu,
-                                                C.byref(self.detect_params), _hp(samples), C.byref(aux), flags,
-                                                _hp(flow_out), _hp(fixed_out), records.ctypes.data, max_det, det,
-                                                self._stream()))
+        check(self.lib.mavd_submit_host(self._h, slot, _hp(frames), n_pairs, pair_stride, imu,
+                                        C.byref(self.detect_params), _hp(samples), C.byref(aux), flags, _hp(flow_out),
+                                        _hp(fixed_out), records.ctypes.data, max_det, det, self._stream()))
         # keep the host buffers alive until the wait
         self._inflight[slot] = (frames, imu, samples, sky, seg, gt_flow, flow_out, fixed_out, records, detections)
         return records
@@ -599,14 +587,9 @@ class Engine:
         flags = (_lib.HOST_SEG_PACKED if seg_packed else 0) | (_lib.HOST_SKY_PACKED if sky_packed else 0) | \
             (_lib.HOST_FIXED_PACKED if fixed_packed else 0)
         max_det, det = self._det_host(detections, n)
-        if det is None:
-            check(self.lib.mavd_detect_host_ex(self._h, flow.ctypes.data, n, imu, C.byref(self.detect_params),
-                                               _hp(samples), C.byref(aux), flags, _hp(fixed_out), records.ctypes.data,
-                                               self._stream()))
-        else:
-            check(self.lib.mavd_detect_host_det(self._h, flow.ctypes.data, n, imu, C.byref(self.detect_params),
-                                                _hp(samples), C.byref(aux), flags, _hp(fixed_out), records.ctypes.data,
-                                                max_det, det, self._stream()))
+        check(self.lib.mavd_detect_host(self._h, flow.ctypes.data, n, imu, C.byref(self.detect_params), _hp(samples),
+                                        C.byref(aux), flags, _hp(fixed_out), records.ctypes.data, max_det, det,
+                                        self._stream()))
         return records
 
     @staticmethod

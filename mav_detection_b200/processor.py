@@ -127,7 +127,8 @@ class Processor:
     # ------------------------------------------------------------------------------------------------
     def _next_frame(self) -> np.ndarray:
         """The next frame as the dataset delivers it: (H, W) gray or (H, W, 3) BGR.  BGR frames travel to the device
-        unchanged and are converted there (mavd_submit_host_bgr), as cv2.cvtColor does at farneback.py:74."""
+        unchanged and are converted there (mavd_submit_host with MAVD_HOST_BGR), as cv2.cvtColor does at
+        farneback.py:74."""
         frame = self.dataset.get_frame()
         if frame is None:
             raise ValueError('Could not load frame.')

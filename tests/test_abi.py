@@ -50,9 +50,9 @@ def test_ctypes_signatures_have_the_header_arity_and_return_types():
         assert res is restype[ret], '%s: header returns %s' % (name, ret)
 
 
-def test_abi_version_3_and_defaults(lib):
+def test_abi_version_4_and_defaults(lib):
     from mav_detection_b200 import _lib
-    assert lib.mavd_abi_version() == _lib.ABI_VERSION == 3
+    assert lib.mavd_abi_version() == _lib.ABI_VERSION == 4
     p = _lib.DetectParams()
     lib.mavd_default_detect_params(C.byref(p))
     # focus_of_expansion.py:22-23, processor.py:333-341
@@ -61,7 +61,7 @@ def test_abi_version_3_and_defaults(lib):
         (0.25, 0.5, 8.0, 0.5, 1.0, 15.0)
 
 
-def test_struct_layouts_of_abi_3():
+def test_struct_layouts_of_abi_4():
     from mav_detection_b200 import _lib
     assert C.sizeof(_lib.Imu) == 40
     assert C.sizeof(_lib.FarnebackParams) == 40

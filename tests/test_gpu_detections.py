@@ -146,7 +146,7 @@ def test_flow_sums_mix_derotation_modes():
 
 
 # ------------------------------------------------------------------------------------------------
-# batch paths: *_det against *_ex, mavd_detections and the oracle
+# batch paths: with a table against without one, mavd_detections and the oracle
 # ------------------------------------------------------------------------------------------------
 def _rec(eng, r):
     return eng.records_to_numpy(r)
@@ -161,16 +161,16 @@ def _check_against_records(det, rec):
 
 def _process_det(eng, frames, imu, samples, n, flow, fixed, rec, max_det, det):
     from mav_detection_b200 import _lib
-    _lib.check(eng.lib.mavd_process_det(eng._h, frames.data_ptr(), n, 1, imu, C.byref(eng.detect_params),
-                                        samples.data_ptr(), C.byref(_lib.AuxInputs()), flow.data_ptr(), None,
-                                        fixed.data_ptr(), rec.data_ptr(), max_det, det.data_ptr(), eng._stream()))
+    _lib.check(eng.lib.mavd_process(eng._h, frames.data_ptr(), n, 1, imu, C.byref(eng.detect_params),
+                                    samples.data_ptr(), C.byref(_lib.AuxInputs()), flow.data_ptr(), None,
+                                    fixed.data_ptr(), rec.data_ptr(), max_det, det.data_ptr(), eng._stream()))
 
 
 def _detect_det(eng, flow, imu, samples, n, fixed, rec, max_det, det):
     from mav_detection_b200 import _lib
-    _lib.check(eng.lib.mavd_detect_det(eng._h, flow.data_ptr(), n, imu, C.byref(eng.detect_params), samples.data_ptr(),
-                                       C.byref(_lib.AuxInputs()), None, fixed.data_ptr(), rec.data_ptr(), max_det,
-                                       det.data_ptr(), eng._stream()))
+    _lib.check(eng.lib.mavd_detect(eng._h, flow.data_ptr(), n, imu, C.byref(eng.detect_params), samples.data_ptr(),
+                                   C.byref(_lib.AuxInputs()), None, fixed.data_ptr(), rec.data_ptr(), max_det,
+                                   det.data_ptr(), eng._stream()))
 
 
 def _table(eng, det, n, max_det):
@@ -180,10 +180,10 @@ def _table(eng, det, n, max_det):
 
 
 @pytest.mark.parametrize('motion', ['zoom', 'translate'])
-def test_batch_paths_match_ex_calls_and_standalone(motion):
-    """process_det / detect_det: records, masks and flow as the _ex calls; tables as mavd_detections on the returned
-    estimate_fixed and flow, as the oracle, and as record.boxes for labels <= 32.  Every call twice (graph capture,
-    then replay) into buffers poisoned before each run."""
+def test_batch_paths_with_a_table_match_calls_without_and_standalone(motion):
+    """mavd_process / mavd_detect with a table: records, masks and flow as the same calls without one; tables as
+    mavd_detections on the returned estimate_fixed and flow, as the oracle, and as record.boxes for labels <= 32.
+    Every call twice (graph capture, then replay) into buffers poisoned before each run."""
     import torch
     from mav_detection_b200 import engine, sharded, synth
     W, H, F = 640, 480, 5
@@ -193,16 +193,16 @@ def test_batch_paths_match_ex_calls_and_standalone(motion):
     frames = torch.from_numpy(seq.frames).cuda()
     samples = torch.from_numpy(sharded.draw_all_samples(n, H, W, seed=5)).cuda()
     imu = engine.make_imu(n, seq.omega[1:], seq.dt, derotate=[i >= 1 for i in range(n)])
-    flow_ex = torch.empty((n, H, W, 2), dtype=torch.float32, device='cuda')
-    fixed_ex = torch.empty((n, H, W), dtype=torch.uint8, device='cuda')
-    rec_ex = _rec(eng, eng.process(frames, imu, samples, flow_out=flow_ex, fixed_out=fixed_ex))
-    rec_dex = _rec(eng, eng.detect(flow_ex, imu, samples))
-    flow = torch.empty_like(flow_ex)
-    fixed = torch.empty_like(fixed_ex)
+    flow_plain = torch.empty((n, H, W, 2), dtype=torch.float32, device='cuda')
+    fixed_plain = torch.empty((n, H, W), dtype=torch.uint8, device='cuda')
+    rec_plain = _rec(eng, eng.process(frames, imu, samples, flow_out=flow_plain, fixed_out=fixed_plain))
+    rec_dplain = _rec(eng, eng.detect(flow_plain, imu, samples))
+    flow = torch.empty_like(flow_plain)
+    fixed = torch.empty_like(fixed_plain)
     rec_t = torch.empty((n, engine.RECORD_DTYPE.itemsize), dtype=torch.uint8, device='cuda')
     det_t = torch.empty((n, 256, 56), dtype=torch.uint8, device='cuda')
-    fd = _derotated(eng, flow_ex, imu)
-    fx = fixed_ex.cpu().numpy()
+    fd = _derotated(eng, flow_plain, imu)
+    fx = fixed_plain.cpu().numpy()
     refs = [oracle(fx[f], fd[f]) for f in range(n)]
     for max_det in (7, 256):
         for call in ('process', 'detect'):
@@ -211,14 +211,14 @@ def test_batch_paths_match_ex_calls_and_standalone(motion):
                     t.view(torch.uint8).fill_(0xAB)
                 if call == 'process':
                     _process_det(eng, frames, imu, samples, n, flow, fixed, rec_t, max_det, det_t)
-                    assert torch.equal(flow, flow_ex)
-                    assert sharded.compare_records(_rec(eng, rec_t), rec_ex) == [], (max_det, run)
+                    assert torch.equal(flow, flow_plain)
+                    assert sharded.compare_records(_rec(eng, rec_t), rec_plain) == [], (max_det, run)
                 else:
-                    _detect_det(eng, flow_ex, imu, samples, n, fixed, rec_t, max_det, det_t)
-                    assert sharded.compare_records(_rec(eng, rec_t), rec_dex) == [], (max_det, run)
-                assert torch.equal(fixed, fixed_ex)
+                    _detect_det(eng, flow_plain, imu, samples, n, fixed, rec_t, max_det, det_t)
+                    assert sharded.compare_records(_rec(eng, rec_t), rec_dplain) == [], (max_det, run)
+                assert torch.equal(fixed, fixed_plain)
                 rec, det = _rec(eng, rec_t), _table(eng, det_t, n, max_det)
-                alone = eng.detections_to_numpy(eng.detections(fixed_ex, flow_ex, imu, max_det=max_det))
+                alone = eng.detections_to_numpy(eng.detections(fixed_plain, flow_plain, imu, max_det=max_det))
                 where = (call, max_det, run)
                 for f in range(n):
                     same_tables(det[f], alone[f], where + (f,))
@@ -228,7 +228,7 @@ def test_batch_paths_match_ex_calls_and_standalone(motion):
     # the engine-level API returns the same tables
     rec2, det2 = eng.process(frames, imu, samples, detections=32)
     det2 = eng.detections_to_numpy(det2)
-    rec3, det3 = eng.detect(flow_ex, imu, samples, detections=32)
+    rec3, det3 = eng.detect(flow_plain, imu, samples, detections=32)
     det3 = eng.detections_to_numpy(det3)
     for f in range(n):
         check_table(det2[f], fx[f], fd[f], 32, ('engine.process', f), ref=refs[f])
@@ -238,7 +238,7 @@ def test_batch_paths_match_ex_calls_and_standalone(motion):
     eng.close()
 
 
-def test_graph_keys_differ_in_max_det():
+def test_process_graph_keys_differ_in_max_det():
     """The same buffers with max_det 7 and then 32: two graphs, and each replay writes its own table size."""
     import torch
     from mav_detection_b200 import _lib, engine, sharded, synth
@@ -257,10 +257,10 @@ def test_graph_keys_differ_in_max_det():
     for _ in range(2):
         for max_det in (7, 32):
             det.fill_(0xAB)
-            _lib.check(eng.lib.mavd_process_det(eng._h, frames.data_ptr(), n, 1, imu, C.byref(eng.detect_params),
-                                                samples.data_ptr(), C.byref(aux), flow.data_ptr(), None,
-                                                fixed.data_ptr(), rec.data_ptr(), max_det, det.data_ptr(),
-                                                eng._stream()))
+            _lib.check(eng.lib.mavd_process(eng._h, frames.data_ptr(), n, 1, imu, C.byref(eng.detect_params),
+                                            samples.data_ptr(), C.byref(aux), flow.data_ptr(), None,
+                                            fixed.data_ptr(), rec.data_ptr(), max_det, det.data_ptr(),
+                                            eng._stream()))
             tables.setdefault(max_det, []).append(_table(eng, det, n, max_det))
     assert eng.graph_stats() == {'captured': 2, 'direct': 0}
     for f in range(n):
@@ -354,7 +354,7 @@ def test_host_calls_fill_the_tables():
             same_tables(det[f], alone[f], (slot, f))
             check_table(det[f], mask[f], fd[f], 32, (slot, f))
             _check_against_records(det[f], rec[f])
-    # detect_host_det from the flow of the last batch
+    # detect_host with a table from the flow of the last batch
     slot, frames, imu, samples, flow, fixed, det, rec = jobs[-1]
     det2 = _pinned((n, 256), engine.DETECTION_DTYPE)
     fixed2 = np.empty((n, H, W), np.uint8)
@@ -442,7 +442,7 @@ def test_processor_detections(tmp_path, flow_source):
 # ------------------------------------------------------------------------------------------------
 # errors and workspace
 # ------------------------------------------------------------------------------------------------
-def test_rejected_arguments_and_lazy_workspace():
+def test_rejected_table_arguments_and_lazy_workspace():
     import torch
     from mav_detection_b200 import _lib, engine, sharded, synth
     W, H = 64, 48
@@ -473,12 +473,12 @@ def test_rejected_arguments_and_lazy_workspace():
     aux = _lib.AuxInputs()
     for md in (0, 257):
         with pytest.raises(ValueError):
-            _lib.check(lib.mavd_process_det(eng._h, frames.data_ptr(), 1, 1, imu, None, samples.data_ptr(),
-                                            C.byref(aux), None, None, None, rec.data_ptr(), md, det.data_ptr(),
-                                            eng._stream()))
+            _lib.check(lib.mavd_process(eng._h, frames.data_ptr(), 1, 1, imu, None, samples.data_ptr(),
+                                        C.byref(aux), None, None, None, rec.data_ptr(), md, det.data_ptr(),
+                                        eng._stream()))
         with pytest.raises(ValueError):
-            _lib.check(lib.mavd_detect_det(eng._h, flow.data_ptr(), 1, imu, None, samples.data_ptr(), C.byref(aux),
-                                           None, None, rec.data_ptr(), md, det.data_ptr(), eng._stream()))
+            _lib.check(lib.mavd_detect(eng._h, flow.data_ptr(), 1, imu, None, samples.data_ptr(), C.byref(aux),
+                                       None, None, rec.data_ptr(), md, det.data_ptr(), eng._stream()))
         with pytest.raises(ValueError):
             eng.process(frames, imu, samples, detections=md)
     with pytest.raises(ValueError):

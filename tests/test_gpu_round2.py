@@ -130,7 +130,7 @@ def test_pack_unpack_mask_kernels(size):
 
 
 def test_host_path_packed_masks_equal_byte_masks():
-    """mavd_submit_host_ex with MAVD_HOST_SEG_PACKED | MAVD_HOST_SKY_PACKED | MAVD_HOST_FIXED_PACKED returns the same
+    """mavd_submit_host with MAVD_HOST_SEG_PACKED | MAVD_HOST_SKY_PACKED | MAVD_HOST_FIXED_PACKED returns the same
     records and (after unpacking) the same estimate_fixed masks as the byte-mask call; copy-only skips the compute."""
     from mav_detection_b200 import engine, synth
     W, H, n = 320, 240, 4

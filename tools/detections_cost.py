@@ -1,4 +1,4 @@
-"""Cost of the per-frame detection tables (mavd_process_det) on bench.py's 1920x1080 workloads.
+"""Cost of the per-frame detection tables (mavd_process with a table) on bench.py's 1920x1080 workloads.
 
 For C2, c2rot and c2dense it times one 64-pair step of the device path (resident frames, graph replay, CUDA events)
 without a table and with max_det 32 and 256, the three arms alternating step by step so that clock drift and other
@@ -56,10 +56,10 @@ def run(name: str, steps: int) -> dict:
         b = s % nb
         f0 = b * B
         aux = eng._aux(None, seg[f0 + 1:f0 + B + 1], None, B)
-        _lib.check(eng.lib.mavd_process_det(eng._h, frames[f0:f0 + B + 1].data_ptr(), B, 1, imus[b],
-                                            C.byref(eng.detect_params), samples[f0:f0 + B].data_ptr(), C.byref(aux),
-                                            None, None, fixed.data_ptr(), records.data_ptr(), md,
-                                            det[md].data_ptr() if md else None, eng._stream()))
+        _lib.check(eng.lib.mavd_process(eng._h, frames[f0:f0 + B + 1].data_ptr(), B, 1, imus[b],
+                                        C.byref(eng.detect_params), samples[f0:f0 + B].data_ptr(), C.byref(aux),
+                                        None, None, fixed.data_ptr(), records.data_ptr(), md,
+                                        det[md].data_ptr() if md else None, eng._stream()))
 
     arms = (0, 32, 256)
     times = {md: [] for md in arms}
