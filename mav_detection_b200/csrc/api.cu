@@ -6,7 +6,6 @@
 #include <stdlib.h>
 #include <string.h>
 
-#include <algorithm>
 #include <new>
 #include <vector>
 
@@ -24,169 +23,10 @@ void set_error(const char* fmt, ...) {
     va_end(ap);
 }
 
-static inline int cv_round(double v) { return (int)nearbyint(v); }  // round-half-even, like cvRound
-
-// cv::resize(INTER_LINEAR) source index / weight per destination index (pixel-centre mapping).
-static void resize_tables(int src, int dst, std::vector<int>& i0, std::vector<float>& a) {
-    i0.resize(dst);
-    a.resize(dst);
-    const double inv_scale = (double)dst / src;
-    const double scale = 1.0 / inv_scale;
-    for (int d = 0; d < dst; ++d) {
-        float f = (float)((d + 0.5) * scale - 0.5);
-        int s = (int)floorf(f);
-        float w = f - (float)s;
-        if (s < 0) { s = 0; w = 0.f; }
-        if (s >= src - 1) { s = src - 1; w = 0.f; }
-        i0[d] = s;
-        a[d] = w;
-    }
-}
-
-// cv::getGaussianKernel(ksz, sigma, CV_32F)
-static std::vector<float> gaussian_kernel(int ksz, double sigma) {
-    std::vector<float> k(ksz);
-    if (sigma <= 0 && ksz == 3) { k[0] = 0.25f; k[1] = 0.5f; k[2] = 0.25f; return k; }
-    if (sigma <= 0) sigma = ((ksz - 1) * 0.5 - 1) * 0.3 + 0.8;
-    std::vector<double> t(ksz);
-    double sum = 0;
-    for (int i = 0; i < ksz; ++i) {
-        double x = i - (ksz - 1) * 0.5;
-        t[i] = exp(-0.5 * x * x / (sigma * sigma));
-        sum += t[i];
-    }
-    for (int i = 0; i < ksz; ++i) k[i] = (float)(t[i] / sum);
-    return k;
-}
-
-// FarnebackPrepareGaussian: taps and the four needed entries of inv(G) (Appendix A of SURVEY.md).
-static int poly_setup(int n, double sigma, PolyConst& pc) {
-    if (sigma < 1.1920929e-07) sigma = n * 0.3;
-    float g[2 * kMaxPolyN + 1], xg[2 * kMaxPolyN + 1], xxg[2 * kMaxPolyN + 1];
-    double s = 0;
-    for (int x = -n; x <= n; ++x) {
-        g[x + n] = (float)exp(-x * x / (2 * sigma * sigma));
-        s += g[x + n];
-    }
-    s = 1. / s;
-    for (int x = -n; x <= n; ++x) {
-        g[x + n] = (float)(g[x + n] * s);
-        xg[x + n] = (float)(x * g[x + n]);
-        xxg[x + n] = (float)(x * x * g[x + n]);
-    }
-    double G[6][6];
-    memset(G, 0, sizeof(G));
-    for (int y = -n; y <= n; ++y)
-        for (int x = -n; x <= n; ++x) {
-            const float gg = g[y + n] * g[x + n];
-            G[0][0] += gg;
-            G[1][1] += gg * x * x;
-            G[3][3] += gg * x * x * x * x;
-            G[5][5] += gg * x * x * y * y;
-        }
-    G[2][2] = G[0][3] = G[0][4] = G[3][0] = G[4][0] = G[1][1];
-    G[4][4] = G[3][3];
-    G[3][4] = G[4][3] = G[5][5];
-    // Gauss-Jordan inverse of the 6x6 (symmetric positive definite) matrix
-    double A[6][12];
-    for (int i = 0; i < 6; ++i)
-        for (int j = 0; j < 12; ++j) A[i][j] = j < 6 ? G[i][j] : (j - 6 == i ? 1.0 : 0.0);
-    for (int c = 0; c < 6; ++c) {
-        int piv = c;
-        for (int r = c + 1; r < 6; ++r)
-            if (fabs(A[r][c]) > fabs(A[piv][c])) piv = r;
-        if (fabs(A[piv][c]) < 1e-300) return MAVD_ERR_INVALID;
-        if (piv != c)
-            for (int j = 0; j < 12; ++j) { double t = A[c][j]; A[c][j] = A[piv][j]; A[piv][j] = t; }
-        const double d = A[c][c];
-        for (int j = 0; j < 12; ++j) A[c][j] /= d;
-        for (int r = 0; r < 6; ++r)
-            if (r != c) {
-                const double f = A[r][c];
-                if (f != 0)
-                    for (int j = 0; j < 12; ++j) A[r][j] -= f * A[c][j];
-            }
-    }
-    pc.n = n;
-    for (int k = 0; k <= kMaxPolyN; ++k) {
-        pc.g[k] = k <= n ? g[n + k] : 0.f;
-        pc.xg[k] = k <= n ? xg[n + k] : 0.f;
-        pc.xxg[k] = k <= n ? xxg[n + k] : 0.f;
-    }
-    pc.ig11 = (float)A[1][6 + 1];
-    pc.ig03 = (float)A[0][6 + 3];
-    pc.ig33 = (float)A[3][6 + 3];
-    pc.ig55 = (float)A[5][6 + 5];
-    return MAVD_OK;
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-// TMA descriptor of a rank-3 tensor {d0, d1, d2} (d0 fastest) of 4-byte floats or bytes with byte strides s1, s2 and a
-// box {b0, b1, b2}; out-of-bounds cells are filled with zeros.  Base and strides must be multiples of 16 bytes.
-bool encode_tensor_map_3d(CUtensorMap* map, bool is_u8, const void* base, uint64_t d0, uint64_t d1, uint64_t d2,
-                          uint64_t s1_bytes, uint64_t s2_bytes, uint32_t b0, uint32_t b1, uint32_t b2) {
-    static std::atomic<EncodeTiledFn> fn_cache{nullptr};
-    EncodeTiledFn fn = fn_cache.load();
-    if (!fn) {
-        void* f = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &f, cudaEnableDefault, &q) != cudaSuccess || !f) {
-            cudaGetLastError();
-            return false;
-        }
-        fn = (EncodeTiledFn)f;
-        fn_cache.store(fn);
-    }
-    if ((reinterpret_cast<uintptr_t>(base) & 15) || (s1_bytes & 15) || (s2_bytes & 15)) return false;
-    cuuint64_t dims[3] = {d0, d1, d2};
-    cuuint64_t strides[2] = {s1_bytes, s2_bytes};
-    cuuint32_t box[3] = {b0, b1, b2};
-    cuuint32_t estr[3] = {1u, 1u, 1u};
-    CUresult r = fn(map, is_u8 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3,
-                    const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                    CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    return r == CUDA_SUCCESS;
-}
-
-// TMA descriptor of a planar buffer: rank-3 float tensor {pitch, h, planes}, box {80, box_h, box_planes}, zero fill.
-static bool make_plane_tensor_map(CUtensorMap* map, float* base, int pitch, int h, int planes, size_t plane, int box_h,
-                                  int box_planes) {
-    return encode_tensor_map_3d(map, false, base, (uint64_t)pitch, (uint64_t)h, (uint64_t)planes,
-                                (uint64_t)pitch * sizeof(float), (uint64_t)plane * sizeof(float), 80u, (uint32_t)box_h,
-                                (uint32_t)box_planes);
-}
-
-struct Arena {
-    std::vector<void*> ptrs;
-    size_t bytes = 0;
-    template <typename T>
-    int alloc(T** out, size_t count) {
-        void* p = nullptr;
-        size_t b = count * sizeof(T);
-        if (b == 0) b = sizeof(T);
-        cudaError_t e = cudaMalloc(&p, b);
-        if (e != cudaSuccess) {
-            set_error("cudaMalloc(%zu bytes) failed: %s", b, cudaGetErrorString(e));
-            return e == cudaErrorMemoryAllocation ? MAVD_ERR_NOMEM : MAVD_ERR_CUDA;
-        }
-        ptrs.push_back(p);
-        bytes += b;
-        *out = (T*)p;
-        return MAVD_OK;
-    }
-    template <typename T>
-    int upload(T** out, const std::vector<T>& v) {
-        int rc = alloc(out, v.size());
-        if (rc != MAVD_OK) return rc;
-        if (!v.empty()) MAVD_CUDA(cudaMemcpy(*out, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
-        return MAVD_OK;
-    }
-};
-
-static int alloc_slot(Arena& A, mavd_handle_s::HostSlot& S, int F, int B, size_t npx) {
+static int alloc_slot(mavd_handle h, mavd_handle_s::HostSlot& S) {
+    Arena& A = h->arena;
+    const int F = h->max_frames, B = h->cfg.max_pairs;
+    const size_t npx = (size_t)h->cfg.width * h->cfg.height;
     int rc;
     if ((rc = A.alloc(&S.d_frames, (size_t)F * npx)) != MAVD_OK) return rc;
     if ((rc = A.alloc(&S.d_samples, (size_t)B * MAVD_SAMPLES_PER_FRAME)) != MAVD_OK) return rc;
@@ -204,14 +44,11 @@ static int alloc_slot(Arena& A, mavd_handle_s::HostSlot& S, int F, int B, size_t
 
 using namespace mavd;
 
-struct mavd_handle_full : mavd_handle_s {
-    Arena arena;
-};
-
 static void drop_graphs(mavd_handle h);
 
-// streams, events, graphs and pinned staging of a handle (everything but the device arena)
-static void release_host_side(mavd_handle_full* H) {
+// device memory, streams, events, graphs and pinned staging of a handle, then the handle
+static void release(mavd_handle H) {
+    for (void* p : H->arena.ptrs) cudaFree(p);
     drop_graphs(H);
     for (auto& S : H->slot) {
         if (S.ev_in) cudaEventDestroy(S.ev_in);
@@ -232,6 +69,7 @@ static void release_host_side(mavd_handle_full* H) {
     if (H->h_imu_ring) cudaFreeHost(H->h_imu_ring);
     for (auto& r : H->prof.recs) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
     for (cudaEvent_t e : H->prof.pool) cudaEventDestroy(e);
+    delete H;
 }
 
 #define TRY(x)                       \
@@ -285,170 +123,17 @@ int mavd_create(const mavd_config* cfg, mavd_handle* out) {
     MAVD_REQUIRE(cfg->device >= 0 && cfg->device < ndev, MAVD_ERR_CUDA, "CUDA device %d not available (%d devices)",
                  cfg->device, ndev);
     DeviceGuard dg(cfg->device);
-    mavd_handle_full* H = new (std::nothrow) mavd_handle_full();
+    mavd_handle H = new (std::nothrow) mavd_handle_s();
     MAVD_REQUIRE(H != nullptr, MAVD_ERR_NOMEM, "out of host memory");
     H->cfg = *cfg;
     mavd_default_tuning(&H->tune);
-    const mavd_farneback_params& fp = cfg->farneback;
-    const int W = cfg->width, Hh = cfg->height, B = cfg->max_pairs;
-    const int F = 2 * B;  // worst case: independent pairs
-    H->max_frames = F;
-    Arena& A = H->arena;
+    H->max_frames = 2 * cfg->max_pairs;  // worst case: independent pairs
     int rc = MAVD_OK;
-    auto fail = [&](int code) {
-        for (void* p : A.ptrs) cudaFree(p);
-        release_host_side(H);
-        delete H;
-        return code;
-    };
-#define C_TRY(x) do { rc = (x); if (rc != MAVD_OK) return fail(rc); } while (0)
-
-    // level schedule (SURVEY §8 a2): levels = N -> up to N+1 images, 32-pixel cap
-    int k = 0;
-    double sc = 1.0;
-    while (k < fp.levels) {
-        sc *= fp.pyr_scale;
-        if (W * sc < 32 || Hh * sc < 32) break;
-        ++k;
-    }
-    if (k + 1 > kMaxLevels) {
-        set_error("too many pyramid levels (%d)", k + 1);
-        return fail(MAVD_ERR_UNSUPPORTED);
-    }
-    H->n_levels = k + 1;
-    for (int li = 0; li < H->n_levels; ++li) {
-        Level& L = H->lv[li];
-        L.k = li;
-        double s = 1.0;
-        for (int i = 0; i < li; ++i) s *= fp.pyr_scale;
-        L.scale = s;
-        const double sigma = (1. / s - 1) * 0.5;
-        L.sigma = (float)sigma;
-        L.ksz = std::max(cv_round(sigma * 5) | 1, 3);
-        L.w = cv_round(W * s);
-        L.h = cv_round(Hh * s);
-        L.pitch = round_up(L.w, 64);
-        L.plane = (size_t)L.pitch * L.h;
-        if (li > 0) {
-            // combined blur + bilinear-resize filter per output sample: c_j = (1-a) k_j + a k_{j-1}
-            const std::vector<float> kk = gaussian_kernel(L.ksz, sigma);
-            const int taps = round_up(L.ksz + 1, 4), r = L.ksz / 2;   // zero padded to whole float4 groups
-            for (int axis = 0; axis < 2; ++axis) {
-                const int src = axis == 0 ? W : Hh, dst = axis == 0 ? L.w : L.h;
-                std::vector<int> i0;
-                std::vector<float> a;
-                resize_tables(src, dst, i0, a);
-                std::vector<int> base(dst);
-                std::vector<float> tab((size_t)dst * taps);
-                for (int d = 0; d < dst; ++d) {
-                    base[d] = i0[d] - r;
-                    for (int j = 0; j < taps; ++j) {
-                        const float k0 = j < L.ksz ? kk[j] : 0.f, k1 = (j >= 1 && j <= L.ksz) ? kk[j - 1] : 0.f;
-                        tab[(size_t)d * taps + j] = (1.f - a[d]) * k0 + a[d] * k1;
-                    }
-                }
-                {
-                    // pyr_scale 0.5 with src = dst * 2^li: the level is an exact decimation (farneback.cu: HalfPyr)
-                    static const int kT[7] = {0, 4, 10, 20, 40, 80, 160}, kNB[7] = {0, 1, 3, 6, 12, 24, 48};
-                    const int lc = std::min(li, 6);
-                    bool half = li <= 6 && L.ksz + 1 == kT[lc] && dst >= 1 && src == dst << lc;
-                    for (int d = 0; half && d < dst; ++d) {
-                        half = base[d] == (d << lc) - kNB[lc];
-                        for (int j = 0; half && j < taps; ++j) half = tab[(size_t)d * taps + j] == tab[j];
-                    }
-                    for (int j = kT[lc]; half && j < taps; ++j) half = tab[j] == 0.f;
-                    (axis == 0 ? L.x_half : L.y_half) = half;
-                    if (half) std::copy(tab.begin(), tab.begin() + kT[lc], axis == 0 ? L.xwt : L.ywt);
-                }
-                if (axis == 0) {
-                    C_TRY(A.upload(&L.xbase, base)); C_TRY(A.upload(&L.xtab, tab));
-                    std::vector<float> tabT((size_t)dst * taps);
-                    for (int d = 0; d < dst; ++d)
-                        for (int j = 0; j < taps; ++j) tabT[(size_t)j * dst + d] = tab[(size_t)d * taps + j];
-                    C_TRY(A.upload(&L.xtabT, tabT));
-                    L.hspan_max = 0;
-                    L.hstride_min = dst > 1 ? src : 0;
-                    for (int d0 = 0; d0 < dst; d0 += 64)
-                        L.hspan_max = std::max(L.hspan_max, base[std::min(d0 + 63, dst - 1)] + taps - base[d0]);
-                    for (int d = 1; d < dst; ++d) L.hstride_min = std::min(L.hstride_min, base[d] - base[d - 1]);
-                }
-                else           { C_TRY(A.upload(&L.ybase, base)); C_TRY(A.upload(&L.ytab, tab)); }
-            }
-            C_TRY(A.alloc(&L.tmp, (size_t)F * L.h * round_up(W, 4)));   // vertical-pass output [F][h_l][Wp]
-        }
-        C_TRY(A.alloc(&L.img, (size_t)F * L.plane));
-        // polynomial expansion of the float levels: one TMA box {80, 32 + 2 poly_n} of the level image per tile
-        L.has_tmap_img = li > 0 && make_plane_tensor_map(&L.tmapImg, L.img, L.pitch, L.h, F, L.plane, 32 + 2 * fp.poly_n, 1);
-        C_TRY(A.alloc(&L.R, (size_t)F * 5 * L.plane));
-        C_TRY(A.alloc(&L.M[0], (size_t)B * 5 * L.plane));
-        C_TRY(A.alloc(&L.M[1], (size_t)B * 5 * L.plane));
-        if (li > 0) C_TRY(A.alloc(&L.flow, (size_t)B * 2 * L.plane));
-        // padded columns of R/M are read by vector loads of edge tiles: keep them finite
-        cudaMemset(L.img, 0, (size_t)F * L.plane * sizeof(float));
-        cudaMemset(L.R, 0, (size_t)F * 5 * L.plane * sizeof(float));
-        cudaMemset(L.M[0], 0, (size_t)B * 5 * L.plane * sizeof(float));
-        cudaMemset(L.M[1], 0, (size_t)B * 5 * L.plane * sizeof(float));
-        const int m = fp.winsize / 2;
-        if (m >= 5 && m <= 8)
-            L.has_tmap = make_plane_tensor_map(&L.tmapM[0], L.M[0], L.pitch, L.h, B * 5, L.plane, 32 + 2 * m, 5) &&
-                         make_plane_tensor_map(&L.tmapM[1], L.M[1], L.pitch, L.h, B * 5, L.plane, 32 + 2 * m, 5) &&
-                         make_plane_tensor_map(&L.tmapR, L.R, L.pitch, L.h, F * 5, L.plane, 48, 10) &&
-                         make_plane_tensor_map(&L.tmapRbox, L.R, L.pitch, L.h, F * 5, L.plane, 32 + 2 * m, 5);
-        if (L.has_tmap)
-            L.has_tmap16 = make_plane_tensor_map(&L.tmapM16[0], L.M[0], L.pitch, L.h, B * 5, L.plane, 16 + 2 * m, 5) &&
-                           make_plane_tensor_map(&L.tmapM16[1], L.M[1], L.pitch, L.h, B * 5, L.plane, 16 + 2 * m, 5) &&
-                           make_plane_tensor_map(&L.tmapRbox16, L.R, L.pitch, L.h, F * 5, L.plane, 16 + 2 * m, 5);
-    }
-    for (int li = 0; li + 1 < H->n_levels; ++li) {
-        Level& L = H->lv[li];
-        const Level& C = H->lv[li + 1];
-        std::vector<int> i0;
-        std::vector<float> a;
-        resize_tables(C.w, L.w, i0, a);
-        C_TRY(A.upload(&L.fxi0, i0));
-        C_TRY(A.upload(&L.fxa, a));
-        resize_tables(C.h, L.h, i0, a);
-        C_TRY(A.upload(&L.fyi0, i0));
-        C_TRY(A.upload(&L.fya, a));
-    }
-    C_TRY(poly_setup(fp.poly_n, fp.poly_sigma, H->poly));
-    {
-        // FarnebackUpdateFlow_GaussianBlur half kernel
-        const int m = fp.winsize / 2;
-        const double sigma = m * 0.3;
-        std::vector<float> kf(m + 1);
-        double s = 0;
-        for (int i = 0; i <= m; ++i) {
-            kf[i] = (float)exp(-i * i / (2 * sigma * sigma));
-            s += (i == 0 ? 1.0 : 2.0) * kf[i];
-        }
-        for (int i = 0; i <= m; ++i) kf[i] = (float)(kf[i] * (1.0 / s));
-        C_TRY(A.upload(&H->gauss_win, kf));
-    }
-    // detection workspace
-    const size_t npx = (size_t)W * Hh;
-    C_TRY(A.alloc(&H->d_imu, B));
-    C_TRY(A.alloc(&H->d_foe, 2 * (size_t)B));
-    C_TRY(A.alloc(&H->d_ninter, B));
-    C_TRY(A.alloc(&H->d_labels, B * npx));
-    C_TRY(A.alloc(&H->d_scan, B * npx + 2 * (size_t)B * (npx / 128 + 2) + 64));   // rank, unit counts, unit list (ccl_*)
-    C_TRY(A.alloc(&H->d_total, B * npx));
-    C_TRY(A.alloc(&H->d_fixed, B * npx));
-    C_TRY(A.alloc(&H->d_flow, B * npx * 2));
-    for (int k = 0; k < MAVD_HOST_SLOTS; ++k) {
-        mavd_handle_s::HostSlot& S = H->slot[k];
-        // slot 0 is always there (mavd_detect_host stages through it); further slots appear on their first submit
-        if (k == 0) C_TRY(alloc_slot(A, S, F, B, npx));
-    }
-    C_TRY(A.alloc(&H->d_stats_tmp, B));
-    {
-        // detector.py:90-91 evaluated with host IEEE doubles: division, subtraction, exact doubling
-        std::vector<double> xn(W), yn(Hh);
-        for (int x = 0; x < W; ++x) { volatile double q = (double)x / (double)W; volatile double d = q - 0.5; xn[x] = -d * 2.0; }
-        for (int y = 0; y < Hh; ++y) { volatile double q = (double)y / (double)Hh; volatile double d = q - 0.5; yn[y] = -d * 2.0; }
-        C_TRY(A.upload(&H->d_xn, xn));
-        C_TRY(A.upload(&H->d_yn, yn));
-    }
+#define C_TRY(x) do { rc = (x); if (rc != MAVD_OK) { release(H); return rc; } } while (0)
+    C_TRY(farneback_setup(H));
+    C_TRY(detect_setup(H));
+    // slot 0 is always there (mavd_detect_host stages through it); further slots appear on their first submit
+    C_TRY(alloc_slot(H, H->slot[0]));
     {
         int lo = 0, hi = 0;
         cudaDeviceGetStreamPriorityRange(&lo, &hi);
@@ -467,33 +152,30 @@ int mavd_create(const mavd_config* cfg, mavd_handle* out) {
         }
     }
     {
-        cudaError_t e = cudaMallocHost((void**)&H->h_imu_ring, sizeof(mavd_imu) * mavd_handle_s::kImuRing * (size_t)B);
+        cudaError_t e = cudaMallocHost((void**)&H->h_imu_ring,
+                                       sizeof(mavd_imu) * mavd_handle_s::kImuRing * (size_t)cfg->max_pairs);
         for (int k = 0; e == cudaSuccess && k < mavd_handle_s::kImuRing; ++k)
             e = cudaEventCreateWithFlags(&H->imu_ev[k], cudaEventDisableTiming);
         if (e != cudaSuccess) {
             set_error("imu staging: %s", cudaGetErrorString(e));
-            return fail(e == cudaErrorMemoryAllocation ? MAVD_ERR_NOMEM : MAVD_ERR_CUDA);
+            C_TRY(e == cudaErrorMemoryAllocation ? MAVD_ERR_NOMEM : MAVD_ERR_CUDA);
         }
     }
-    H->bytes = A.bytes;
     cudaError_t e = cudaDeviceSynchronize();
     if (e != cudaSuccess) {
         set_error("device error during create: %s", cudaGetErrorString(e));
-        return fail(MAVD_ERR_CUDA);
+        C_TRY(MAVD_ERR_CUDA);
     }
+#undef C_TRY
     *out = H;
     return MAVD_OK;
-#undef C_TRY
 }
 
 int mavd_destroy(mavd_handle h) {
     if (!h) return MAVD_OK;
-    mavd_handle_full* H = static_cast<mavd_handle_full*>(h);
-    DeviceGuard dg(H->cfg.device);
+    DeviceGuard dg(h->cfg.device);
     cudaDeviceSynchronize();
-    for (void* p : H->arena.ptrs) cudaFree(p);
-    release_host_side(H);
-    delete H;
+    release(h);
     return MAVD_OK;
 }
 
@@ -589,7 +271,7 @@ int mavd_debug_force_generic_iteration(mavd_handle h, int32_t on) {
 
 int mavd_workspace_bytes(mavd_handle h, size_t* out) {
     MAVD_REQUIRE(h && out, MAVD_ERR_INVALID, "NULL argument");
-    *out = h->bytes;
+    *out = h->arena.bytes;
     return MAVD_OK;
 }
 
@@ -760,11 +442,8 @@ static int check_det(mavd_handle h, int max_det, const void* det, const char* wh
     MAVD_REQUIRE((reinterpret_cast<uintptr_t>(det) & 7) == 0, MAVD_ERR_INVALID, "%s: detections must be 8-byte aligned",
                  what);
     if (h->d_det_area) return MAVD_OK;
-    mavd_handle_full* H = static_cast<mavd_handle_full*>(h);
-    TRY(H->arena.alloc(&H->d_det_area, (size_t)h->cfg.max_pairs * det_lab_stride(h)));
-    TRY(H->arena.alloc(&H->d_det_nlabels, (size_t)h->cfg.max_pairs));
-    H->bytes = H->arena.bytes;
-    return MAVD_OK;
+    TRY(h->arena.alloc(&h->d_det_area, (size_t)h->cfg.max_pairs * det_lab_stride(h)));
+    return h->arena.alloc(&h->d_det_nlabels, (size_t)h->cfg.max_pairs);
 }
 
 int mavd_detections(mavd_handle h, const uint8_t* d_mask, int32_t n, const float* d_flow, const mavd_imu* h_imu,
@@ -780,29 +459,6 @@ int mavd_detections(mavd_handle h, const uint8_t* d_mask, int32_t n, const float
     if (d_flow) TRY(upload_imu(h, h_imu, n, s, nullptr, nullptr));
     const DetArgs da{d_det, max_det, h->d_det_area, det_lab_stride(h), d_flow, h->d_imu};
     return ccl_run(h, d_mask, n, nullptr, nullptr, 0, 0, h->d_det_nlabels, sizeof(int32_t), s, false, &da);
-}
-
-// The corner workspace of mavd::gftt_chunk() frames, carved from one allocation made by the first corner call.
-static GfttWork gftt_work(mavd_handle h) {
-    const int W = h->cfg.width, Hh = h->cfg.height, G = gftt_chunk();
-    const size_t npx = (size_t)W * Hh;
-    char* p = (char*)h->sp_gftt;
-    GfttWork w;
-    w.rows = (double*)p;                  p += sizeof(double) * 3 * npx * G;
-    w.keys = (unsigned long long*)p;      p += sizeof(unsigned long long) * gftt_key_cap(W, Hh) * G;
-    w.cov = (float3*)p;                   p += sizeof(float3) * npx * G;
-    w.eig = (float*)p;                    p += sizeof(float) * npx * G;
-    w.grid = (int*)p;                     p += sizeof(int) * gftt_grid_cap(W, Hh) * G;
-    w.maxv = (uint32_t*)p;                p += sizeof(uint32_t) * G;
-    w.n_cand = (int*)p;
-    return w;
-}
-
-static size_t gftt_work_bytes(mavd_handle h) {
-    const int W = h->cfg.width, Hh = h->cfg.height, G = gftt_chunk();
-    const size_t npx = (size_t)W * Hh;
-    return (sizeof(double) * 3 * npx + sizeof(unsigned long long) * gftt_key_cap(W, Hh) + sizeof(float3) * npx +
-            sizeof(float) * npx + sizeof(int) * gftt_grid_cap(W, Hh) + sizeof(uint32_t) + sizeof(int)) * G;
 }
 
 int mavd_good_features_to_track(mavd_handle h, const uint8_t* d_frames, int32_t n_frames, const mavd_gftt_params* prm,
@@ -827,14 +483,7 @@ int mavd_good_features_to_track(mavd_handle h, const uint8_t* d_frames, int32_t 
     if (n_frames == 0) return MAVD_OK;
     MAVD_REQUIRE(d_frames && d_count && (d_corners || p.max_corners == 0), MAVD_ERR_INVALID,
                  "good_features_to_track: NULL buffer");
-    if (!h->sp_gftt) {
-        mavd_handle_full* H = static_cast<mavd_handle_full*>(h);
-        char* base = nullptr;
-        TRY(H->arena.alloc(&base, gftt_work_bytes(h)));
-        H->sp_gftt = base;
-        H->bytes = H->arena.bytes;
-    }
-    return gftt_run(h, gftt_work(h), d_frames, n_frames, p, d_mask, d_mask ? mask_stride : 0, d_corners, d_count, d_eig,
+    return gftt_run(h, d_frames, n_frames, p, d_mask, d_mask ? mask_stride : 0, d_corners, d_count, d_eig,
                     (cudaStream_t)stream);
 }
 
@@ -861,19 +510,8 @@ int mavd_pyr_lk(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int32_t
                  "pyr_lk: criteria_type %d not supported", p.criteria_type);
     if (n_pairs == 0 || n_points == 0) return MAVD_OK;
     MAVD_REQUIRE(d_frames && d_prev_pts && d_next_pts && d_status && d_err, MAVD_ERR_INVALID, "pyr_lk: NULL buffer");
-    if (!h->sp_pyr) {
-        mavd_handle_full* H = static_cast<mavd_handle_full*>(h);
-        const int W = h->cfg.width, Hh = h->cfg.height;
-        uint8_t* pyr = nullptr;
-        short2* der = nullptr;
-        TRY(H->arena.alloc(&pyr, (size_t)h->max_frames * lk_pyr_frame_bytes(W, Hh)));
-        TRY(H->arena.alloc(&der, (size_t)h->max_frames * lk_der_frame_elems(W, Hh)));
-        H->sp_pyr = pyr;
-        H->sp_der = der;
-        H->bytes = H->arena.bytes;
-    }
-    return lk_run(h, h->sp_pyr, h->sp_der, d_frames, n_pairs, pair_stride, p, d_prev_pts, n_points, d_n_points,
-                  d_next_pts, d_status, d_err, (cudaStream_t)stream);
+    return lk_run(h, d_frames, n_pairs, pair_stride, p, d_prev_pts, n_points, d_n_points, d_next_pts, d_status, d_err,
+                  (cudaStream_t)stream);
 }
 
 int mavd_ccl(mavd_handle h, const uint8_t* d_mask, int32_t n, int32_t* d_labels, int32_t* d_boxes, int32_t max_boxes,
@@ -1161,21 +799,20 @@ int mavd_process(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int32_
 // ------------------------------------------------------------------------------------------------
 static int ensure_slot(mavd_handle h, int slot, bool want_flow_out, bool want_flow_in, bool want_bits_in, bool want_bits_out,
                        bool want_gt, bool want_det) {
-    mavd_handle_full* H = static_cast<mavd_handle_full*>(h);
-    mavd_handle_s::HostSlot& S = H->slot[slot];
+    mavd_handle_s::HostSlot& S = h->slot[slot];
     const size_t npx = (size_t)h->cfg.width * h->cfg.height;
     const size_t pb = (size_t)packed_mask_bytes((int64_t)npx);
     const int B = h->cfg.max_pairs;
-    if (!S.d_frames) TRY(alloc_slot(H->arena, S, h->max_frames, B, npx));
-    if (want_flow_out && !S.d_flow) TRY(H->arena.alloc(&S.d_flow, B * npx * 2));
-    if (want_flow_in && !S.d_flow_in) TRY(H->arena.alloc(&S.d_flow_in, B * npx * 2));
-    if (want_bits_in && !S.d_bits_in) TRY(H->arena.alloc(&S.d_bits_in, 2 * B * pb));
-    if (want_bits_out && !S.d_bits_out) TRY(H->arena.alloc(&S.d_bits_out, B * pb));
-    if (want_gt && !S.d_gt_flow) TRY(H->arena.alloc(&S.d_gt_flow, B * npx * 2));
-    if (want_det && !S.d_det) TRY(H->arena.alloc(&S.d_det, (size_t)B * MAVD_MAX_DETECTIONS));
-    if (!H->s_in) MAVD_CUDA(cudaStreamCreateWithFlags(&H->s_in, cudaStreamNonBlocking));
-    if (!H->s_out) MAVD_CUDA(cudaStreamCreateWithFlags(&H->s_out, cudaStreamNonBlocking));
-    H->bytes = H->arena.bytes;
+    Arena& A = h->arena;
+    if (!S.d_frames) TRY(alloc_slot(h, S));
+    if (want_flow_out && !S.d_flow) TRY(A.alloc(&S.d_flow, B * npx * 2));
+    if (want_flow_in && !S.d_flow_in) TRY(A.alloc(&S.d_flow_in, B * npx * 2));
+    if (want_bits_in && !S.d_bits_in) TRY(A.alloc(&S.d_bits_in, 2 * B * pb));
+    if (want_bits_out && !S.d_bits_out) TRY(A.alloc(&S.d_bits_out, B * pb));
+    if (want_gt && !S.d_gt_flow) TRY(A.alloc(&S.d_gt_flow, B * npx * 2));
+    if (want_det && !S.d_det) TRY(A.alloc(&S.d_det, (size_t)B * MAVD_MAX_DETECTIONS));
+    if (!h->s_in) MAVD_CUDA(cudaStreamCreateWithFlags(&h->s_in, cudaStreamNonBlocking));
+    if (!h->s_out) MAVD_CUDA(cudaStreamCreateWithFlags(&h->s_out, cudaStreamNonBlocking));
     return MAVD_OK;
 }
 
@@ -1289,11 +926,7 @@ int mavd_submit_host(mavd_handle h, int32_t slot, const uint8_t* h_frames, int32
     mavd_handle_s::HostSlot& S = h->slot[slot];
     MAVD_REQUIRE(!S.busy, MAVD_ERR_INVALID, "slot %d is still in flight: call mavd_wait_host first", slot);
     const int n_frames = pair_stride == 1 ? n_pairs + 1 : 2 * n_pairs;
-    if (bgr && !S.d_bgr) {
-        mavd_handle_full* H = static_cast<mavd_handle_full*>(h);
-        TRY(H->arena.alloc(&S.d_bgr, (size_t)h->max_frames * npx * 3));
-        H->bytes = H->arena.bytes;
-    }
+    if (bgr && !S.d_bgr) TRY(h->arena.alloc(&S.d_bgr, (size_t)h->max_frames * npx * 3));
     StreamScope ss(h, stream);
     cudaStream_t s = ss.s;
     // copy-in stream (BGR frames are converted to gray there too, so the compute stream sees gray frames only)

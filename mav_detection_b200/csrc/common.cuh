@@ -115,6 +115,35 @@ static inline int round_up(int a, int b) { return ceil_div(a, b) * b; }
 constexpr int kMaxPolyN = 8;
 constexpr int kMaxLevels = 16;
 constexpr int kMaxWinHalf = 31;
+constexpr int HP_MAXT = 160;   // taps of the coarsest exact power-of-two level (farneback.cu: HalfPyr, HP_MAXLV)
+
+// Every device allocation of a handle: freed together by mavd_destroy, counted by mavd_workspace_bytes.
+struct Arena {
+    std::vector<void*> ptrs;
+    size_t bytes = 0;
+    template <typename T>
+    int alloc(T** out, size_t count) {
+        void* p = nullptr;
+        size_t b = count * sizeof(T);
+        if (b == 0) b = sizeof(T);
+        cudaError_t e = cudaMalloc(&p, b);
+        if (e != cudaSuccess) {
+            set_error("cudaMalloc(%zu bytes) failed: %s", b, cudaGetErrorString(e));
+            return e == cudaErrorMemoryAllocation ? MAVD_ERR_NOMEM : MAVD_ERR_CUDA;
+        }
+        ptrs.push_back(p);
+        bytes += b;
+        *out = (T*)p;
+        return MAVD_OK;
+    }
+    template <typename T>
+    int upload(T** out, const std::vector<T>& v) {
+        int rc = alloc(out, v.size());
+        if (rc != MAVD_OK) return rc;
+        if (!v.empty()) MAVD_CUDA(cudaMemcpy(*out, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
+        return MAVD_OK;
+    }
+};
 
 // One pyramid level: geometry, resize/blur tables and per-level buffers (all device memory).
 struct Level {
@@ -135,7 +164,7 @@ struct Level {
     // exact power-of-two level (farneback.cu: HalfPyr): every output sample has the same ksz + 1 weights and its window
     // starts 2^k samples after its neighbour's; host copies of those weights for the kernels that exploit it
     bool x_half = false, y_half = false;
-    float xwt[160] = {}, ywt[160] = {};
+    float xwt[HP_MAXT] = {}, ywt[HP_MAXT] = {};
     // flow upsample tables (next-coarser level -> this level)
     int* fxi0 = nullptr; float* fxa = nullptr;  // [w]
     int* fyi0 = nullptr; float* fya = nullptr;  // [h]
@@ -145,14 +174,15 @@ struct Level {
     float* M[2] = {nullptr, nullptr};  // [pairs][5][h][pitch]
     float* flow = nullptr;  // [pairs][h][pitch] float2 (unused for level 0: written to the caller's buffer)
     int last_m = 0;         // which M buffer holds the last update (for taps)
-    CUtensorMap tmapM[2];   // TMA descriptors of M[0] / M[1]: dims {pitch, h, pairs*5}, box {80, 32+2m, 5}
-    CUtensorMap tmapR;      // TMA descriptor of R: dims {pitch, h, frames*5}, box {80, 48, 10} (L2 prefetch only)
-    CUtensorMap tmapRbox;   // TMA descriptor of R with the M box geometry {80, 32+2m, 5}: R1 staged in shared memory
+    // TMA descriptors (farneback.cu: farneback_setup builds them with the boxes their kernels expect)
+    CUtensorMap tmapM[2];   // M[0] / M[1], 64 x 32 tiles
+    CUtensorMap tmapR;      // R, L2 prefetch only
+    CUtensorMap tmapRbox;   // R with the M box geometry: R1 staged in shared memory
     bool has_tmap = false;
-    CUtensorMap tmapM16[2]; // the same with 64 x 16 tiles: box {80, 16+2m, 5}
+    CUtensorMap tmapM16[2]; // the same with 64 x 16 tiles
     CUtensorMap tmapRbox16;
     bool has_tmap16 = false;
-    CUtensorMap tmapImg;    // TMA descriptor of img: dims {pitch, h, frames}, box {80, 32+2 poly_n, 1} (polynomial expansion)
+    CUtensorMap tmapImg;    // img, polynomial expansion of the levels >= 1
     bool has_tmap_img = false;
 };
 
@@ -201,14 +231,14 @@ struct mavd_handle_s {
     mavd::PolyConst poly;
     float* gauss_win = nullptr;     // [m+1] device, FarnebackUpdateFlow_GaussianBlur half kernel
     int max_frames = 0;
-    size_t bytes = 0;
+    mavd::Arena arena;
     // detection workspace
     mavd_imu* d_imu = nullptr;      // [max_pairs]
     double* d_foe = nullptr;        // [max_pairs][2]
     int32_t* d_ninter = nullptr;    // [max_pairs]
     int32_t* d_labels = nullptr;    // [max_pairs][H][W]
-    int32_t* d_scan = nullptr;      // CCL scratch
-    double* d_xn = nullptr;         // [W] -(x/w - 0.5)*2, detector.py:90 (host-built, IEEE identical to NumPy)
+    int32_t* d_scan = nullptr;      // labelling scratch (detect.cu: ccl_scratch_ints)
+    double* d_xn = nullptr;         // [W] -(x/w - 0.5)*2, detector.py:90 (detect.cu: residual_setup)
     double* d_yn = nullptr;         // [H] -(y/h - 0.5)*2, detector.py:91
     mavd_frame_stats* d_stats_tmp = nullptr;  // [max_pairs] scratch for mavd_get_phi
     bool force_exact_residual = false;        // tests: disable the float32 pre-decision
@@ -219,7 +249,7 @@ struct mavd_handle_s {
     int32_t* d_det_area = nullptr;  // [max_pairs][det_lab_stride]: area per label, then -(slot + 1) of a selected label
     int32_t* d_det_nlabels = nullptr;   // [max_pairs] label counts of mavd_detections
     // sparse features (allocated by the first call that needs them: mavd_workspace_bytes is unchanged otherwise)
-    void* sp_gftt = nullptr;        // corner workspace of mavd::gftt_chunk() frames (sparse.cu: gftt_run)
+    void* sp_gftt = nullptr;        // corner workspace (sparse.cu: gftt_layout)
     uint8_t* sp_pyr = nullptr;      // [max_frames] pyramid levels 1.. of mavd_pyr_lk
     short2* sp_der = nullptr;       // [max_frames] int16 Scharr derivatives of every level
     // host-path staging: MAVD_HOST_SLOTS independent sets of device buffers + the streams/events that let
@@ -288,14 +318,15 @@ static inline bool pdl_next(mavd_handle h, int lane = 0) {
 }
 static inline void pdl_break(mavd_handle h, int lane = 0) { h->pdl_ok[lane] = false; }
 
-// api.cu
-bool encode_tensor_map_3d(CUtensorMap* map, bool is_u8, const void* base, uint64_t d0, uint64_t d1, uint64_t d2,
-                          uint64_t s1_bytes, uint64_t s2_bytes, uint32_t b0, uint32_t b1, uint32_t b2);
 // farneback.cu
+// the pyramid levels of a new handle: schedule, tables, buffers and TMA descriptors (from h->cfg and h->max_frames)
+int farneback_setup(mavd_handle h);
 int farneback_run(mavd_handle h, const uint8_t* d_frames, int n_pairs, int pair_stride, float* d_flow,
                   cudaStream_t s);
 int farneback_tap(mavd_handle h, int kind, int level, int index, float* d_out, cudaStream_t s);
 // detect.cu
+// the detection workspace of a new handle (the host slots are api.cu's)
+int detect_setup(mavd_handle h);
 int bgr2gray_run(const uint8_t* d_bgr, uint8_t* d_gray, int64_t n, cudaStream_t s);
 int derotate_run(mavd_handle h, const void* d_flow, int flow_is_f64, int n, const mavd_imu* d_imu, double* d_out,
                  cudaStream_t s);
@@ -344,25 +375,10 @@ static inline int det_lab_stride(mavd_handle h) { return ((h->cfg.width + 1) / 2
 int ccl_run(mavd_handle h, const uint8_t* d_mask, int n, int32_t* d_labels, int32_t* d_boxes, size_t boxes_stride,
             int max_boxes, int32_t* d_n_labels, size_t nlabels_stride_bytes, cudaStream_t s, bool list_ready = false,
             const DetArgs* det = nullptr);
-// sparse.cu: corners and pyramidal Lucas-Kanade
-struct GfttWork {
-    float3* cov;                    // [chunk][H][W] products of the Sobel derivatives
-    double* rows;                   // [chunk][H][W][3] row sums of the block
-    float* eig;                     // [chunk][H][W] when the caller wants no eig image
-    unsigned long long* keys;       // [chunk][gftt_key_cap] candidates
-    int* grid;                      // [chunk][gftt_grid_cap] accepted corners by cell
-    uint32_t* maxv;                 // [chunk]
-    int* n_cand;                    // [chunk]
-};
-size_t gftt_key_cap(int W, int H);
-size_t gftt_grid_cap(int W, int H);
-int gftt_chunk();
-int gftt_run(mavd_handle h, const GfttWork& ws, const uint8_t* d_frames, int n, const mavd_gftt_params& p,
-             const uint8_t* d_mask, int64_t mask_stride, float* d_corners, int32_t* d_count, float* d_eig,
-             cudaStream_t s);
-size_t lk_pyr_frame_bytes(int W, int H);
-size_t lk_der_frame_elems(int W, int H);
-int lk_run(mavd_handle h, uint8_t* pyr, short2* der, const uint8_t* d_frames, int n_pairs, int pair_stride,
-           const mavd_lk_params& p, const float* d_prev, int n_points, const int32_t* d_n_points, float* d_next,
-           uint8_t* d_status, float* d_err, cudaStream_t s);
+// sparse.cu: corners and pyramidal Lucas-Kanade (each allocates its workspace in h->arena on its first call)
+int gftt_run(mavd_handle h, const uint8_t* d_frames, int n, const mavd_gftt_params& p, const uint8_t* d_mask,
+             int64_t mask_stride, float* d_corners, int32_t* d_count, float* d_eig, cudaStream_t s);
+int lk_run(mavd_handle h, const uint8_t* d_frames, int n_pairs, int pair_stride, const mavd_lk_params& p,
+           const float* d_prev, int n_points, const int32_t* d_n_points, float* d_next, uint8_t* d_status, float* d_err,
+           cudaStream_t s);
 }  // namespace mavd

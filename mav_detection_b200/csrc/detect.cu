@@ -799,6 +799,17 @@ __global__ void stats_final_kernel(char* stats_base, size_t stats_stride, int n,
     if (no_max_phi && (imu == nullptr || imu[f].derotate != 0)) st->max_phi = -1.0;
 }
 
+// The derotation tables xn, yn of residual_kernel: detector.py:90-91 evaluated with host IEEE doubles (division,
+// subtraction, exact doubling).
+static int residual_setup(mavd_handle H) {
+    const int W = H->cfg.width, Hh = H->cfg.height;
+    std::vector<double> xn(W), yn(Hh);
+    for (int x = 0; x < W; ++x) { volatile double q = (double)x / (double)W; volatile double d = q - 0.5; xn[x] = -d * 2.0; }
+    for (int y = 0; y < Hh; ++y) { volatile double q = (double)y / (double)Hh; volatile double d = q - 0.5; yn[y] = -d * 2.0; }
+    TRY_RC(H->arena.upload(&H->d_xn, xn));
+    return H->arena.upload(&H->d_yn, yn);
+}
+
 template <int MODE, bool FAST>
 static int launch_residual(const ResidualArgs& A, const FastPrm& fp, int n, bool vec4, cudaStream_t s, bool pdl,
                            bool no_rotation = false) {
@@ -828,7 +839,7 @@ int residual_prepare(mavd_handle H, int n, const uint8_t* d_seg, int64_t seg_str
                      size_t stats_stride, cudaStream_t s, int lane) {
     if (!d_stats) return MAVD_OK;
     ProfScope ps(&H->prof, MAVD_PROF_RESIDUAL, s);
-    int* seg_max = reinterpret_cast<int*>(H->d_scan);  // scratch: n ints
+    int* seg_max = reinterpret_cast<int*>(H->d_scan);  // scratch: n ints (ccl_scratch_ints)
     MAVD_CUDA(launch_chained(pdl_next(H, lane), stats_init_kernel, ceil_div(n, 128), 128, 0, s, (char*)d_stats, stats_stride, n,
                              d_seg ? seg_max : nullptr));
     MAVD_LAUNCHED();
@@ -850,7 +861,7 @@ int residual_run(mavd_handle H, const void* d_flow, int flow_kind, int n, const 
     ProfScope ps(&H->prof, MAVD_PROF_RESIDUAL, s);
     const int w = H->cfg.width, h = H->cfg.height;
     const int64_t npx = (int64_t)w * h;
-    int* seg_max = reinterpret_cast<int*>(H->d_scan);  // scratch: n ints
+    int* seg_max = reinterpret_cast<int*>(H->d_scan);  // scratch: n ints (ccl_scratch_ints)
     // FAST needs: phi not requested, and the parameter ranges its guard bands were derived for
     const bool fast = !H->force_exact_residual && d_phi == nullptr && p.fixed_angle >= 0.0 && p.dyn_gain >= 0.0 &&
                       p.dyn_offset - p.dyn_base < -1e-2 && p.dyn_min_mag >= 0.0 && p.fixed_min_mag >= 0.0 &&
@@ -2127,12 +2138,37 @@ __global__ void det_final_kernel(mavd_detection* det, int total) {
     d.box[3] = d.box[3] - d.box[1] + 1;
 }
 
-// scratch behind the rank array: [count (4 ints)] [unit_cnt: max_pairs x n_units] [entries: max_pairs x n_units]
+// The labelling scratch d_scan, in ints:
+//   rank   [max_pairs][npx]       ccl_launch: label ranks, written and read at roots only; its first n ints are also
+//                                 the per-frame segmentation maxima (seg_max) of residual_prepare / residual_run
+//   count  [4]                    ccl_unit_count: entries of the unit list
+//   marks  [max_pairs][n_units]   ccl_unit_marks: "listed" mark, then root count, then label offset of each unit
+//   list   [max_pairs][n_units]   ccl_unit_list: the occupied CCL_UNIT-pixel units
 int ccl_n_units(mavd_handle H) { return ceil_div(H->cfg.width * H->cfg.height, CCL_UNIT); }
 static int* ccl_count_ptr(mavd_handle H) { return H->d_scan + (size_t)H->cfg.max_pairs * H->cfg.width * H->cfg.height; }
 int* ccl_unit_marks(mavd_handle H) { return ccl_count_ptr(H) + 4; }
 int* ccl_unit_list(mavd_handle H) { return ccl_unit_marks(H) + (size_t)H->cfg.max_pairs * ccl_n_units(H); }
 int* ccl_unit_count(mavd_handle H) { return ccl_count_ptr(H); }
+// npx / CCL_UNIT + 2 >= ccl_n_units per frame and array, 64 >= the count
+static size_t ccl_scratch_ints(mavd_handle H) {
+    const size_t B = H->cfg.max_pairs, npx = (size_t)H->cfg.width * H->cfg.height;
+    return B * npx + 2 * B * (npx / CCL_UNIT + 2) + 64;
+}
+
+int detect_setup(mavd_handle H) {
+    Arena& A = H->arena;
+    const size_t B = H->cfg.max_pairs, npx = (size_t)H->cfg.width * H->cfg.height;
+    TRY_RC(A.alloc(&H->d_imu, B));
+    TRY_RC(A.alloc(&H->d_foe, 2 * B));
+    TRY_RC(A.alloc(&H->d_ninter, B));
+    TRY_RC(A.alloc(&H->d_labels, B * npx));
+    TRY_RC(A.alloc(&H->d_scan, ccl_scratch_ints(H)));
+    TRY_RC(A.alloc(&H->d_total, B * npx));
+    TRY_RC(A.alloc(&H->d_fixed, B * npx));
+    TRY_RC(A.alloc(&H->d_flow, B * npx * 2));
+    TRY_RC(A.alloc(&H->d_stats_tmp, B));
+    return residual_setup(H);
+}
 
 // zeroes the list counter and the per-unit marks of n frames (a kernel, not a memset: it stays inside the chain of
 // programmatic dependent launches, common.cuh)

@@ -21,6 +21,10 @@
 //                             5..8 (winsize 10..17), 64x32 or 64x16 tiles                88P (28P for the last)
 //   iter_kernel               the same for the other window sizes (generic staging); reference of the bit-equality tests
 #include <math.h>
+#include <string.h>
+
+#include <algorithm>
+#include <vector>
 
 #include "common.cuh"
 
@@ -210,10 +214,10 @@ __global__ void __launch_bounds__(256) pyr_hsecond_staged_kernel(int W, int Wp, 
 }
 
 // ------------------------------------------------------------------------------------------------
-// Exact power-of-two levels (pyr_scale 0.5, frame size divisible by 2^l; api.cu checks the tables): every output
-// sample of level l has the SAME T = ksz + 1 weights and its window starts S = 2^l samples after its neighbour's,
-// at S * d - NB.  The generic kernels above do not know that: they convert every u8 sample once per tap that uses it
-// (2.5 times per level) and spend most of their instructions finding their level and their table rows.
+// Exact power-of-two levels (pyr_scale 0.5, frame size divisible by 2^l; farneback_setup checks the tables): every
+// output sample of level l has the SAME T = ksz + 1 weights and its window starts S = 2^l samples after its
+// neighbour's, at S * d - NB.  The generic kernels above do not know that: they convert every u8 sample once per tap
+// that uses it (2.5 times per level) and spend most of their instructions finding their level and their table rows.
 //   pyr_vsweep   vertical pass of levels 1..NLV in ONE sweep down the frame: thread = 4 adjacent columns (one 32-bit
 //                word per row, coalesced), each row is loaded and converted once and added to the <= 3 live output
 //                rows of every level (polyphase decimation: the tap index of (row, live output) is a compile-time
@@ -233,7 +237,8 @@ struct HalfPyr {    // level l = 1..6: stride, taps, -(window start of output 0)
     __host__ __device__ static constexpr int K(int l) { return (T(l) + S(l) - 1) / S(l); }
 };
 constexpr int VS_MAXLV = 4, VS_MAXT = 40;      // levels one sweep takes; their taps
-constexpr int HP_MAXLV = 6, HP_MAXT = 160;     // levels with a uniform horizontal pass; their taps
+constexpr int HP_MAXLV = 6;                    // levels with a uniform horizontal pass; their taps are HP_MAXT
+static_assert(HalfPyr::T(HP_MAXLV) == HP_MAXT && HalfPyr::T(VS_MAXLV) == VS_MAXT, "tap counts of the last levels");
 struct VSweepDesc {
     float* tmp[VS_MAXLV];
     size_t tmp_stride[VS_MAXLV];   // floats per frame
@@ -725,7 +730,7 @@ __device__ __forceinline__ void update_matrices_px(int x, int y, int w, int h, i
 
 // Level entry: flow_l = resize(flow_{l+1}) * (1/pyr_scale) (zeros on the coarsest level), then
 // UpdateMatrices.  The upsampled flow itself is never stored: BlurBox rebuilds the flow from M alone.
-// cv::resize(INTER_LINEAR) source index / weight of destination index d (api.cu: resize_tables), evaluated with the
+// cv::resize(INTER_LINEAR) source index / weight of destination index d (resize_tables below), evaluated with the
 // same double operations, one rounding each, so the values equal the host-built tables bit for bit
 __device__ __forceinline__ void resize_coord(int d, double scale, int src, int& i0, float& a) {
     const float f = (float)__dsub_rn(__dmul_rn(__dadd_rn((double)d, 0.5), scale), 0.5);
@@ -819,6 +824,11 @@ __global__ void __launch_bounds__(256, 8) matrices_init_kernel(const float* __re
 // phase is per pixel with x fastest so R0 loads, the R1 gather and the M' stores are coalesced.
 // ------------------------------------------------------------------------------------------------
 constexpr int IT_TX = 64, IT_TY = 32;
+// iter_box_tma_kernel: 64 x IT_TY_SMALL tiles for launches that would leave SMs idle; the box of M (and of R1) is IT_RW
+// columns, IT_HX of them halo on each side; the R prefetch box covers IT_PF_ROWS rows of the IT_PF_PLANES planes of
+// both frames
+constexpr int IT_TY_SMALL = 16, IT_HX = 8, IT_RW = IT_TX + 2 * IT_HX;
+constexpr int IT_PF_ROWS = IT_TY + 2 * IT_HX, IT_PF_PLANES = 2 * 5;
 // Consecutive pairs share an R plane (R1 of pair p is R0 of pair p+1): iter_box_tma_kernel interleaves the pairs of a
 // tile in groups of 4 in its CTA order so that the second reader hits L2 (4502 vs 4441 pairs/s ungrouped, 4338 with the
 // whole 64-pair batch interleaved: too many concurrent HBM regions).
@@ -1266,7 +1276,7 @@ __global__ void __launch_bounds__(256, 3) iter_box_tma_kernel(const __grid_const
                                                               const __grid_constant__ CUtensorMap tmapRbox, IterArgs a) {
     pdl_entry();
     constexpr int NT = 256;                 // threads
-    constexpr int RW = IT_TX + 16;          // 80 staged columns (halo 8 each side, 16-byte aligned)
+    constexpr int RW = IT_RW;               // staged columns (halo IT_HX each side, 16-byte aligned)
     constexpr int RH = TY + 2 * M_;      // staged rows
     constexpr int CH = RH * RW;             // floats per plane box
     constexpr int NC = IT_TX + 2 * M_;      // columns the vertical pass must produce
@@ -1307,12 +1317,12 @@ __global__ void __launch_bounds__(256, 3) iter_box_tma_kernel(const __grid_const
         // the barrier to the waiters, so the transfer is already in flight while the other warps arrive
         mbar_init(&bar, 1);
         mbar_expect_tx(&bar, 5 * CH * (uint32_t)sizeof(float));
-        tma_load_3d(box, &tmap, x0 - 8, y0 - M_, p * 5, &bar);
+        tma_load_3d(box, &tmap, x0 - IT_HX, y0 - M_, p * 5, &bar);
         // R0 (this tile) and R1 (this tile displaced by the flow) are read ~10 us from now by the per-pixel
         // phase: start their HBM -> L2 transfer now (10 consecutive planes = both frames' expansions)
-        if (!LAST) tma_prefetch_3d(&tmapR, x0 - 8, y0 - 8, p * a.pair_stride * 5);
+        if (!LAST) tma_prefetch_3d(&tmapR, x0 - IT_HX, y0 - IT_HX, p * a.pair_stride * 5);
     }
-    const bool interior = (x0 - 8 >= 0) && (x0 + IT_TX + 8 <= w) && (y0 - M_ >= 0) && (y0 + TY + M_ <= h);
+    const bool interior = (x0 - IT_HX >= 0) && (x0 + IT_TX + IT_HX <= w) && (y0 - M_ >= 0) && (y0 + TY + M_ <= h);
     __syncthreads();
     mbar_wait(&bar, 0);
 
@@ -1322,7 +1332,7 @@ __global__ void __launch_bounds__(256, 3) iter_box_tma_kernel(const __grid_const
         // whole rows above / below it (which copy already completed rows) — a few hundred cells per plane, not the
         // whole box: border tiles are 12 % of a 1080p level and up to 40 % of the coarse ones, and walking all
         // 5 x RH x 80 cells with a division each made such a tile cost twice an interior one
-        const int xlo = max(0, 8 - x0), xhi = min(RW, w - x0 + 8);          // in-image box columns [xlo, xhi)
+        const int xlo = max(0, IT_HX - x0), xhi = min(RW, w - x0 + IT_HX);  // in-image box columns [xlo, xhi)
         const int ylo = max(0, M_ - y0), yhi = min(RH, h - y0 + M_);        // in-image box rows [ylo, yhi)
         const int ncol = xlo + (RW - xhi), nrow_in = yhi - ylo;
         if (ncol > 0) {
@@ -1354,7 +1364,7 @@ __global__ void __launch_bounds__(256, 3) iter_box_tma_kernel(const __grid_const
     for (int t = warp; t < 15; t += NW) {
         const int c = t / 3, col = (t - 3 * c) * 32 + lane;
         if (col < NC) {
-            float* q = box + c * CH + (8 - M_) + col;
+            float* q = box + c * CH + (IT_HX - M_) + col;
             float in[RH];
             float s = 0.f;
 #pragma unroll
@@ -1514,7 +1524,7 @@ __global__ void __launch_bounds__(256, 3) iter_box_tma_kernel(const __grid_const
         if (cx == IT_TX / 2 && r == TY / 2) {
             // box origin: tile origin displaced by the centre pixel's flow, x a multiple of 4
             const float cfx = fminf(fmaxf(ffx[j], -1.0e5f), 1.0e5f), cfy = fminf(fmaxf(ffy[j], -1.0e5f), 1.0e5f);
-            s_org[0] = ((x0 + (int)floorf(cfx == cfx ? cfx : 0.f)) & ~3) - 8;
+            s_org[0] = ((x0 + (int)floorf(cfx == cfx ? cfx : 0.f)) & ~3) - IT_HX;
             s_org[1] = y0 + (int)floorf(cfy == cfy ? cfy : 0.f) - M_;
         }
     }
@@ -1575,7 +1585,7 @@ static int launch_iter(const IterArgs& a, dim3 grid, size_t smem, cudaStream_t s
 template <int M_, bool LAST, int TY, bool GAUSS>
 static int launch_iter_tma(const CUtensorMap& map, const CUtensorMap& mapR, const CUtensorMap& mapRbox, const IterArgs& a,
                            dim3 grid, cudaStream_t s, bool pdl) {
-    constexpr size_t smem = sizeof(float) * 5 * (TY + 2 * M_) * (IT_TX + 16);
+    constexpr size_t smem = sizeof(float) * 5 * (TY + 2 * M_) * IT_RW;
     MAVD_CUDA((ensure_dynamic_smem<iter_box_tma_kernel<M_, LAST, TY, GAUSS>>(smem)));
     MAVD_CUDA(launch_chained(pdl, iter_box_tma_kernel<M_, LAST, TY, GAUSS>, grid, 256, smem, s, map, mapR, mapRbox, a));
     MAVD_LAUNCHED();
@@ -1592,10 +1602,270 @@ static int launch_iter_tma_m(int m, bool gauss, bool small_tiles, const CUtensor
     { launch_iter_tma<5, LAST, TY, GAUSS>, launch_iter_tma<6, LAST, TY, GAUSS>, launch_iter_tma<7, LAST, TY, GAUSS>,     \
       launch_iter_tma<8, LAST, TY, GAUSS> }
     static const Launch table[2][2][4] = {   // [Gaussian window][64 x 16 tiles][m - 5]
-        {ITER_TMA_M(IT_TY, false), ITER_TMA_M(16, false)},
-        {ITER_TMA_M(IT_TY, true), ITER_TMA_M(16, true)}};
+        {ITER_TMA_M(IT_TY, false), ITER_TMA_M(IT_TY_SMALL, false)},
+        {ITER_TMA_M(IT_TY, true), ITER_TMA_M(IT_TY_SMALL, true)}};
 #undef ITER_TMA_M
     return table[gauss][small_tiles][m - 5](map, mapR, mapRbox, a, grid, s, pdl);
+}
+
+// floats per row of a level's tmp rows (the vertical-pass output): full-resolution width, whole float4 groups
+static int pyr_tmp_pitch(int W) { return round_up(W, 4); }
+
+static inline int cv_round(double v) { return (int)nearbyint(v); }  // round-half-even, like cvRound
+
+// cv::resize(INTER_LINEAR) source index / weight per destination index (pixel-centre mapping).
+static void resize_tables(int src, int dst, std::vector<int>& i0, std::vector<float>& a) {
+    i0.resize(dst);
+    a.resize(dst);
+    const double inv_scale = (double)dst / src;
+    const double scale = 1.0 / inv_scale;
+    for (int d = 0; d < dst; ++d) {
+        float f = (float)((d + 0.5) * scale - 0.5);
+        int s = (int)floorf(f);
+        float w = f - (float)s;
+        if (s < 0) { s = 0; w = 0.f; }
+        if (s >= src - 1) { s = src - 1; w = 0.f; }
+        i0[d] = s;
+        a[d] = w;
+    }
+}
+
+// cv::getGaussianKernel(ksz, sigma, CV_32F)
+static std::vector<float> gaussian_kernel(int ksz, double sigma) {
+    std::vector<float> k(ksz);
+    if (sigma <= 0 && ksz == 3) { k[0] = 0.25f; k[1] = 0.5f; k[2] = 0.25f; return k; }
+    if (sigma <= 0) sigma = ((ksz - 1) * 0.5 - 1) * 0.3 + 0.8;
+    std::vector<double> t(ksz);
+    double sum = 0;
+    for (int i = 0; i < ksz; ++i) {
+        double x = i - (ksz - 1) * 0.5;
+        t[i] = exp(-0.5 * x * x / (sigma * sigma));
+        sum += t[i];
+    }
+    for (int i = 0; i < ksz; ++i) k[i] = (float)(t[i] / sum);
+    return k;
+}
+
+// FarnebackPrepareGaussian: taps and the four needed entries of inv(G) (Appendix A of SURVEY.md).
+static int poly_setup(int n, double sigma, PolyConst& pc) {
+    if (sigma < 1.1920929e-07) sigma = n * 0.3;
+    float g[2 * kMaxPolyN + 1], xg[2 * kMaxPolyN + 1], xxg[2 * kMaxPolyN + 1];
+    double s = 0;
+    for (int x = -n; x <= n; ++x) {
+        g[x + n] = (float)exp(-x * x / (2 * sigma * sigma));
+        s += g[x + n];
+    }
+    s = 1. / s;
+    for (int x = -n; x <= n; ++x) {
+        g[x + n] = (float)(g[x + n] * s);
+        xg[x + n] = (float)(x * g[x + n]);
+        xxg[x + n] = (float)(x * x * g[x + n]);
+    }
+    double G[6][6];
+    memset(G, 0, sizeof(G));
+    for (int y = -n; y <= n; ++y)
+        for (int x = -n; x <= n; ++x) {
+            const float gg = g[y + n] * g[x + n];
+            G[0][0] += gg;
+            G[1][1] += gg * x * x;
+            G[3][3] += gg * x * x * x * x;
+            G[5][5] += gg * x * x * y * y;
+        }
+    G[2][2] = G[0][3] = G[0][4] = G[3][0] = G[4][0] = G[1][1];
+    G[4][4] = G[3][3];
+    G[3][4] = G[4][3] = G[5][5];
+    // Gauss-Jordan inverse of the 6x6 (symmetric positive definite) matrix
+    double A[6][12];
+    for (int i = 0; i < 6; ++i)
+        for (int j = 0; j < 12; ++j) A[i][j] = j < 6 ? G[i][j] : (j - 6 == i ? 1.0 : 0.0);
+    for (int c = 0; c < 6; ++c) {
+        int piv = c;
+        for (int r = c + 1; r < 6; ++r)
+            if (fabs(A[r][c]) > fabs(A[piv][c])) piv = r;
+        if (fabs(A[piv][c]) < 1e-300) return MAVD_ERR_INVALID;
+        if (piv != c)
+            for (int j = 0; j < 12; ++j) { double t = A[c][j]; A[c][j] = A[piv][j]; A[piv][j] = t; }
+        const double d = A[c][c];
+        for (int j = 0; j < 12; ++j) A[c][j] /= d;
+        for (int r = 0; r < 6; ++r)
+            if (r != c) {
+                const double f = A[r][c];
+                if (f != 0)
+                    for (int j = 0; j < 12; ++j) A[r][j] -= f * A[c][j];
+            }
+    }
+    pc.n = n;
+    for (int k = 0; k <= kMaxPolyN; ++k) {
+        pc.g[k] = k <= n ? g[n + k] : 0.f;
+        pc.xg[k] = k <= n ? xg[n + k] : 0.f;
+        pc.xxg[k] = k <= n ? xxg[n + k] : 0.f;
+    }
+    pc.ig11 = (float)A[1][6 + 1];
+    pc.ig03 = (float)A[0][6 + 3];
+    pc.ig33 = (float)A[3][6 + 3];
+    pc.ig55 = (float)A[5][6 + 5];
+    return MAVD_OK;
+}
+
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
+                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
+                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+
+// TMA descriptor of a rank-3 tensor {d0, d1, d2} (d0 fastest) of 4-byte floats or bytes with byte strides s1, s2 and a
+// box {b0, b1, b2}; out-of-bounds cells are filled with zeros.  Base and strides must be multiples of 16 bytes.
+static bool encode_tensor_map_3d(CUtensorMap* map, bool is_u8, const void* base, uint64_t d0, uint64_t d1, uint64_t d2,
+                                 uint64_t s1_bytes, uint64_t s2_bytes, uint32_t b0, uint32_t b1, uint32_t b2) {
+    static std::atomic<EncodeTiledFn> fn_cache{nullptr};
+    EncodeTiledFn fn = fn_cache.load();
+    if (!fn) {
+        void* f = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &f, cudaEnableDefault, &q) != cudaSuccess || !f) {
+            cudaGetLastError();
+            return false;
+        }
+        fn = (EncodeTiledFn)f;
+        fn_cache.store(fn);
+    }
+    if ((reinterpret_cast<uintptr_t>(base) & 15) || (s1_bytes & 15) || (s2_bytes & 15)) return false;
+    cuuint64_t dims[3] = {d0, d1, d2};
+    cuuint64_t strides[2] = {s1_bytes, s2_bytes};
+    cuuint32_t box[3] = {b0, b1, b2};
+    cuuint32_t estr[3] = {1u, 1u, 1u};
+    CUresult r = fn(map, is_u8 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3,
+                    const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                    CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    return r == CUDA_SUCCESS;
+}
+
+// TMA descriptor of a planar buffer of level L: rank-3 float tensor {pitch, h, planes}, box {box_w, box_h, box_planes},
+// zero fill.
+static bool make_plane_tensor_map(CUtensorMap* map, const Level& L, float* base, int planes, int box_w, int box_h,
+                                  int box_planes) {
+    return encode_tensor_map_3d(map, false, base, (uint64_t)L.pitch, (uint64_t)L.h, (uint64_t)planes,
+                                (uint64_t)L.pitch * sizeof(float), (uint64_t)L.plane * sizeof(float), (uint32_t)box_w,
+                                (uint32_t)box_h, (uint32_t)box_planes);
+}
+
+int farneback_setup(mavd_handle H) {
+    const mavd_farneback_params& fp = H->cfg.farneback;
+    const int W = H->cfg.width, Hh = H->cfg.height, B = H->cfg.max_pairs, F = H->max_frames;
+    Arena& A = H->arena;
+    // level schedule (SURVEY §8 a2): levels = N -> up to N+1 images, 32-pixel cap
+    int k = 0;
+    double sc = 1.0;
+    while (k < fp.levels) {
+        sc *= fp.pyr_scale;
+        if (W * sc < 32 || Hh * sc < 32) break;
+        ++k;
+    }
+    MAVD_REQUIRE(k + 1 <= kMaxLevels, MAVD_ERR_UNSUPPORTED, "too many pyramid levels (%d)", k + 1);
+    H->n_levels = k + 1;
+    const int m = fp.winsize / 2;
+    for (int li = 0; li < H->n_levels; ++li) {
+        Level& L = H->lv[li];
+        L.k = li;
+        double s = 1.0;
+        for (int i = 0; i < li; ++i) s *= fp.pyr_scale;
+        L.scale = s;
+        const double sigma = (1. / s - 1) * 0.5;
+        L.sigma = (float)sigma;
+        L.ksz = std::max(cv_round(sigma * 5) | 1, 3);
+        L.w = cv_round(W * s);
+        L.h = cv_round(Hh * s);
+        L.pitch = round_up(L.w, 64);
+        L.plane = (size_t)L.pitch * L.h;
+        if (li > 0) {
+            // combined blur + bilinear-resize filter per output sample: c_j = (1-a) k_j + a k_{j-1}
+            const std::vector<float> kk = gaussian_kernel(L.ksz, sigma);
+            const int taps = round_up(L.ksz + 1, 4), r = L.ksz / 2;   // zero padded to whole float4 groups
+            for (int axis = 0; axis < 2; ++axis) {
+                const int src = axis == 0 ? W : Hh, dst = axis == 0 ? L.w : L.h;
+                std::vector<int> i0;
+                std::vector<float> a;
+                resize_tables(src, dst, i0, a);
+                std::vector<int> base(dst);
+                std::vector<float> tab((size_t)dst * taps);
+                for (int d = 0; d < dst; ++d) {
+                    base[d] = i0[d] - r;
+                    for (int j = 0; j < taps; ++j) {
+                        const float k0 = j < L.ksz ? kk[j] : 0.f, k1 = (j >= 1 && j <= L.ksz) ? kk[j - 1] : 0.f;
+                        tab[(size_t)d * taps + j] = (1.f - a[d]) * k0 + a[d] * k1;
+                    }
+                }
+                // pyr_scale 0.5 with src = dst * 2^li: the level is an exact decimation (HalfPyr), per axis
+                const int T = li <= HP_MAXLV ? HalfPyr::T(li) : 0;
+                bool half = L.ksz + 1 == T && dst >= 1 && src == dst << li;
+                for (int d = 0; half && d < dst; ++d) {
+                    half = base[d] == (d << li) - HalfPyr::NB(li);
+                    for (int j = 0; half && j < taps; ++j) half = tab[(size_t)d * taps + j] == tab[j];
+                }
+                for (int j = T; half && j < taps; ++j) half = tab[j] == 0.f;
+                (axis == 0 ? L.x_half : L.y_half) = half;
+                if (half) std::copy(tab.begin(), tab.begin() + T, axis == 0 ? L.xwt : L.ywt);
+                if (axis == 0) {
+                    TRY_RC(A.upload(&L.xbase, base)); TRY_RC(A.upload(&L.xtab, tab));
+                    std::vector<float> tabT((size_t)dst * taps);
+                    for (int d = 0; d < dst; ++d)
+                        for (int j = 0; j < taps; ++j) tabT[(size_t)j * dst + d] = tab[(size_t)d * taps + j];
+                    TRY_RC(A.upload(&L.xtabT, tabT));
+                    L.hspan_max = 0;
+                    L.hstride_min = dst > 1 ? src : 0;
+                    for (int d0 = 0; d0 < dst; d0 += 64)
+                        L.hspan_max = std::max(L.hspan_max, base[std::min(d0 + 63, dst - 1)] + taps - base[d0]);
+                    for (int d = 1; d < dst; ++d) L.hstride_min = std::min(L.hstride_min, base[d] - base[d - 1]);
+                }
+                else           { TRY_RC(A.upload(&L.ybase, base)); TRY_RC(A.upload(&L.ytab, tab)); }
+            }
+            TRY_RC(A.alloc(&L.tmp, (size_t)F * L.h * pyr_tmp_pitch(W)));
+        }
+        TRY_RC(A.alloc(&L.img, (size_t)F * L.plane));
+        // polynomial expansion of the float levels: the tile and its poly_n halo rows (polyexp_tma_kernel)
+        L.has_tmap_img = li > 0 && make_plane_tensor_map(&L.tmapImg, L, L.img, F, PE_RW, PE_TY + 2 * fp.poly_n, 1);
+        TRY_RC(A.alloc(&L.R, (size_t)F * 5 * L.plane));
+        TRY_RC(A.alloc(&L.M[0], (size_t)B * 5 * L.plane));
+        TRY_RC(A.alloc(&L.M[1], (size_t)B * 5 * L.plane));
+        if (li > 0) TRY_RC(A.alloc(&L.flow, (size_t)B * 2 * L.plane));
+        // padded columns of R/M are read by vector loads of edge tiles: keep them finite
+        cudaMemset(L.img, 0, (size_t)F * L.plane * sizeof(float));
+        cudaMemset(L.R, 0, (size_t)F * 5 * L.plane * sizeof(float));
+        cudaMemset(L.M[0], 0, (size_t)B * 5 * L.plane * sizeof(float));
+        cudaMemset(L.M[1], 0, (size_t)B * 5 * L.plane * sizeof(float));
+        // iter_box_tma_kernel's boxes: the five planes of a tile and its m halo rows, and the R prefetch
+        if (m >= 5 && m <= 8)
+            L.has_tmap = make_plane_tensor_map(&L.tmapM[0], L, L.M[0], B * 5, IT_RW, IT_TY + 2 * m, 5) &&
+                         make_plane_tensor_map(&L.tmapM[1], L, L.M[1], B * 5, IT_RW, IT_TY + 2 * m, 5) &&
+                         make_plane_tensor_map(&L.tmapR, L, L.R, F * 5, IT_RW, IT_PF_ROWS, IT_PF_PLANES) &&
+                         make_plane_tensor_map(&L.tmapRbox, L, L.R, F * 5, IT_RW, IT_TY + 2 * m, 5);
+        if (L.has_tmap)
+            L.has_tmap16 = make_plane_tensor_map(&L.tmapM16[0], L, L.M[0], B * 5, IT_RW, IT_TY_SMALL + 2 * m, 5) &&
+                           make_plane_tensor_map(&L.tmapM16[1], L, L.M[1], B * 5, IT_RW, IT_TY_SMALL + 2 * m, 5) &&
+                           make_plane_tensor_map(&L.tmapRbox16, L, L.R, F * 5, IT_RW, IT_TY_SMALL + 2 * m, 5);
+    }
+    // flow upsample tables (next-coarser level -> this level)
+    for (int li = 0; li + 1 < H->n_levels; ++li) {
+        Level& L = H->lv[li];
+        const Level& C = H->lv[li + 1];
+        std::vector<int> i0;
+        std::vector<float> a;
+        resize_tables(C.w, L.w, i0, a);
+        TRY_RC(A.upload(&L.fxi0, i0));
+        TRY_RC(A.upload(&L.fxa, a));
+        resize_tables(C.h, L.h, i0, a);
+        TRY_RC(A.upload(&L.fyi0, i0));
+        TRY_RC(A.upload(&L.fya, a));
+    }
+    TRY_RC(poly_setup(fp.poly_n, fp.poly_sigma, H->poly));
+    // FarnebackUpdateFlow_GaussianBlur half kernel
+    const double sigma = m * 0.3;
+    std::vector<float> kf(m + 1);
+    double s = 0;
+    for (int i = 0; i <= m; ++i) {
+        kf[i] = (float)exp(-i * i / (2 * sigma * sigma));
+        s += (i == 0 ? 1.0 : 2.0) * kf[i];
+    }
+    for (int i = 0; i <= m; ++i) kf[i] = (float)(kf[i] * (1.0 / s));
+    return A.upload(&H->gauss_win, kf);
 }
 
 int farneback_run(mavd_handle H, const uint8_t* d_frames, int n_pairs, int pair_stride, float* d_flow,
@@ -1608,7 +1878,6 @@ int farneback_run(mavd_handle H, const uint8_t* d_frames, int n_pairs, int pair_
     const int hx = round_up(m, 4);
     const size_t frame_bytes = (size_t)W * Hh;
 
-    // pyramid images of every coarser level for all frames: two launches
     // pyramid images of levels lo..hi (1 <= lo <= hi) for all frames: two launches
     // programmatic dependent launch: lane 0 = the caller's stream, lane 1 = the side stream (common.cuh: pdl_next)
     auto lane = [&](cudaStream_t st) { return (st == H->s_aux && st != s) ? 1 : 0; };
@@ -1617,7 +1886,7 @@ int farneback_run(mavd_handle H, const uint8_t* d_frames, int n_pairs, int pair_
     auto build_pyramid = [&](cudaStream_t st, int lo, int hi) -> int {
         if (H->n_levels <= 1 || lo > hi) return MAVD_OK;
         ProfScope ps(&H->prof, MAVD_PROF_PYRAMID, st);
-        const int Wp = round_up(W, 4);
+        const int Wp = pyr_tmp_pitch(W);
         const bool pyr_staged_env = H->tune.pyr_staged != 0;
         const int word_ok = ((W & 3) == 0 && (reinterpret_cast<uintptr_t>(d_frames) & 3) == 0) ? 1 : 0;
         // descriptor of levels a..b for the generic kernels
@@ -1831,7 +2100,7 @@ int farneback_run(mavd_handle H, const uint8_t* d_frames, int n_pairs, int pair_
             // tiles: twice the CTAs, half the serial work per CTA (tuning.iter_small_tiles)
             const bool small_tiles =
                 H->tune.iter_small_tiles != 0 && L.has_tmap16 && (long long)g.x * g.y * g.z <= 3LL * 148;
-            const dim3 g1(small_tiles ? g.x * ceil_div(L.h, 16) * g.z : g.x * g.y * g.z);
+            const dim3 g1(small_tiles ? g.x * ceil_div(L.h, IT_TY_SMALL) * g.z : g.x * g.y * g.z);
             const int RW = IT_TX + 2 * hx, RH = IT_TY + 2 * m;
             const size_t smem = sizeof(float) * ((size_t)RH * RW + (size_t)IT_TY * RW + 5 * IT_TX * IT_TY);
             ProfScope ps(&H->prof, li > 0 ? MAVD_PROF_ITER_COARSE : (last ? MAVD_PROF_ITER_FULL_LAST : MAVD_PROF_ITER_FULL), st);
@@ -1885,10 +2154,6 @@ int farneback_run(mavd_handle H, const uint8_t* d_frames, int n_pairs, int pair_
             TRY_RC(solve_level(li, s));
         }
     }
-    H->last_pairs = n_pairs;
-    H->last_stride = pair_stride;
-    H->last_flow0 = d_flow;
-    H->last_frames = d_frames;
     return MAVD_OK;
 }
 

@@ -482,21 +482,57 @@ __global__ void __launch_bounds__(kLkWarps * 32) lk_track_kernel(
 
 }  // namespace
 
-// workspace sizes of the sparse path (allocated on first use by api.cu)
+// workspace sizes of the corner path
 size_t gftt_key_cap(int W, int H) {
     size_t n = (size_t)max(W - 2, 1) * (size_t)max(H - 2, 1), c = 2;
     while (c < n) c <<= 1;
     return c;
 }
 size_t gftt_grid_cap(int W, int H) { return (size_t)((W + 1) / 2) * ((H + 1) / 2) * 4; }
-int gftt_chunk() { return kGfttChunk; }
 
-int gftt_run(mavd_handle h, const GfttWork& ws, const uint8_t* d_frames, int n, const mavd_gftt_params& p,
-             const uint8_t* d_mask, int64_t mask_stride, float* d_corners, int32_t* d_count, float* d_eig,
-             cudaStream_t s) {
+struct GfttWork {
+    double* rows;                   // [chunk][H][W][3] row sums of the block
+    unsigned long long* keys;       // [chunk][gftt_key_cap] candidates
+    float3* cov;                    // [chunk][H][W] products of the Sobel derivatives
+    float* eig;                     // [chunk][H][W] when the caller wants no eig image
+    int* grid;                      // [chunk][gftt_grid_cap] accepted corners by cell
+    uint32_t* maxv;                 // [chunk]
+    int* n_cand;                    // [chunk]
+};
+
+template <typename T>
+static void carve(char* base, size_t& off, T*& p, size_t count) {
+    p = base ? reinterpret_cast<T*>(base + off) : nullptr;
+    off += sizeof(T) * count;
+}
+
+// The corner workspace of kGfttChunk frames, carved from one allocation at base.  Returns its size, which is all it
+// computes when base is NULL.
+static size_t gftt_layout(int W, int H, char* base, GfttWork& w) {
+    const size_t npx = (size_t)W * H, G = kGfttChunk;
+    size_t off = 0;
+    carve(base, off, w.rows, 3 * npx * G);
+    carve(base, off, w.keys, gftt_key_cap(W, H) * G);
+    carve(base, off, w.cov, npx * G);
+    carve(base, off, w.eig, npx * G);
+    carve(base, off, w.grid, gftt_grid_cap(W, H) * G);
+    carve(base, off, w.maxv, G);
+    carve(base, off, w.n_cand, G);
+    return off;
+}
+
+int gftt_run(mavd_handle h, const uint8_t* d_frames, int n, const mavd_gftt_params& p, const uint8_t* d_mask,
+             int64_t mask_stride, float* d_corners, int32_t* d_count, float* d_eig, cudaStream_t s) {
     const int W = h->cfg.width, H = h->cfg.height;
     const size_t npx = (size_t)W * H;
     const size_t kcap = gftt_key_cap(W, H), gcap = gftt_grid_cap(W, H);
+    GfttWork ws;
+    if (!h->sp_gftt) {
+        char* base = nullptr;
+        TRY_RC(h->arena.alloc(&base, gftt_layout(W, H, nullptr, ws)));
+        h->sp_gftt = base;
+    }
+    gftt_layout(W, H, (char*)h->sp_gftt, ws);
     const bool grid = p.min_distance > 1.0;
     for (int f0 = 0; f0 < n; f0 += kGfttChunk) {
         const int g = min(kGfttChunk, n - f0);
@@ -554,14 +590,19 @@ static LkGeom lk_geom(int W, int H, int levels) {
     g.der_frame = doff;
     return g;
 }
-size_t lk_pyr_frame_bytes(int W, int H) { return lk_geom(W, H, 1).pyr_frame; }
-size_t lk_der_frame_elems(int W, int H) { return lk_geom(W, H, 1).der_frame; }
 
-int lk_run(mavd_handle h, uint8_t* pyr, short2* der, const uint8_t* d_frames, int n_pairs, int pair_stride,
-           const mavd_lk_params& p, const float* d_prev, int n_points, const int32_t* d_n_points, float* d_next,
-           uint8_t* d_status, float* d_err, cudaStream_t s) {
+int lk_run(mavd_handle h, const uint8_t* d_frames, int n_pairs, int pair_stride, const mavd_lk_params& p,
+           const float* d_prev, int n_points, const int32_t* d_n_points, float* d_next, uint8_t* d_status, float* d_err,
+           cudaStream_t s) {
     const int W = h->cfg.width, H = h->cfg.height;
     const LkGeom g = lk_geom(W, H, lk_levels(W, H, p.win_w, p.win_h, p.max_level));
+    if (!h->sp_der) {
+        // max_frames frames of every level up to MAVD_LK_MAX_LEVEL: g's frame sizes do not depend on the call's levels
+        TRY_RC(h->arena.alloc(&h->sp_pyr, (size_t)h->max_frames * g.pyr_frame));
+        TRY_RC(h->arena.alloc(&h->sp_der, (size_t)h->max_frames * g.der_frame));
+    }
+    uint8_t* pyr = h->sp_pyr;
+    short2* der = h->sp_der;
     const int n_frames = (n_pairs - 1) * pair_stride + 2;
     for (int l = 1; l < g.levels; ++l) {
         lk_pyr_down_kernel<<<dim3(ceil_div(g.w[l], 128), g.h[l], n_frames), 128, 0, s>>>(d_frames, pyr, g, l);

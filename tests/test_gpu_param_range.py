@@ -74,7 +74,7 @@ def _check_against_oracle_and_cv2(prev, nxt, p, flow, levels):
 
 
 def _staged_stride(src, dst):
-    """Smallest distance between the first source samples of adjacent outputs of a resize src -> dst (api.cu:
+    """Smallest distance between the first source samples of adjacent outputs of a resize src -> dst (farneback.cu:
     hstride_min); the staged horizontal pyramid pass runs on levels where it is >= 8."""
     from oracle import farneback_np as fb
     i0 = fb._resize_axis_coeffs(src, dst)[0]

@@ -3,7 +3,8 @@ pyr_hpass_kernel, pyr_hpass1_kernel), restated with Python loops and checked aga
 
 1. The constants the kernels are specialised on (stride S = 2^l, taps T, window start S * d - NB) are what the
    collapsed blur + resize filter of a pyr_scale 0.5 level IS, derived from oracle/farneback_np's resize coefficients
-   and blur parameters (api.cu makes the same check on its tables at mavd_create and falls back per level and axis).
+   and blur parameters (farneback.cu: farneback_setup makes the same check on its tables at mavd_create and falls
+   back per level and axis).
 2. The polyphase schedule of the sweep — which (output row, tap) a source row feeds in which of the <= 3 live
    accumulators, when an output is finished, which band stores it — gives every output row of every level exactly
    its T taps, in ascending order, from the REFLECT_101 rows, once.
