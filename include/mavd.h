@@ -225,7 +225,8 @@ int mavd_bgr2gray(const uint8_t* d_bgr, uint8_t* d_gray, int64_t n_pixels, void*
 int mavd_farneback(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int32_t pair_stride,
                    float* d_flow, void* stream);
 
-/* Test tap: copy an internal buffer of the LAST mavd_farneback call out as a dense array.
+/* Test tap: copy an internal buffer of the LAST mavd_farneback call out as a dense array (not after a frame-stream
+ * call, see mavd_stream_start).
  * kind 0: pyramid image (h_l, w_l); 1: polynomial expansion R (h_l, w_l, 5), index = frame;
  * 2: matrices M after the last update (h_l, w_l, 5), index = pair; 3: level flow (h_l, w_l, 2). */
 int mavd_farneback_tap(mavd_handle h, int32_t kind, int32_t level, int32_t index, float* d_out,
@@ -367,6 +368,35 @@ int mavd_submit_host(mavd_handle h, int32_t slot, const uint8_t* h_frames, int32
                      const mavd_aux_inputs* h_aux, int32_t flags, float* h_flow_out, uint8_t* h_fixed_out,
                      mavd_frame_record* h_records, int32_t max_det, mavd_detection* h_det, void* stream);
 int mavd_wait_host(mavd_handle h, int32_t slot);
+
+/* ---- frame streams: Farneback.process() (src/farneback.py:72-81) for up to max_pairs cameras at once ----
+ * A handle has max_pairs streams, ids 0 .. max_pairs-1.  A stream keeps the pyramid's polynomial expansions of its last
+ * frame on the device, so every new frame of a camera makes a pair with the previous one and is expanded once.
+ *  - mavd_stream_start stores the first frame of each named stream (no flow); starting a stream again restarts it.
+ *  - a step (mavd_stream_farneback / _process / _submit_host) takes one new frame per id: pair i is (stream h_ids[i]'s
+ *    kept frame, frame i), and frame i becomes that stream's kept frame.  Its flow, records, masks and detection
+ *    tables are bit-identical to the pair_stride 2 call on the explicit (previous, new) frames.
+ *  - h_ids: n distinct ids in any order (any subset of the streams); copied before the call returns.  Duplicate or
+ *    out-of-range ids, n > max_pairs, a NULL h_ids (whatever n), NULL buffers and a step naming a stream that is not
+ *    started return MAVD_ERR_INVALID; a rejected call changes no stream.
+ *  - stream state advances when a call is submitted, in submit order (the handle's one-stream rule above).
+ *  - the streams' expansions live in the workspace of the ordinary calls: ANY non-stream Farneback call on the handle
+ *    (mavd_farneback, mavd_process, mavd_submit_host without MAVD_HOST_COPY_ONLY) ends every stream, which must then
+ *    be started again.  mavd_set_tuning keeps them.
+ *  - after a stream call mavd_farneback_tap returns MAVD_ERR_INVALID until the next non-stream Farneback call.
+ * d_frames / h_frames hold the n new frames, dense; the remaining arguments are those of mavd_farneback, mavd_process
+ * and mavd_submit_host (flags included; mavd_wait_host completes a stream submit). */
+int mavd_stream_start(mavd_handle h, const uint8_t* d_frames, int32_t n, const int32_t* h_ids, void* stream);
+int mavd_stream_farneback(mavd_handle h, const uint8_t* d_frames, int32_t n, const int32_t* h_ids, float* d_flow,
+                          void* stream);
+int mavd_stream_process(mavd_handle h, const uint8_t* d_frames, int32_t n, const int32_t* h_ids, const mavd_imu* h_imu,
+                        const mavd_detect_params* prm, const int32_t* d_samples, const mavd_aux_inputs* d_aux,
+                        float* d_flow_out, uint8_t* d_total_out, uint8_t* d_fixed_out, mavd_frame_record* d_records,
+                        int32_t max_det, mavd_detection* d_det, void* stream);
+int mavd_stream_submit_host(mavd_handle h, int32_t slot, const uint8_t* h_frames, int32_t n, const int32_t* h_ids,
+                            const mavd_imu* h_imu, const mavd_detect_params* prm, const int32_t* h_samples,
+                            const mavd_aux_inputs* h_aux, int32_t flags, float* h_flow_out, uint8_t* h_fixed_out,
+                            mavd_frame_record* h_records, int32_t max_det, mavd_detection* h_det, void* stream);
 
 /* Detection from a HOST flow field (n x H x W x 2 float32), the Dataset.get_flow_uv seam end to end.  Waits for
  * slot 0, uses its staging buffers on `stream` alone, and returns after the results have landed (it synchronises).

@@ -131,6 +131,12 @@ SIGNATURES = {
     'mavd_submit_host': (C.c_int, [_P, C.c_int32, _P, C.c_int32, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams),
                                    _P, C.POINTER(AuxInputs), C.c_int32, _P, _P, _P, C.c_int32, _P, _P]),
     'mavd_wait_host': (C.c_int, [_P, C.c_int32]),
+    'mavd_stream_start': (C.c_int, [_P, _P, C.c_int32, _P, _P]),
+    'mavd_stream_farneback': (C.c_int, [_P, _P, C.c_int32, _P, _P, _P]),
+    'mavd_stream_process': (C.c_int, [_P, _P, C.c_int32, _P, C.POINTER(Imu), C.POINTER(DetectParams), _P,
+                                      C.POINTER(AuxInputs), _P, _P, _P, _P, C.c_int32, _P, _P]),
+    'mavd_stream_submit_host': (C.c_int, [_P, C.c_int32, _P, C.c_int32, _P, C.POINTER(Imu), C.POINTER(DetectParams),
+                                          _P, C.POINTER(AuxInputs), C.c_int32, _P, _P, _P, C.c_int32, _P, _P]),
     'mavd_detect_host': (C.c_int, [_P, _P, C.c_int32, C.POINTER(Imu), C.POINTER(DetectParams), _P,
                                    C.POINTER(AuxInputs), C.c_int32, _P, _P, C.c_int32, _P, _P]),
     'mavd_good_features_to_track': (C.c_int, [_P, _P, C.c_int32, C.POINTER(GfttParams), _P, C.c_int64, _P, _P, _P,

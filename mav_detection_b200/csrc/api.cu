@@ -67,6 +67,9 @@ static void release(mavd_handle H) {
     for (cudaEvent_t e : H->imu_ev)
         if (e) cudaEventDestroy(e);
     if (H->h_imu_ring) cudaFreeHost(H->h_imu_ring);
+    for (cudaEvent_t e : H->stream_ev)
+        if (e) cudaEventDestroy(e);
+    if (H->h_stream_ring) cudaFreeHost(H->h_stream_ring);
     for (auto& r : H->prof.recs) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
     for (cudaEvent_t e : H->prof.pool) cudaEventDestroy(e);
     delete H;
@@ -128,6 +131,8 @@ int mavd_create(const mavd_config* cfg, mavd_handle* out) {
     H->cfg = *cfg;
     mavd_default_tuning(&H->tune);
     H->max_frames = 2 * cfg->max_pairs;  // worst case: independent pairs
+    H->stream_live.assign(cfg->max_pairs, 0);
+    H->stream_parity.assign(cfg->max_pairs, 0);
     int rc = MAVD_OK;
 #define C_TRY(x) do { rc = (x); if (rc != MAVD_OK) { release(H); return rc; } } while (0)
     C_TRY(farneback_setup(H));
@@ -300,19 +305,74 @@ static int check_batch(mavd_handle h, int n, const char* what) {
     return MAVD_OK;
 }
 
-// taps read "the last mavd_farneback call": recorded here, outside the (possibly replayed) launch sequence
+// taps read "the last mavd_farneback call": recorded here, outside the (possibly replayed) launch sequence.  A
+// non-stream call expands its frames into the R slots the streams keep theirs in: it ends every stream.
 static void note_farneback_call(mavd_handle h, const uint8_t* d_frames, int n_pairs, int pair_stride, float* d_flow) {
     h->last_pairs = n_pairs;
     h->last_stride = pair_stride;
     h->last_flow0 = d_flow;
     h->last_frames = d_frames;
+    h->last_was_stream = false;
+    std::fill(h->stream_live.begin(), h->stream_live.end(), 0);
 }
 
 int mavd_farneback_tap(mavd_handle h, int32_t kind, int32_t level, int32_t index, float* d_out, void* stream) {
     MAVD_REQUIRE(h && d_out, MAVD_ERR_INVALID, "tap: NULL argument");
     DeviceGuard dg(h->cfg.device);
+    MAVD_REQUIRE(!h->last_was_stream, MAVD_ERR_INVALID, "tap: the last Farneback call was a frame-stream call");
     MAVD_REQUIRE(index >= 0 && index < h->max_frames, MAVD_ERR_INVALID, "tap: index out of range");
     return farneback_tap(h, kind, level, index, d_out, (cudaStream_t)stream);
+}
+
+// ids of a frame-stream call: n distinct streams in 0..max_pairs-1; a step (not a start) also needs every one of them
+// started and not ended since.  Checked before anything is staged or launched: a rejected call changes no stream.
+static int check_stream_ids(mavd_handle h, const int32_t* h_ids, int n, bool step, const char* what) {
+    MAVD_REQUIRE(h_ids != nullptr, MAVD_ERR_INVALID, "%s: ids array is NULL", what);
+    std::vector<uint8_t> seen(h->cfg.max_pairs, 0);
+    for (int i = 0; i < n; ++i) {
+        const int32_t id = h_ids[i];
+        MAVD_REQUIRE(id >= 0 && id < h->cfg.max_pairs, MAVD_ERR_INVALID, "%s: ids[%d] = %d outside 0..%d", what, i, id,
+                     h->cfg.max_pairs - 1);
+        MAVD_REQUIRE(!seen[id], MAVD_ERR_INVALID, "%s: stream %d appears twice", what, id);
+        seen[id] = 1;
+        MAVD_REQUIRE(!step || h->stream_live[id], MAVD_ERR_INVALID,
+                     "%s: stream %d is not started (never, or ended by a non-stream Farneback call since)", what, id);
+    }
+    return MAVD_OK;
+}
+
+// The R slot tables of a checked stream call (FrameSlots), staged like the imu: a pinned ring slot, then an
+// asynchronous copy into the fixed device tables that the (possibly replayed) launch sequence reads.  Frame i goes to
+// the slot of its stream that does not hold the kept frame; pair i reads (kept, new).
+static int upload_stream_slots(mavd_handle h, const int32_t* h_ids, int n, cudaStream_t s) {
+    const int B = h->cfg.max_pairs;
+    if (!h->d_stream_slots) TRY(h->arena.alloc(&h->d_stream_slots, (size_t)3 * B));
+    for (cudaEvent_t& e : h->stream_ev)
+        if (!e) MAVD_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    if (!h->h_stream_ring)
+        MAVD_CUDA(cudaMallocHost((void**)&h->h_stream_ring, sizeof(int32_t) * 3 * B * mavd_handle_s::kImuRing));
+    const int k = h->stream_next;
+    h->stream_next = (k + 1) % mavd_handle_s::kImuRing;
+    MAVD_CUDA(cudaEventSynchronize(h->stream_ev[k]));
+    int32_t* stage = h->h_stream_ring + (size_t)k * 3 * B;
+    for (int i = 0; i < n; ++i) {
+        const int kept = 2 * h_ids[i] + h->stream_parity[h_ids[i]];
+        stage[i] = kept ^ 1;
+        stage[B + 2 * i] = kept;
+        stage[B + 2 * i + 1] = kept ^ 1;
+    }
+    MAVD_CUDA(cudaMemcpyAsync(h->d_stream_slots, stage, sizeof(int32_t) * 3 * B, cudaMemcpyHostToDevice, s));
+    MAVD_CUDA(cudaEventRecord(h->stream_ev[k], s));
+    return MAVD_OK;
+}
+
+// a stream call was enqueued: each named stream now keeps the frame it was given
+static void advance_streams(mavd_handle h, const int32_t* h_ids, int n) {
+    for (int i = 0; i < n; ++i) {
+        h->stream_parity[h_ids[i]] ^= 1;
+        h->stream_live[h_ids[i]] = 1;
+    }
+    h->last_was_stream = true;
 }
 
 static int upload_imu(mavd_handle h, const mavd_imu* h_imu, int n, cudaStream_t s, int* n64, int* n32) {
@@ -763,17 +823,20 @@ int mavd_detect(mavd_handle h, const float* d_flow, int32_t n, const mavd_imu* h
                        });
 }
 
-int mavd_process(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int32_t pair_stride, const mavd_imu* h_imu,
-                 const mavd_detect_params* prm, const int32_t* d_samples, const mavd_aux_inputs* d_aux,
-                 float* d_flow_out, uint8_t* d_total_out, uint8_t* d_fixed_out, mavd_frame_record* d_records,
-                 int32_t max_det, mavd_detection* d_det, void* stream) {
-    DeviceGuard dg(h ? h->cfg.device : -1);
-    TRY(check_batch(h, n_pairs, "process"));
-    MAVD_REQUIRE(pair_stride == 1 || pair_stride == 2, MAVD_ERR_INVALID, "pair_stride must be 1 or 2");
-    TRY(check_det(h, max_det, d_det, "process"));
+// mavd_process (step false: pairs by pair_stride) and mavd_stream_process (step true: one new frame per id of h_ids)
+static int process_run(mavd_handle h, const uint8_t* d_frames, int n_pairs, int pair_stride, bool step,
+                       const int32_t* h_ids, const mavd_imu* h_imu, const mavd_detect_params* prm, const int32_t* d_samples,
+                       const mavd_aux_inputs* d_aux, float* d_flow_out, uint8_t* d_total_out, uint8_t* d_fixed_out,
+                       mavd_frame_record* d_records, int max_det, mavd_detection* d_det, void* stream) {
+    const char* what = step ? "stream_process" : "process";
+    MAVD_REQUIRE(!step || h_ids, MAVD_ERR_INVALID, "%s: ids array is NULL", what);
+    TRY(check_batch(h, n_pairs, what));
+    MAVD_REQUIRE(step || pair_stride == 1 || pair_stride == 2, MAVD_ERR_INVALID, "pair_stride must be 1 or 2");
+    TRY(check_det(h, max_det, d_det, what));
     if (!d_det) max_det = 0;
     if (n_pairs == 0) return MAVD_OK;
-    MAVD_REQUIRE(d_frames && d_samples && d_records, MAVD_ERR_INVALID, "process: NULL buffer");
+    MAVD_REQUIRE(d_frames && d_samples && d_records, MAVD_ERR_INVALID, "%s: NULL buffer", what);
+    if (step) TRY(check_stream_ids(h, h_ids, n_pairs, true, what));
     StreamScope ss(h, stream);
     mavd_detect_params p;
     if (prm) p = *prm; else mavd_default_detect_params(&p);
@@ -782,15 +845,67 @@ int mavd_process(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int32_
     uint8_t* fixed = d_fixed_out ? d_fixed_out : h->d_fixed;
     int n64 = 0, n32 = 0;
     TRY(upload_imu(h, h_imu, n_pairs, ss.s, &n64, &n32));
-    note_farneback_call(h, d_frames, n_pairs, pair_stride, flow);
-    return run_graphed(h, std::move(KeyBuilder()(int64_t(3))(d_frames)(int64_t(n_pairs))(int64_t(pair_stride))(p)(int64_t(n64))(int64_t(h->batch_rot > 0))
+    if (step) TRY(upload_stream_slots(h, h_ids, n_pairs, ss.s));
+    else note_farneback_call(h, d_frames, n_pairs, pair_stride, flow);
+    const FrameSlots fs = h->stream_slots(n_pairs);
+    TRY(run_graphed(h, std::move(KeyBuilder()(int64_t(step ? 5 : 3))(d_frames)(int64_t(n_pairs))(int64_t(pair_stride))(p)(int64_t(n64))(int64_t(h->batch_rot > 0))
                                         (int64_t(n32))(d_samples)(aux)(flow)(d_total_out)(fixed)(d_records)(int64_t(max_det))
                                         (d_det).k),
-                       ss.s, [&](cudaStream_t s) {
-                           TRY(farneback_run(h, d_frames, n_pairs, pair_stride, flow, s));
-                           return detect_run(h, flow, n_pairs, p, n64, n32, d_samples, aux, d_total_out, fixed, d_records,
-                                             max_det, d_det, s);
-                       });
+                    ss.s, [&](cudaStream_t s) {
+                        TRY(farneback_run(h, d_frames, n_pairs, pair_stride, flow, s, step ? &fs : nullptr));
+                        return detect_run(h, flow, n_pairs, p, n64, n32, d_samples, aux, d_total_out, fixed, d_records,
+                                          max_det, d_det, s);
+                    }));
+    if (step) advance_streams(h, h_ids, n_pairs);
+    return MAVD_OK;
+}
+
+int mavd_process(mavd_handle h, const uint8_t* d_frames, int32_t n_pairs, int32_t pair_stride, const mavd_imu* h_imu,
+                 const mavd_detect_params* prm, const int32_t* d_samples, const mavd_aux_inputs* d_aux,
+                 float* d_flow_out, uint8_t* d_total_out, uint8_t* d_fixed_out, mavd_frame_record* d_records,
+                 int32_t max_det, mavd_detection* d_det, void* stream) {
+    DeviceGuard dg(h ? h->cfg.device : -1);
+    return process_run(h, d_frames, n_pairs, pair_stride, false, nullptr, h_imu, prm, d_samples, d_aux, d_flow_out, d_total_out,
+                       d_fixed_out, d_records, max_det, d_det, stream);
+}
+
+int mavd_stream_process(mavd_handle h, const uint8_t* d_frames, int32_t n, const int32_t* h_ids, const mavd_imu* h_imu,
+                        const mavd_detect_params* prm, const int32_t* d_samples, const mavd_aux_inputs* d_aux,
+                        float* d_flow_out, uint8_t* d_total_out, uint8_t* d_fixed_out, mavd_frame_record* d_records,
+                        int32_t max_det, mavd_detection* d_det, void* stream) {
+    DeviceGuard dg(h ? h->cfg.device : -1);
+    return process_run(h, d_frames, n, 2, true, h_ids, h_imu, prm, d_samples, d_aux, d_flow_out, d_total_out, d_fixed_out,
+                       d_records, max_det, d_det, stream);
+}
+
+// mavd_stream_farneback (step) and mavd_stream_start (expansions only)
+static int stream_farneback_run(mavd_handle h, bool step, const uint8_t* d_frames, int n, const int32_t* h_ids,
+                                float* d_flow, void* stream) {
+    const char* what = step ? "stream_farneback" : "stream_start";
+    MAVD_REQUIRE(h_ids != nullptr, MAVD_ERR_INVALID, "%s: ids array is NULL", what);
+    TRY(check_batch(h, n, what));
+    if (n == 0) return MAVD_OK;
+    MAVD_REQUIRE(d_frames && (d_flow || !step), MAVD_ERR_INVALID, "%s: NULL buffer", what);
+    TRY(check_stream_ids(h, h_ids, n, step, what));
+    StreamScope ss(h, stream);
+    TRY(upload_stream_slots(h, h_ids, n, ss.s));
+    const FrameSlots fs = h->stream_slots(n);
+    const int n_pairs = step ? n : 0;
+    TRY(run_graphed(h, std::move(KeyBuilder()(int64_t(step ? 4 : 6))(d_frames)(int64_t(n))(d_flow).k), ss.s,
+                    [&](cudaStream_t s) { return farneback_run(h, d_frames, n_pairs, 2, d_flow, s, &fs); }));
+    advance_streams(h, h_ids, n);
+    return MAVD_OK;
+}
+
+int mavd_stream_start(mavd_handle h, const uint8_t* d_frames, int32_t n, const int32_t* h_ids, void* stream) {
+    DeviceGuard dg(h ? h->cfg.device : -1);
+    return stream_farneback_run(h, false, d_frames, n, h_ids, nullptr, stream);
+}
+
+int mavd_stream_farneback(mavd_handle h, const uint8_t* d_frames, int32_t n, const int32_t* h_ids, float* d_flow,
+                          void* stream) {
+    DeviceGuard dg(h ? h->cfg.device : -1);
+    return stream_farneback_run(h, true, d_frames, n, h_ids, d_flow, stream);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -908,24 +1023,28 @@ static int copy_out(mavd_handle h, mavd_handle_s::HostSlot& S, int n, int flags,
     return MAVD_OK;
 }
 
-int mavd_submit_host(mavd_handle h, int32_t slot, const uint8_t* h_frames, int32_t n_pairs, int32_t pair_stride,
-                     const mavd_imu* h_imu, const mavd_detect_params* prm, const int32_t* h_samples,
-                     const mavd_aux_inputs* h_aux, int32_t flags, float* h_flow_out, uint8_t* h_fixed_out,
-                     mavd_frame_record* h_records, int32_t max_det, mavd_detection* h_det, void* stream) {
-    DeviceGuard dg(h ? h->cfg.device : -1);
-    TRY(check_batch(h, n_pairs, "submit_host"));
+// mavd_submit_host (step false: pairs by pair_stride) and mavd_stream_submit_host (step true: one new frame per id)
+static int submit_host_run(mavd_handle h, int slot, const uint8_t* h_frames, int n_pairs, int pair_stride, bool step,
+                           const int32_t* h_ids, const mavd_imu* h_imu, const mavd_detect_params* prm,
+                           const int32_t* h_samples, const mavd_aux_inputs* h_aux, int flags, float* h_flow_out,
+                           uint8_t* h_fixed_out, mavd_frame_record* h_records, int max_det, mavd_detection* h_det,
+                           void* stream) {
+    const char* what = step ? "stream_submit_host" : "submit_host";
+    MAVD_REQUIRE(!step || h_ids, MAVD_ERR_INVALID, "%s: ids array is NULL", what);
+    TRY(check_batch(h, n_pairs, what));
     MAVD_REQUIRE(slot >= 0 && slot < MAVD_HOST_SLOTS, MAVD_ERR_INVALID, "slot %d out of range", slot);
-    MAVD_REQUIRE(pair_stride == 1 || pair_stride == 2, MAVD_ERR_INVALID, "pair_stride must be 1 or 2");
-    MAVD_REQUIRE(n_pairs >= 1, MAVD_ERR_INVALID, "submit_host: empty batch");
+    MAVD_REQUIRE(step || pair_stride == 1 || pair_stride == 2, MAVD_ERR_INVALID, "pair_stride must be 1 or 2");
+    MAVD_REQUIRE(n_pairs >= 1, MAVD_ERR_INVALID, "%s: empty batch", what);
     const mavd_aux_inputs ha = h_aux ? *h_aux : kNoAux;
-    TRY(check_host_args(h, "submit_host", n_pairs, h_frames, h_samples, h_records, ha, flags, max_det, h_det));
+    TRY(check_host_args(h, what, n_pairs, h_frames, h_samples, h_records, ha, flags, max_det, h_det));
+    if (step) TRY(check_stream_ids(h, h_ids, n_pairs, !(flags & MAVD_HOST_COPY_ONLY), what));
     const size_t npx = (size_t)h->cfg.width * h->cfg.height;
     const bool bgr = (flags & MAVD_HOST_BGR) != 0;
     TRY(ensure_slot(h, slot, h_flow_out != nullptr, false, (flags & (MAVD_HOST_SEG_PACKED | MAVD_HOST_SKY_PACKED)) != 0,
                     (flags & MAVD_HOST_FIXED_PACKED) && h_fixed_out, ha.gt_flow != nullptr, h_det != nullptr));
     mavd_handle_s::HostSlot& S = h->slot[slot];
     MAVD_REQUIRE(!S.busy, MAVD_ERR_INVALID, "slot %d is still in flight: call mavd_wait_host first", slot);
-    const int n_frames = pair_stride == 1 ? n_pairs + 1 : 2 * n_pairs;
+    const int n_frames = step ? n_pairs : pair_stride == 1 ? n_pairs + 1 : 2 * n_pairs;
     if (bgr && !S.d_bgr) TRY(h->arena.alloc(&S.d_bgr, (size_t)h->max_frames * npx * 3));
     StreamScope ss(h, stream);
     cudaStream_t s = ss.s;
@@ -945,9 +1064,9 @@ int mavd_submit_host(mavd_handle h, int32_t slot, const uint8_t* h_frames, int32
     // the next batch's Farneback, was measured: no gain, the GPU is already full and the work is only re-ordered.)
     MAVD_CUDA(cudaStreamWaitEvent(s, S.ev_in, 0));
     if (!(flags & MAVD_HOST_COPY_ONLY))
-        TRY(mavd_process(h, S.d_frames, n_pairs, pair_stride, h_imu, prm, S.d_samples, &da,
-                         h_flow_out ? S.d_flow : nullptr, nullptr, S.d_fixed, S.d_records, max_det,
-                         h_det ? S.d_det : nullptr, s));
+        TRY(process_run(h, S.d_frames, n_pairs, pair_stride, step, h_ids, h_imu, prm, S.d_samples, &da,
+                        h_flow_out ? S.d_flow : nullptr, nullptr, S.d_fixed, S.d_records, max_det,
+                        h_det ? S.d_det : nullptr, s));
     MAVD_CUDA(cudaEventRecord(S.ev_done, s));
     // copy-out stream
     MAVD_CUDA(cudaStreamWaitEvent(h->s_out, S.ev_done, 0));
@@ -958,6 +1077,24 @@ int mavd_submit_host(mavd_handle h, int32_t slot, const uint8_t* h_frames, int32
     // the next batch's copy-in must not overwrite staging a kernel still reads: ordered by slot reuse rule
     S.busy = true;
     return MAVD_OK;
+}
+
+int mavd_submit_host(mavd_handle h, int32_t slot, const uint8_t* h_frames, int32_t n_pairs, int32_t pair_stride,
+                     const mavd_imu* h_imu, const mavd_detect_params* prm, const int32_t* h_samples,
+                     const mavd_aux_inputs* h_aux, int32_t flags, float* h_flow_out, uint8_t* h_fixed_out,
+                     mavd_frame_record* h_records, int32_t max_det, mavd_detection* h_det, void* stream) {
+    DeviceGuard dg(h ? h->cfg.device : -1);
+    return submit_host_run(h, slot, h_frames, n_pairs, pair_stride, false, nullptr, h_imu, prm, h_samples, h_aux, flags,
+                           h_flow_out, h_fixed_out, h_records, max_det, h_det, stream);
+}
+
+int mavd_stream_submit_host(mavd_handle h, int32_t slot, const uint8_t* h_frames, int32_t n, const int32_t* h_ids,
+                            const mavd_imu* h_imu, const mavd_detect_params* prm, const int32_t* h_samples,
+                            const mavd_aux_inputs* h_aux, int32_t flags, float* h_flow_out, uint8_t* h_fixed_out,
+                            mavd_frame_record* h_records, int32_t max_det, mavd_detection* h_det, void* stream) {
+    DeviceGuard dg(h ? h->cfg.device : -1);
+    return submit_host_run(h, slot, h_frames, n, 2, true, h_ids, h_imu, prm, h_samples, h_aux, flags, h_flow_out, h_fixed_out,
+                           h_records, max_det, h_det, stream);
 }
 
 int mavd_wait_host(mavd_handle h, int32_t slot) {

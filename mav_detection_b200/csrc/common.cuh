@@ -216,6 +216,14 @@ struct ProfScope {
     }
 };
 
+// R slots of a frame-stream call (api.cu: mavd_stream_*), device tables: the call's frame z is expanded into R slot
+// z_slot[z]; pair p reads its first frame's expansions from slot pair_slot[2p] and its second's from pair_slot[2p + 1].
+struct FrameSlots {
+    int n_frames;
+    const int* z_slot;
+    const int* pair_slot;
+};
+
 struct PolyConst {
     float g[kMaxPolyN + 1], xg[kMaxPolyN + 1], xxg[kMaxPolyN + 1];
     float ig11, ig03, ig33, ig55;
@@ -304,6 +312,17 @@ struct mavd_handle_s {
     int last_pairs = 0, last_stride = 1;
     float* last_flow0 = nullptr;
     const uint8_t* last_frames = nullptr;
+    bool last_was_stream = false;     // the last Farneback call was a frame-stream call: taps refuse
+    // frame streams (api.cu: mavd_stream_*): stream s keeps the expansions of its last frame in R slot
+    // 2s + stream_parity[s]; a step writes the new frame into the other slot of the two
+    std::vector<uint8_t> stream_live, stream_parity;   // [max_pairs]
+    int32_t* d_stream_slots = nullptr;  // [3][max_pairs]: FrameSlots::z_slot, then pair_slot (first stream call)
+    int32_t* h_stream_ring = nullptr;   // pinned [kImuRing][3][max_pairs]: staged like the imu
+    cudaEvent_t stream_ev[kImuRing] = {};
+    int stream_next = 0;
+    mavd::FrameSlots stream_slots(int n_frames) const {
+        return {n_frames, d_stream_slots, d_stream_slots + cfg.max_pairs};
+    }
 };
 
 namespace mavd {
@@ -321,8 +340,10 @@ static inline void pdl_break(mavd_handle h, int lane = 0) { h->pdl_ok[lane] = fa
 // farneback.cu
 // the pyramid levels of a new handle: schedule, tables, buffers and TMA descriptors (from h->cfg and h->max_frames)
 int farneback_setup(mavd_handle h);
+// fs == nullptr: the call's frames are R slots 0.., pair p reads slots p * pair_stride and p * pair_stride + 1.
+// A frame-stream call passes its device tables instead; with n_pairs == 0 it only expands its frames.
 int farneback_run(mavd_handle h, const uint8_t* d_frames, int n_pairs, int pair_stride, float* d_flow,
-                  cudaStream_t s);
+                  cudaStream_t s, const FrameSlots* fs = nullptr);
 int farneback_tap(mavd_handle h, int kind, int level, int index, float* d_out, cudaStream_t s);
 // detect.cu
 // the detection workspace of a new handle (the host slots are api.cu's)

@@ -552,10 +552,17 @@ __device__ __forceinline__ void polyexp_passes(const float* __restrict__ raw, fl
 
 // N_ > 0: poly_n known at compile time (5, 7 and 8 are instantiated: OpenCV's sample value, its other GPU value
 // and the reference's) so the tap loops carry no predicates; N_ == 0: any poly_n <= 8 at run time.
-template <bool U8, int N_>
+// R slot of the call's frame z: z itself, or (SLOTS: a frame-stream call) the table's entry (common.cuh: FrameSlots).
+// SLOTS is a template parameter so that the pair calls' instantiations are unchanged.
+template <bool SLOTS>
+__device__ __forceinline__ size_t r_slot_of(const int* __restrict__ z_slot, int z) {
+    return (size_t)(SLOTS ? __ldg(z_slot + z) : z);
+}
+
+template <bool U8, int N_, bool SLOTS>
 __global__ void __launch_bounds__(256, 4) polyexp_kernel(const void* __restrict__ src_base, size_t src_stride, int w,
                                                      int h, int pitch, int u8_aligned, PolyConst pc,
-                                                     float* __restrict__ R, size_t plane) {
+                                                     float* __restrict__ R, size_t plane, const int* __restrict__ z_slot) {
     pdl_entry();
     __shared__ __align__(16) float raw[(PE_TY + 2 * PE_H) * PE_RW];
     __shared__ __align__(16) float t[3][PE_TY * PE_RW];
@@ -656,7 +663,7 @@ __global__ void __launch_bounds__(256, 4) polyexp_kernel(const void* __restrict_
         }
     }
     __syncthreads();
-    polyexp_passes<N_>(raw, t, pc, n, tid, x0, y0, h, pitch, R + (size_t)blockIdx.z * 5 * plane, plane);
+    polyexp_passes<N_>(raw, t, pc, n, tid, x0, y0, h, pitch, R + r_slot_of<SLOTS>(z_slot, blockIdx.z) * 5 * plane, plane);
 }
 
 // a global store whose address space survives the register pinning of the base pointer below (a plain store through
@@ -757,7 +764,9 @@ __device__ __forceinline__ void resize_coord_pow2(int d, float scale, int src, i
 
 constexpr int MI_TX = 64, MI_TY = 4;   // matrices_init_kernel block: 64 x 4 pixels
 
-template <int COORD>
+// SLOTS: a frame-stream call, R0 / R1 from pair_slot (common.cuh: FrameSlots); the pair calls' instantiations keep the
+// affine addressing without a branch (registers and schedule of the hot kernels unchanged)
+template <int COORD, bool SLOTS>
 __global__ void __launch_bounds__(256, 8) matrices_init_kernel(const float* __restrict__ R, size_t plane, int w, int h,
                                                            int pitch, size_t R_pair_stride,
                                                            const float2* __restrict__ cflow, int cw, int ch,
@@ -766,7 +775,8 @@ __global__ void __launch_bounds__(256, 8) matrices_init_kernel(const float* __re
                                                            const float* __restrict__ fxa,
                                                            const int* __restrict__ fyi0,
                                                            const float* __restrict__ fya, float up_scale,
-                                                           float* __restrict__ M, double xscale, double yscale, int r0_first) {
+                                                           float* __restrict__ M, double xscale, double yscale, int r0_first,
+                                                           const int* __restrict__ pair_slot) {
     pdl_entry();
     // 3-D grid (pairs, tiles_x, tiles_y): blocks are scheduled x-fastest, so the pair index is fastest (same L2 sharing
     // of R between consecutive pairs as in iter_box_tma_kernel) and no thread pays for an integer division: with one
@@ -780,7 +790,7 @@ __global__ void __launch_bounds__(256, 8) matrices_init_kernel(const float* __re
     // stays a run-time branch because the compile-time form (R0 loaded first, no second load site) is slower: 2.15 vs
     // 2.05 ms per C2 step (B200, 1000 W).  With the order fixed, ptxas keeps the 64-bit pixel offset live from the R0
     // loads to the M stores and issues the R1 gather in smaller groups.
-    const float* R0 = R + (size_t)p * R_pair_stride;
+    const float* R0 = SLOTS ? R + (size_t)__ldg(pair_slot + 2 * p) * 5 * plane : R + (size_t)p * R_pair_stride;
     R0Px r0;
     if (r0_first) r0 = load_r0_px(R0, (size_t)y * pitch + x, plane);
     float dx = 0.f, dy = 0.f;
@@ -814,7 +824,8 @@ __global__ void __launch_bounds__(256, 8) matrices_init_kernel(const float* __re
     // than they save: the kernel is bound by the latency of its dependent memory round trips.  Round 2 repeated the
     // experiment at 32 registers (unsigned 32-bit element offsets from pinned base pointers, one IMAD.WIDE.U32 per
     // address, 352 instead of 384 SASS instructions, no spills): 2.20 vs 2.04 ms per 64-pair step — slower again.
-    update_matrices_px(x, y, w, h, pitch, plane, dx, dy, r0, R0 + 5 * plane, M + (size_t)p * 5 * plane);
+    const float* R1 = SLOTS ? R + (size_t)__ldg(pair_slot + 2 * p + 1) * 5 * plane : R0 + 5 * plane;
+    update_matrices_px(x, y, w, h, pitch, plane, dx, dy, r0, R1, M + (size_t)p * 5 * plane);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -847,9 +858,17 @@ struct IterArgs {
     int hx;                 // column halo, m rounded up to a multiple of 4
     float scale;            // 1 / winsize^2 (box) or 1 (Gaussian: kernel already normalised)
     int pair_stride;
+    const int* pair_slot;   // SLOTS kernels: R slots of pair p at [2p] / [2p + 1] (common.cuh: FrameSlots)
     const float* gk;        // Gaussian half kernel [m+1] (device) or nullptr
     int n_pairs, tiles_x;   // TMA kernel: 1-D grid (see iter_box_tma_kernel)
 };
+
+// R slot of pair p's first (k = 0) or second (k = 1) frame: the frame-stream table (SLOTS) or the pair calls' affine
+// layout.  SLOTS is a template parameter of the iteration kernels so that the pair calls' instantiations are unchanged.
+template <bool SLOTS>
+__device__ __forceinline__ int pair_r_slot(const IterArgs& a, int p, int k) {
+    return SLOTS ? __ldg(a.pair_slot + 2 * p + k) : p * a.pair_stride + k;
+}
 
 template <int M_>
 __device__ __forceinline__ void hsum_box(const float (&u)[20], float (&o)[4]) {
@@ -891,7 +910,7 @@ __device__ __forceinline__ void hsum_gauss_reg(const float (&u)[20], const float
     }
 }
 
-template <bool GAUSS, bool LAST>
+template <bool GAUSS, bool LAST, bool SLOTS>
 __global__ void __launch_bounds__(256, 3) iter_kernel(IterArgs a) {
     pdl_entry();
     extern __shared__ __align__(16) float smem[];
@@ -1008,8 +1027,8 @@ __global__ void __launch_bounds__(256, 3) iter_kernel(IterArgs a) {
     __syncthreads();
 
     // ---- per-pixel solve + matrix update (x fastest) ----
-    const float* R0 = a.R + (size_t)(p * a.pair_stride) * 5 * plane;
-    const float* R1 = R0 + 5 * plane;
+    const float* R0 = a.R + (size_t)pair_r_slot<SLOTS>(a, p, 0) * 5 * plane;
+    const float* R1 = SLOTS ? a.R + (size_t)pair_r_slot<true>(a, p, 1) * 5 * plane : R0 + 5 * plane;
     float* Mout = LAST ? nullptr : a.Mout + (size_t)p * 5 * plane;
 #pragma unroll 2
     for (int j = 0; j < (IT_TX * IT_TY) / 256; ++j) {
@@ -1086,9 +1105,10 @@ __device__ __forceinline__ void tma_prefetch_3d(const CUtensorMap* map, int c0, 
 // ------------------------------------------------------------------------------------------------
 constexpr int PE_BW = 96;   // bytes per staged u8 row: x0 - 16 .. x0 + 79 (16-byte aligned box origin)
 
-template <bool U8, int N_>
+template <bool U8, int N_, bool SLOTS>
 __global__ void __launch_bounds__(256, 4) polyexp_tma_kernel(const __grid_constant__ CUtensorMap tmap, int w, int h,
-                                                         int pitch, PolyConst pc, float* __restrict__ R, size_t plane) {
+                                                         int pitch, PolyConst pc, float* __restrict__ R, size_t plane,
+                                                         const int* __restrict__ z_slot) {
     pdl_entry();
     __shared__ __align__(128) float raw[(PE_TY + 2 * PE_H) * PE_RW];
     __shared__ __align__(128) float t[3][PE_TY * PE_RW];
@@ -1182,7 +1202,8 @@ __global__ void __launch_bounds__(256, 4) polyexp_tma_kernel(const __grid_consta
         }
     }
     // the passes address the tile with its first staged row at row PE_H - n
-    polyexp_passes<N_>(raw0 - (PE_H - n) * PE_RW, t, pc, n, tid, x0, y0, h, pitch, R + (size_t)blockIdx.z * 5 * plane, plane);
+    polyexp_passes<N_>(raw0 - (PE_H - n) * PE_RW, t, pc, n, tid, x0, y0, h, pitch,
+                       R + r_slot_of<SLOTS>(z_slot, blockIdx.z) * 5 * plane, plane);
 }
 
 // UpdateMatrices with the R1 footprint read from a shared-memory box [5][RH][RW] whose cell (0, 0) is image pixel
@@ -1270,7 +1291,7 @@ __device__ __forceinline__ void update_matrices_box(int x, int y, int w, int h, 
 // GAUSS: OPTFLOW_FARNEBACK_GAUSSIAN windows (FarnebackUpdateFlow_GaussianBlur): the vertical pass is the 2m+1-tap
 // filter on the same register window (in place, like the running sums), the horizontal one hsum_gauss; both with the
 // generic kernel's expressions, so the two kernels stay bit-identical.
-template <int M_, bool LAST, int TY, bool GAUSS>
+template <int M_, bool LAST, int TY, bool GAUSS, bool SLOTS>
 __global__ void __launch_bounds__(256, 3) iter_box_tma_kernel(const __grid_constant__ CUtensorMap tmap,
                                                               const __grid_constant__ CUtensorMap tmapR,
                                                               const __grid_constant__ CUtensorMap tmapRbox, IterArgs a) {
@@ -1319,8 +1340,11 @@ __global__ void __launch_bounds__(256, 3) iter_box_tma_kernel(const __grid_const
         mbar_expect_tx(&bar, 5 * CH * (uint32_t)sizeof(float));
         tma_load_3d(box, &tmap, x0 - IT_HX, y0 - M_, p * 5, &bar);
         // R0 (this tile) and R1 (this tile displaced by the flow) are read ~10 us from now by the per-pixel
-        // phase: start their HBM -> L2 transfer now (10 consecutive planes = both frames' expansions)
-        if (!LAST) tma_prefetch_3d(&tmapR, x0 - IT_HX, y0 - IT_HX, p * a.pair_stride * 5);
+        // phase: start their HBM -> L2 transfer now (10 consecutive planes = both frames' expansions: a stream's two
+        // R slots are adjacent too, in either order)
+        if (!LAST)
+            tma_prefetch_3d(&tmapR, x0 - IT_HX, y0 - IT_HX,
+                            (SLOTS ? min(pair_r_slot<true>(a, p, 0), pair_r_slot<true>(a, p, 1)) : p * a.pair_stride) * 5);
     }
     const bool interior = (x0 - IT_HX >= 0) && (x0 + IT_TX + IT_HX <= w) && (y0 - M_ >= 0) && (y0 + TY + M_ <= h);
     __syncthreads();
@@ -1460,8 +1484,8 @@ __global__ void __launch_bounds__(256, 3) iter_box_tma_kernel(const __grid_const
     //     into the box; (c) the bilinear gather reads shared memory with immediate offsets (one base address per
     //     pixel, ~30-cycle latency) instead of 20 global loads.  Pixels whose footprint leaves the box (flow
     //     differs from the centre's by more than ~5 px) take the global path; values are identical either way.
-    const float* R0 = a.R + (size_t)(p * a.pair_stride) * 5 * a.plane;
-    const float* R1 = R0 + 5 * a.plane;
+    const float* R0 = a.R + (size_t)pair_r_slot<SLOTS>(a, p, 0) * 5 * a.plane;
+    const float* R1 = SLOTS ? a.R + (size_t)pair_r_slot<true>(a, p, 1) * 5 * a.plane : R0 + 5 * a.plane;
     float* Mout = a.Mout + (size_t)p * 5 * a.plane;
     // keep the pair's M' base as ONE 64-bit register pair: the compiler otherwise carries (kernel argument + 64-bit
     // element offset) and rebuilds every store address with a 4-instruction add / shift chain instead of one
@@ -1533,7 +1557,7 @@ __global__ void __launch_bounds__(256, 3) iter_box_tma_kernel(const __grid_const
     if (tid == 0) {
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy reads before the async write
         mbar_expect_tx(&bar, 5 * CH * (uint32_t)sizeof(float));
-        tma_load_3d(box, &tmapRbox, bx, by, (p * a.pair_stride + 1) * 5, &bar);
+        tma_load_3d(box, &tmapRbox, bx, by, pair_r_slot<SLOTS>(a, p, 1) * 5, &bar);
     }
     // R0 of the first pixel is requested before waiting for the box, and R0 of pixel j + 1 while pixel j is being
     // worked on: the (L2-prefetched) loads are never waited for
@@ -1574,33 +1598,35 @@ __global__ void tap_flow_kernel(const float2* __restrict__ src, int w, int h, in
 // ------------------------------------------------------------------------------------------------
 // host-side orchestration
 // ------------------------------------------------------------------------------------------------
-template <bool GAUSS, bool LAST>
+template <bool GAUSS, bool LAST, bool SLOTS>
 static int launch_iter(const IterArgs& a, dim3 grid, size_t smem, cudaStream_t s, bool pdl) {
-    MAVD_CUDA((ensure_dynamic_smem<iter_kernel<GAUSS, LAST>>(200 * 1024)));
-    MAVD_CUDA(launch_chained(pdl, iter_kernel<GAUSS, LAST>, grid, 256, smem, s, a));
+    MAVD_CUDA((ensure_dynamic_smem<iter_kernel<GAUSS, LAST, SLOTS>>(200 * 1024)));
+    MAVD_CUDA(launch_chained(pdl, iter_kernel<GAUSS, LAST, SLOTS>, grid, 256, smem, s, a));
     MAVD_LAUNCHED();
     return MAVD_OK;
 }
 
-template <int M_, bool LAST, int TY, bool GAUSS>
+template <int M_, bool LAST, int TY, bool GAUSS, bool SLOTS>
 static int launch_iter_tma(const CUtensorMap& map, const CUtensorMap& mapR, const CUtensorMap& mapRbox, const IterArgs& a,
                            dim3 grid, cudaStream_t s, bool pdl) {
     constexpr size_t smem = sizeof(float) * 5 * (TY + 2 * M_) * IT_RW;
-    MAVD_CUDA((ensure_dynamic_smem<iter_box_tma_kernel<M_, LAST, TY, GAUSS>>(smem)));
-    MAVD_CUDA(launch_chained(pdl, iter_box_tma_kernel<M_, LAST, TY, GAUSS>, grid, 256, smem, s, map, mapR, mapRbox, a));
+    MAVD_CUDA((ensure_dynamic_smem<iter_box_tma_kernel<M_, LAST, TY, GAUSS, SLOTS>>(smem)));
+    MAVD_CUDA(launch_chained(pdl, iter_box_tma_kernel<M_, LAST, TY, GAUSS, SLOTS>, grid, 256, smem, s, map, mapR, mapRbox,
+                             a));
     MAVD_LAUNCHED();
     return MAVD_OK;
 }
 
-// 5 <= m <= 8; with small_tiles the caller built `grid` and the descriptors for 64 x 16 tiles
-template <bool LAST>
+// 5 <= m <= 8; with small_tiles the caller built `grid` and the descriptors for 64 x 16 tiles.  The last iteration
+// reads no R: SLOTS only for the others.
+template <bool LAST, bool SLOTS>
 static int launch_iter_tma_m(int m, bool gauss, bool small_tiles, const CUtensorMap& map, const CUtensorMap& mapR,
                              const CUtensorMap& mapRbox, const IterArgs& a, dim3 grid, cudaStream_t s, bool pdl) {
     using Launch = int (*)(const CUtensorMap&, const CUtensorMap&, const CUtensorMap&, const IterArgs&, dim3, cudaStream_t,
                            bool);
 #define ITER_TMA_M(TY, GAUSS)                                                                                             \
-    { launch_iter_tma<5, LAST, TY, GAUSS>, launch_iter_tma<6, LAST, TY, GAUSS>, launch_iter_tma<7, LAST, TY, GAUSS>,     \
-      launch_iter_tma<8, LAST, TY, GAUSS> }
+    { launch_iter_tma<5, LAST, TY, GAUSS, SLOTS>, launch_iter_tma<6, LAST, TY, GAUSS, SLOTS>,                          \
+      launch_iter_tma<7, LAST, TY, GAUSS, SLOTS>, launch_iter_tma<8, LAST, TY, GAUSS, SLOTS> }
     static const Launch table[2][2][4] = {   // [Gaussian window][64 x 16 tiles][m - 5]
         {ITER_TMA_M(IT_TY, false), ITER_TMA_M(IT_TY_SMALL, false)},
         {ITER_TMA_M(IT_TY, true), ITER_TMA_M(IT_TY_SMALL, true)}};
@@ -1869,10 +1895,12 @@ int farneback_setup(mavd_handle H) {
 }
 
 int farneback_run(mavd_handle H, const uint8_t* d_frames, int n_pairs, int pair_stride, float* d_flow,
-                  cudaStream_t s) {
+                  cudaStream_t s, const FrameSlots* fs) {
     const mavd_farneback_params& fp = H->cfg.farneback;
     const int W = H->cfg.width, Hh = H->cfg.height;
-    const int n_frames = pair_stride == 1 ? n_pairs + 1 : 2 * n_pairs;
+    const int n_frames = fs ? fs->n_frames : pair_stride == 1 ? n_pairs + 1 : 2 * n_pairs;
+    const int* z_slot = fs ? fs->z_slot : nullptr;
+    const int* pair_slot = fs ? fs->pair_slot : nullptr;
     const bool gauss = (fp.flags & MAVD_FARNEBACK_GAUSSIAN) != 0;
     const int m = fp.winsize / 2;
     const int hx = round_up(m, 4);
@@ -2024,26 +2052,32 @@ int farneback_run(mavd_handle H, const uint8_t* d_frames, int n_pairs, int pair_
         else if (use_tma)
             use_tma = L.has_tmap_img;
         const bool pdl = pdl_next(H, lane(st));
-#define PE_LAUNCH(N)                                                                                                   \
+#define PE_LAUNCH(N, S)                                                                                                \
         do {                                                                                                           \
             if (li == 0 && use_tma)                                                                                    \
-                MAVD_CUDA(launch_chained(pdl, polyexp_tma_kernel<true, N>, g, 256, 0, st, tmap_u8, L.w, L.h, L.pitch,   \
-                                         H->poly, L.R, L.plane));                                                      \
+                MAVD_CUDA(launch_chained(pdl, polyexp_tma_kernel<true, N, S>, g, 256, 0, st, tmap_u8, L.w, L.h,         \
+                                         L.pitch, H->poly, L.R, L.plane, z_slot));                                     \
             else if (li == 0)                                                                                          \
-                MAVD_CUDA(launch_chained(pdl, polyexp_kernel<true, N>, g, 256, 0, st, (const void*)d_frames,            \
-                                         frame_bytes, L.w, L.h, L.pitch, aligned, H->poly, L.R, L.plane));              \
+                MAVD_CUDA(launch_chained(pdl, polyexp_kernel<true, N, S>, g, 256, 0, st, (const void*)d_frames,         \
+                                         frame_bytes, L.w, L.h, L.pitch, aligned, H->poly, L.R, L.plane, z_slot));      \
             else if (use_tma)                                                                                          \
-                MAVD_CUDA(launch_chained(pdl, polyexp_tma_kernel<false, N>, g, 256, 0, st, L.tmapImg, L.w, L.h,         \
-                                         L.pitch, H->poly, L.R, L.plane));                                             \
+                MAVD_CUDA(launch_chained(pdl, polyexp_tma_kernel<false, N, S>, g, 256, 0, st, L.tmapImg, L.w, L.h,      \
+                                         L.pitch, H->poly, L.R, L.plane, z_slot));                                     \
             else                                                                                                       \
-                MAVD_CUDA(launch_chained(pdl, polyexp_kernel<false, N>, g, 256, 0, st, (const void*)L.img, L.plane,     \
-                                         L.w, L.h, L.pitch, 0, H->poly, L.R, L.plane));                                \
+                MAVD_CUDA(launch_chained(pdl, polyexp_kernel<false, N, S>, g, 256, 0, st, (const void*)L.img, L.plane,  \
+                                         L.w, L.h, L.pitch, 0, H->poly, L.R, L.plane, z_slot));                        \
         } while (0)
-        switch (H->poly.n) {
-            case 5: PE_LAUNCH(5); break;
-            case 7: PE_LAUNCH(7); break;
-            case 8: PE_LAUNCH(8); break;
-            default: PE_LAUNCH(0); break;
+        switch (H->poly.n * 2 + (z_slot ? 1 : 0)) {
+            case 10: PE_LAUNCH(5, false); break;
+            case 11: PE_LAUNCH(5, true); break;
+            case 14: PE_LAUNCH(7, false); break;
+            case 15: PE_LAUNCH(7, true); break;
+            case 16: PE_LAUNCH(8, false); break;
+            case 17: PE_LAUNCH(8, true); break;
+            default:
+                if (z_slot) PE_LAUNCH(0, true);
+                else PE_LAUNCH(0, false);
+                break;
         }
 #undef PE_LAUNCH
         MAVD_LAUNCHED();
@@ -2051,6 +2085,7 @@ int farneback_run(mavd_handle H, const uint8_t* d_frames, int n_pairs, int pair_
     };
     // matrices from the upsampled coarser flow, then the iterations of one level
     auto solve_level = [&](int li, cudaStream_t st) -> int {
+        if (n_pairs == 0) return MAVD_OK;        // mavd_stream_start: the expansions are all it keeps
         Level& L = H->lv[li];
         {
             ProfScope ps(&H->prof, MAVD_PROF_MATRICES, st);
@@ -2064,11 +2099,14 @@ int farneback_run(mavd_handle H, const uint8_t* d_frames, int n_pairs, int pair_
             const dim3 g3(n_pairs, ceil_div(L.w, MI_TX), ceil_div(L.h, MI_TY));       // pair index fastest
 #define MI_ARGS L.R, L.plane, L.w, L.h, L.pitch, (size_t)pair_stride * 5 * L.plane,                                     \
                 top ? nullptr : (const float2*)C->flow, top ? 0 : C->w, top ? 0 : C->h, top ? 0 : C->pitch,             \
-                top ? 0 : C->plane, L.fxi0, L.fxa, L.fyi0, L.fya, (float)(1.0 / fp.pyr_scale), L.M[0], xscale, yscale, 1
+                top ? 0 : C->plane, L.fxi0, L.fxa, L.fyi0, L.fya, (float)(1.0 / fp.pyr_scale), L.M[0], xscale, yscale, 1, pair_slot
             const bool pdl = pdl_next(H, lane(st));
-            if (coord == MI_COORD_TABLES) MAVD_CUDA(launch_chained(pdl, matrices_init_kernel<MI_COORD_TABLES>, g3, 256, 0, st, MI_ARGS));
-            else if (coord == MI_COORD_POW2) MAVD_CUDA(launch_chained(pdl, matrices_init_kernel<MI_COORD_POW2>, g3, 256, 0, st, MI_ARGS));
-            else MAVD_CUDA(launch_chained(pdl, matrices_init_kernel<MI_COORD_F64>, g3, 256, 0, st, MI_ARGS));
+#define MI_LAUNCH(C) MAVD_CUDA(pair_slot ? launch_chained(pdl, matrices_init_kernel<C, true>, g3, 256, 0, st, MI_ARGS)       \
+                                         : launch_chained(pdl, matrices_init_kernel<C, false>, g3, 256, 0, st, MI_ARGS))
+            if (coord == MI_COORD_TABLES) MI_LAUNCH(MI_COORD_TABLES);
+            else if (coord == MI_COORD_POW2) MI_LAUNCH(MI_COORD_POW2);
+            else MI_LAUNCH(MI_COORD_F64);
+#undef MI_LAUNCH
 #undef MI_ARGS
             MAVD_LAUNCHED();
         }
@@ -2083,6 +2121,7 @@ int farneback_run(mavd_handle H, const uint8_t* d_frames, int n_pairs, int pair_
             a.m = m; a.hx = hx;
             a.scale = gauss ? 1.f : (float)(1.0 / ((double)fp.winsize * fp.winsize));
             a.pair_stride = pair_stride;
+            a.pair_slot = pair_slot;
             a.gk = gauss ? H->gauss_win : nullptr;
             if (last) {
                 if (li == 0) {
@@ -2109,11 +2148,16 @@ int farneback_run(mavd_handle H, const uint8_t* d_frames, int n_pairs, int pair_
             if (m >= 5 && m <= 8 && L.has_tmap && !H->force_generic_iter) {
                 const CUtensorMap& mM = small_tiles ? L.tmapM16[cur] : L.tmapM[cur];
                 const CUtensorMap& mRb = small_tiles ? L.tmapRbox16 : L.tmapRbox;
-                rc = last ? launch_iter_tma_m<true>(m, gauss, small_tiles, mM, L.tmapR, mRb, a, g1, st, pdl)
-                          : launch_iter_tma_m<false>(m, gauss, small_tiles, mM, L.tmapR, mRb, a, g1, st, pdl);
+                rc = last ? launch_iter_tma_m<true, false>(m, gauss, small_tiles, mM, L.tmapR, mRb, a, g1, st, pdl)
+                   : pair_slot ? launch_iter_tma_m<false, true>(m, gauss, small_tiles, mM, L.tmapR, mRb, a, g1, st, pdl)
+                               : launch_iter_tma_m<false, false>(m, gauss, small_tiles, mM, L.tmapR, mRb, a, g1, st, pdl);
+            } else {
+                using Launch = int (*)(const IterArgs&, dim3, size_t, cudaStream_t, bool);
+                static const Launch generic[2][3] = {   // [Gaussian window][last, not last, not last from the tables]
+                    {launch_iter<false, true, false>, launch_iter<false, false, false>, launch_iter<false, false, true>},
+                    {launch_iter<true, true, false>, launch_iter<true, false, false>, launch_iter<true, false, true>}};
+                rc = generic[gauss][last ? 0 : pair_slot ? 2 : 1](a, g, smem, st, pdl);
             }
-            else if (gauss) rc = last ? launch_iter<true, true>(a, g, smem, st, pdl) : launch_iter<true, false>(a, g, smem, st, pdl);
-            else       rc = last ? launch_iter<false, true>(a, g, smem, st, pdl) : launch_iter<false, false>(a, g, smem, st, pdl);
             if (rc != MAVD_OK) return rc;
             if (!last) cur ^= 1;
         }

@@ -85,6 +85,9 @@ class Engine:
         self.detect_params = DetectParams()
         self.lib.mavd_default_detect_params(C.byref(self.detect_params))
         self._inflight: Dict[int, tuple] = {}
+        self._open_streams: set = set()
+        # counts the non-stream Farneback calls made through this engine: each one ends every frame stream
+        self.stream_epoch = 0
 
     # -- lifecycle --------------------------------------------------------------------------
     def close(self) -> None:
@@ -242,6 +245,7 @@ class Engine:
         self._check_frames(frames, n_pairs, pair_stride)
         if out is None:
             out = torch.empty((n_pairs, self.height, self.width, 2), dtype=torch.float32, device=self.device)
+        self.stream_epoch += 1
         check(self.lib.mavd_farneback(self._h, frames.data_ptr(), n_pairs, pair_stride, out.data_ptr(),
                                       self._stream()))
         return out
@@ -484,6 +488,7 @@ class Engine:
             records = torch.empty((n_pairs, RECORD_DTYPE.itemsize), dtype=torch.uint8, device=self.device)
         aux = self._aux(sky, seg, gt_flow, n_pairs)
         max_det, det = self._det_device(detections, n_pairs)
+        self.stream_epoch += 1
         check(self.lib.mavd_process(self._h, frames.data_ptr(), n_pairs, pair_stride, imu, C.byref(self.detect_params),
                                     samples.data_ptr(), C.byref(aux), _ptr(flow_out), _ptr(total_out), _ptr(fixed_out),
                                     records.data_ptr(), max_det, _ptr(det), self._stream()))
@@ -509,7 +514,8 @@ class Engine:
                                    _ptr(det), self._stream()))
         return records if det is None else (records, det)
 
-    def _host_args(self, frames, samples, n_pairs, pair_stride, flow_out, fixed_out, records, fixed_packed=False):
+    def _host_args(self, frames, samples, n_pairs, pair_stride, flow_out, fixed_out, records, fixed_packed=False,
+                   stream_step=False):
         if n_pairs is None:
             n_pairs = frames.shape[0] - 1 if pair_stride == 1 else frames.shape[0] // 2
         if records is None:
@@ -519,7 +525,7 @@ class Engine:
                 raise ValueError('%s must be C-contiguous' % name)
         if samples.dtype != np.int32 or samples.size < n_pairs * _lib.SAMPLES_PER_FRAME:
             raise ValueError('samples must be int32 (n, %d)' % _lib.SAMPLES_PER_FRAME)
-        need = n_pairs + 1 if pair_stride == 1 else 2 * n_pairs
+        need = n_pairs if stream_step else n_pairs + 1 if pair_stride == 1 else 2 * n_pairs
         if frames is not None and (frames.dtype != np.uint8 or frames.shape[0] < need or
                                    tuple(frames.shape[1:]) not in ((self.height, self.width),
                                                                    (self.height, self.width, 3))):
@@ -554,16 +560,33 @@ class Engine:
         seg_packed / sky_packed: the masks are given at 1 bit per pixel (pack_mask_host); fixed_packed: fixed_out
         receives (n, packed_mask_bytes) bits; copy_only: move the bytes but skip the compute (host-feed ceiling);
         detections: an (n, max_det) DETECTION_DTYPE host array (pinned) that receives each pair's detection table."""
+        return self._submit_host(slot, frames, None, imu, samples, n_pairs, pair_stride, sky, seg, flow_out, fixed_out,
+                                 records, gt_flow, seg_packed, sky_packed, fixed_packed, copy_only, detections)
+
+    def _submit_host(self, slot, frames, ids, imu, samples, n_pairs, pair_stride, sky, seg, flow_out, fixed_out, records,
+                     gt_flow, seg_packed, sky_packed, fixed_packed, copy_only, detections) -> np.ndarray:
+        """submit_host (ids None) or stream_submit_host."""
+        if ids is not None:
+            n_pairs, id_arr = self._stream_ids(ids)
         n_pairs, records = self._host_args(frames, samples, n_pairs, pair_stride, flow_out, fixed_out, records,
-                                           fixed_packed)
+                                           fixed_packed, stream_step=ids is not None)
         aux = self._aux(sky, seg, gt_flow, n_pairs, host=True, sky_packed=sky_packed, seg_packed=seg_packed)
         flags = (_lib.HOST_BGR if frames.ndim == 4 else 0) | (_lib.HOST_SEG_PACKED if seg_packed else 0) | \
             (_lib.HOST_SKY_PACKED if sky_packed else 0) | (_lib.HOST_FIXED_PACKED if fixed_packed else 0) | \
             (_lib.HOST_COPY_ONLY if copy_only else 0)
         max_det, det = self._det_host(detections, n_pairs)
-        check(self.lib.mavd_submit_host(self._h, slot, _hp(frames), n_pairs, pair_stride, imu,
-                                        C.byref(self.detect_params), _hp(samples), C.byref(aux), flags, _hp(flow_out),
-                                        _hp(fixed_out), records.ctypes.data, max_det, det, self._stream()))
+        if ids is None:
+            if not copy_only:
+                self.stream_epoch += 1
+            check(self.lib.mavd_submit_host(self._h, slot, _hp(frames), n_pairs, pair_stride, imu,
+                                            C.byref(self.detect_params), _hp(samples), C.byref(aux), flags,
+                                            _hp(flow_out), _hp(fixed_out), records.ctypes.data, max_det, det,
+                                            self._stream()))
+        else:
+            check(self.lib.mavd_stream_submit_host(self._h, slot, _hp(frames), n_pairs, id_arr, imu,
+                                                   C.byref(self.detect_params), _hp(samples), C.byref(aux), flags,
+                                                   _hp(flow_out), _hp(fixed_out), records.ctypes.data, max_det, det,
+                                                   self._stream()))
         # keep the host buffers alive until the wait
         self._inflight[slot] = (frames, imu, samples, sky, seg, gt_flow, flow_out, fixed_out, records, detections)
         return records
@@ -571,6 +594,75 @@ class Engine:
     def wait_host(self, slot: int) -> None:
         check(self.lib.mavd_wait_host(self._h, slot))
         self._inflight.pop(slot, None)
+
+    # -- frame streams (include/mavd.h: mavd_stream_start) ------------------------------------------
+    def open_stream(self) -> int:
+        """A free stream id of this engine (0 .. max_pairs-1).  Raises ValueError when all max_pairs are open."""
+        for i in range(self.max_pairs):
+            if i not in self._open_streams:
+                self._open_streams.add(i)
+                return i
+        raise ValueError('all %d frame streams of this engine are open' % self.max_pairs)
+
+    def close_stream(self, stream_id: int) -> None:
+        """Give a stream id back to open_stream."""
+        self._open_streams.discard(int(stream_id))
+
+    def _stream_ids(self, ids: Iterable[int]) -> Tuple[int, C.Array]:
+        ids = [int(i) for i in ids]
+        return len(ids), (C.c_int32 * max(1, len(ids)))(*ids)
+
+    def _check_stream_frames(self, frames: torch.Tensor, n: int) -> None:
+        if frames.dtype != torch.uint8 or not frames.is_cuda or not frames.is_contiguous() or frames.dim() != 3 or \
+                tuple(frames.shape) != (n, self.height, self.width):
+            raise ValueError('frames must be a contiguous CUDA uint8 tensor (%d, %d, %d): one new frame per id'
+                             % (n, self.height, self.width))
+
+    def stream_start(self, frames: torch.Tensor, ids: Sequence[int]) -> None:
+        """(Re)start the streams `ids` with frames[i] as stream ids[i]'s first frame (no flow)."""
+        n, id_arr = self._stream_ids(ids)
+        self._check_stream_frames(frames, n)
+        check(self.lib.mavd_stream_start(self._h, frames.data_ptr(), n, id_arr, self._stream()))
+
+    def stream_farneback(self, frames: torch.Tensor, ids: Sequence[int],
+                         out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """One step of the streams `ids`: flow of (stream ids[i]'s kept frame, frames[i]) for every i, which is then
+        kept.  Equals farneback() with pair_stride 2 on the explicit pairs, bit for bit."""
+        n, id_arr = self._stream_ids(ids)
+        self._check_stream_frames(frames, n)
+        if out is None:
+            out = torch.empty((n, self.height, self.width, 2), dtype=torch.float32, device=self.device)
+        check(self.lib.mavd_stream_farneback(self._h, frames.data_ptr(), n, id_arr, out.data_ptr(), self._stream()))
+        return out
+
+    def stream_process(self, frames: torch.Tensor, ids: Sequence[int], imu, samples: torch.Tensor,
+                       sky: Optional[torch.Tensor] = None, seg: Optional[torch.Tensor] = None,
+                       flow_out: Optional[torch.Tensor] = None, total_out: Optional[torch.Tensor] = None,
+                       fixed_out: Optional[torch.Tensor] = None, records: Optional[torch.Tensor] = None,
+                       gt_flow: Optional[torch.Tensor] = None, detections: Optional[int] = None):
+        """process() for one step of the streams `ids` (stream_farneback's pairs); returns what process() returns."""
+        n, id_arr = self._stream_ids(ids)
+        self._check_stream_frames(frames, n)
+        self._check_samples(samples, n)
+        if records is None:
+            records = torch.empty((n, RECORD_DTYPE.itemsize), dtype=torch.uint8, device=self.device)
+        aux = self._aux(sky, seg, gt_flow, n)
+        max_det, det = self._det_device(detections, n)
+        check(self.lib.mavd_stream_process(self._h, frames.data_ptr(), n, id_arr, imu, C.byref(self.detect_params),
+                                           samples.data_ptr(), C.byref(aux), _ptr(flow_out), _ptr(total_out),
+                                           _ptr(fixed_out), records.data_ptr(), max_det, _ptr(det), self._stream()))
+        return records if det is None else (records, det)
+
+    def stream_submit_host(self, slot: int, frames: np.ndarray, ids: Sequence[int], imu, samples: np.ndarray,
+                           sky: Optional[np.ndarray] = None, seg: Optional[np.ndarray] = None,
+                           flow_out: Optional[np.ndarray] = None, fixed_out: Optional[np.ndarray] = None,
+                           records: Optional[np.ndarray] = None, gt_flow: Optional[np.ndarray] = None,
+                           seg_packed: bool = False, sky_packed: bool = False, fixed_packed: bool = False,
+                           copy_only: bool = False, detections: Optional[np.ndarray] = None) -> np.ndarray:
+        """submit_host for one step of the streams `ids`: HOST frames (n, H, W) gray or (n, H, W, 3) BGR, one per id;
+        outputs valid after wait_host(slot)."""
+        return self._submit_host(slot, frames, ids, imu, samples, None, 2, sky, seg, flow_out, fixed_out, records,
+                                 gt_flow, seg_packed, sky_packed, fixed_packed, copy_only, detections)
 
     def detect_host(self, flow: np.ndarray, imu, samples: np.ndarray, sky: Optional[np.ndarray] = None,
                     seg: Optional[np.ndarray] = None, fixed_out: Optional[np.ndarray] = None,

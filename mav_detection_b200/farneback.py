@@ -6,12 +6,17 @@
 converts it to gray on the device (mavd_bgr2gray == cv2.cvtColor, :74), computes the dense flow against the
 previous frame with the reference's parameters (mavd_farneback == cv2.calcOpticalFlowFarneback(..., 0.4, 1, 12,
 10, 8, 1.2, 0), :76-80), keeps `prevgray` (:81) and returns the HSV visualisation (:83-99) built by
-mavd_flow_vis.  The reference discards the flow; here it stays available as `self.flow` ((H, W, 2) float32
+mavd_flow_vis.  The previous frame is kept expanded on the device in one frame stream of the engine
+(mavd_stream_farneback), so each call expands only the new frame; when the engine has no free stream the call pairs
+the two frames explicitly, with the same result.  Another user's non-stream call on the engine ends the stream; after
+that has happened before two calls in a row, process() pairs explicitly (one launch sequence, where a restart and a
+step would take two) until a call finds that nobody else used the engine since the previous one.  The reference discards the flow; here it stays available as `self.flow` ((H, W, 2) float32
 CUDA tensor) for callers that want the field itself.  draw_flow / draw_hsv / warp_flow (:28-69) are unused
 drawing helpers and are not rebuilt."""
 from __future__ import annotations
 
 import ctypes as C
+import weakref
 from typing import Any, Dict, Optional
 
 import numpy as np
@@ -47,6 +52,15 @@ class Farneback:
         self.rolling_history_id = 0
         self.flow: Optional['torch.Tensor'] = None
         self._scratch = torch.zeros((3,), dtype=torch.int32, device=engine.device)
+        self._live = False               # the stream holds prevgray
+        self._ended_in_a_row = 0         # calls in a row before which another user's non-stream call ended the stream
+        self._stream_epoch = engine.stream_epoch
+        try:
+            self._stream: Optional[int] = engine.open_stream()
+        except ValueError:
+            self._stream = None          # every stream of the engine is taken: explicit pairs
+        else:
+            weakref.finalize(self, engine.close_stream, self._stream)
 
     @property
     def prevgray(self) -> np.ndarray:
@@ -57,8 +71,18 @@ class Farneback:
         _, img = self.capture.read()
         img = np.ascontiguousarray(img)
         gray = eng.bgr2gray(torch.from_numpy(img).to(eng.device))
-        pair = torch.stack([self._prevgray_d, gray])
-        self.flow = eng.farneback(pair, n_pairs=1)[0]
+        # a non-stream Farneback call by another user of the engine since our last call ended the stream
+        ended = eng.stream_epoch != self._stream_epoch
+        self._ended_in_a_row = self._ended_in_a_row + 1 if ended else 0
+        if self._stream is None or self._ended_in_a_row >= 2:
+            self.flow = eng.farneback(torch.stack([self._prevgray_d, gray]), n_pairs=1)[0]
+            self._live = False           # that call ended our stream too
+        else:
+            if ended or not self._live:
+                eng.stream_start(self._prevgray_d[None], [self._stream])
+            self.flow = eng.stream_farneback(gray[None], [self._stream])[0]
+            self._live = True
+        self._stream_epoch = eng.stream_epoch
         self._prevgray_d = gray
         h, w = gray.shape
         bgr = torch.empty((h, w, 3), dtype=torch.uint8, device=eng.device)
